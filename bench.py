@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — extrinsic cost evaluations / s at KITTI-00 shape (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c1|c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c1|c2|c3|c4|c5] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 BASELINE.json configs -> `--config` (default c2, the one the metric is quoted on):
@@ -77,7 +77,24 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the side measurements (poll batch, per-query plane fit)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--seed", type=int, default=1000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0's record; with "
+                         "--shard candidates that covers only rank 0's candidates)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+def dump_outputs(d, eval_sums, lin_sums):
+    """The record of the last timed step as float64 arrays: DIR/eval_sums.npy, the [B,12] BAError sums
+    (stl_eval_sums_t), and DIR/lin_sums.npy, the [B,62] cost / J^T r / J^T J (stl_lin_sums_t) when the step
+    linearises.  The inputs follow from the arguments alone (seeded generator and candidates), so two builds run
+    with the same arguments can be compared array for array.  Rank 0 writes its record: with keyframes sharded that is
+    the whole step, with `--shard candidates` only rank 0's B candidates."""
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "eval_sums.npy"), np.ascontiguousarray(eval_sums, dtype=np.float64))
+    if lin_sums is not None:
+        np.save(os.path.join(d, "lin_sums.npy"), np.ascontiguousarray(lin_sums, dtype=np.float64))
 
 
 def workload_config(args):
@@ -259,8 +276,10 @@ def run_reference(args, rank):
         arm.step(cands(i))
     t0 = time.perf_counter()
     for i in range(args.steps):
-        arm.step(cands(args.warmup + i))
+        last = arm.step(cands(args.warmup + i))
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last)
     frac = (nkf_s / F) * (B_s / c["B"])          # share of one step's work the sample covers
     val = c["B"] * frac / dt
     sample = (f"{nkf_s} of {F} keyframes x {B_s} of {c['B']} candidates per step"
@@ -400,6 +419,9 @@ def main():
     exch = ctx.comm_stats() if (by_kf and world > 1) else {}
     launches = int(wc["launches"] - launches0)
     rec = d_out.cpu().numpy()                  # [steps, B, W]
+    if args.dump_outputs and rank == 0:
+        E = _abi.STL_EVAL_NSUMS
+        dump_outputs(args.dump_outputs, rec[args.steps - 1][:, :E], rec[args.steps - 1][:, E:] if mode != "eval" else None)
 
     # ---- end to end through the host-facing C-ABI (host buffers in and out)
     barrier()

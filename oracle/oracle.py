@@ -8,6 +8,7 @@ cpu_baseline / --impl reference legs may import this module.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import importlib
 import os
 import subprocess
@@ -118,6 +119,19 @@ def load_refmath():
 
 def have_ref() -> bool:
     return os.path.exists(REF_PATH)
+
+
+def digest(*arrays) -> int:
+    """64-bit BLAKE2b of the arrays' dtypes, shapes and bytes (-0.0 counted as 0.0): what a stored fixture keeps
+    of an output too large to store, equal exactly when the arrays are equal bit for bit."""
+    h = hashlib.blake2b(digest_size=8)
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        if a.dtype.kind == "f":
+            a = a + a.dtype.type(0)
+        h.update(f"{a.dtype.str}{a.shape}".encode())
+        h.update(a.tobytes())
+    return int.from_bytes(h.digest(), "little")
 
 
 def _d(a):

@@ -2,77 +2,73 @@
 
 oracle/_ref/liboracle_refmath.so holds include/pointcloud.h:126-158 (ComputeCovariance), :194-288 (ComputeEigenvector0/1),
 :378-463 (FastEigen3x3_EV) and include/g2o_tools.h:58-69,105-140,149-183 (skew, Sim3Exp<T>, SE3Exp<T>) cut out of
-/root/reference and compiled verbatim against a stand-in for the Eigen types they use (oracle/ref_shim_eigen.hpp).
-This pins the restatement (oracle_math.hpp) mechanically: any drift from the reference's text shows up here."""
+the reference's sources and compiled verbatim against a stand-in for the Eigen types they use (oracle/ref_shim_eigen.hpp).
+This pins the restatement (oracle_math.hpp) mechanically: any drift from the reference's text shows up here.
+
+The restatement is compared with the stored results of tests/golden/pin/refmath.npz (made by
+tests/golden/pin/make_pin_golden.py, whose seeded inputs the tests rebuild; `backend` names what produced them)
+and, where the library is built, with it live."""
 import ctypes as C
+import os
+import sys
 
 import numpy as np
 import pytest
+
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "pin")
+sys.path.insert(0, GOLDEN)
+import make_pin_golden as M  # noqa: E402
 
 _dp = C.POINTER(C.c_double)
 
 
 @pytest.fixture(scope="module")
-def refm(oracle_mod):
-    lib = oracle_mod.load_refmath()
-    if lib is None:
-        pytest.skip("oracle/_ref/liboracle_refmath.so not built (needs /root/reference)")
-    return lib
+def stored(oracle_mod):
+    g = np.load(os.path.join(GOLDEN, "refmath.npz"))
+    inputs = M.refmath_inputs()
+    assert oracle_mod.digest(*inputs) == int(g["input_digest"]), "the seeded inputs changed"
+    return g, inputs
 
 
 def _d(a):
     return a.ctypes.data_as(_dp)
 
 
-def test_covariance_and_smallest_eigenvector_bit_exact(refm, oracle_mod):
+def test_covariance_and_smallest_eigenvector_bit_exact(stored, oracle_mod):
+    g, (Pall, idxall, off, kinds, _) = stored
     port = oracle_mod.load("port")
-    rng = np.random.default_rng(0)
-    n_plane = n_general = 0
-    for trial in range(400):
-        m = int(rng.integers(3, 31))
-        kind = trial % 4
-        if kind == 0:      # points near a plane (the common case on LiDAR scans)
-            nrm = rng.normal(size=3); nrm /= np.linalg.norm(nrm)
-            P = rng.normal(0, 0.3, (m, 3)); P -= np.outer(P @ nrm, nrm) * 0.98
-            n_plane += 1
-        elif kind == 1:    # general position
-            P = rng.normal(0, 0.3, (m, 3)); n_general += 1
-        elif kind == 2:    # nearly collinear
-            d = rng.normal(size=3); P = np.outer(rng.normal(0, 0.5, m), d) + rng.normal(0, 1e-3, (m, 3))
-        else:              # axis-aligned grid: zero off-diagonal covariance (the `norm > 0` else-branch)
-            P = np.zeros((m, 3)); P[:, trial % 3] = np.arange(m) * 0.1
-        P = (P + rng.uniform(-30, 30, 3)).astype(np.float32).astype(np.float64)   # scan coordinates are float32 values
-        idx = rng.permutation(m).astype(np.uint32)
-        cov_ref = np.zeros(9); cov_port = np.zeros(6)
-        refm.refm_covariance(_d(P), m, idx.ctypes.data_as(C.POINTER(C.c_uint32)), m, _d(cov_ref))
+    refm = oracle_mod.load_refmath()
+    assert (kinds == 0).any() and (kinds == 1).any()   # near a plane (the common case on LiDAR scans), general position
+    for trial in range(len(off) - 1):
+        P = np.ascontiguousarray(Pall[off[trial]:off[trial + 1]])
+        idx = np.ascontiguousarray(idxall[off[trial]:off[trial + 1]])
+        m = len(idx)
+        cov_port, ev_port = np.zeros(6), np.zeros(3)
         port.orc_covariance(_d(P), idx.ctypes.data_as(C.POINTER(C.c_uint32)), m, _d(cov_port))
-        full = cov_ref.reshape(3, 3)
-        assert np.array_equal(full, full.T)
-        assert np.array_equal(cov_port, full[np.triu_indices(3)]), trial
-        ev_ref, eval_ref, ev_port = np.zeros(3), np.zeros(3), np.zeros(3)
-        refm.refm_fast_eigen(_d(cov_ref), _d(ev_ref), _d(eval_ref))
         port.orc_smallest_eigvec(_d(cov_port), _d(ev_port))
-        assert np.array_equal(ev_port, ev_ref), (trial, ev_port, ev_ref)
-    assert n_plane and n_general
+        assert np.array_equal(cov_port, g["cov"][trial]), trial
+        assert np.array_equal(ev_port, g["ev"][trial]), (trial, ev_port, g["ev"][trial])
+        if refm is not None:
+            cov_ref = np.zeros(9)
+            refm.refm_covariance(_d(P), m, idx.ctypes.data_as(C.POINTER(C.c_uint32)), m, _d(cov_ref))
+            full = cov_ref.reshape(3, 3)
+            assert np.array_equal(full, full.T)
+            assert np.array_equal(cov_port, full[np.triu_indices(3)]), trial
+            ev_ref, eval_ref = np.zeros(3), np.zeros(3)
+            refm.refm_fast_eigen(_d(cov_ref), _d(ev_ref), _d(eval_ref))
+            assert np.array_equal(ev_port, ev_ref), (trial, ev_port, ev_ref)
 
 
-def test_sim3exp_se3exp_bit_exact_including_jets(refm, oracle_mod):
+def test_sim3exp_se3exp_bit_exact_including_jets(stored, oracle_mod):
+    """Sim3Exp values AND all 7 partials of R, t, s (the dual), and SE3Exp(-x[0:6])."""
+    g, (_, _, _, _, xs) = stored
     port = oracle_mod.load("port")
-    rng = np.random.default_rng(1)
-    for trial in range(300):
-        x = np.concatenate([rng.normal(0, 1.0, 3), rng.normal(0, 0.5, 3), [rng.uniform(0.5, 30)]])
-        if trial % 5 == 0:
-            x[:3] *= 1e-5                                    # Taylor branch (theta < 1e-4)
-        R1, t1, R2, t2 = np.zeros(9), np.zeros(3), np.zeros(9), np.zeros(3)
-        s1, s2 = C.c_double(0), C.c_double(0)
-        refm.refm_sim3exp(_d(x), _d(R1), _d(t1), C.byref(s1))
-        port.orc_sim3exp(_d(x), _d(R2), _d(t2), C.byref(s2))
-        assert np.array_equal(R1, R2) and np.array_equal(t1, t2) and s1.value == s2.value == x[6]
-        d1, d2 = np.zeros(13 * 8), np.zeros(13 * 8)
-        refm.refm_sim3exp_dual(_d(x), _d(d1))
-        port.orc_sim3exp_dual(_d(x), _d(d2))
-        assert np.array_equal(d1, d2), trial                 # values AND all 7 partials of R, t, s
-        xm = np.ascontiguousarray(-x[:6])
-        refm.refm_se3exp(_d(xm), _d(R1), _d(t1))
-        port.orc_se3exp(_d(xm), _d(R2), _d(t2))
-        assert np.array_equal(R1, R2) and np.array_equal(t1, t2)
+    refm = oracle_mod.load_refmath()
+    assert (np.abs(xs[:, :3]).max(axis=1) < 1e-4).any()   # the Taylor branch (theta < 1e-4) is exercised
+    for trial, x in enumerate(xs):
+        got = M.sim3_se3(port, "orc_", x)
+        assert got[2][0] == x[6]
+        assert oracle_mod.digest(*got) == int(g["exp"][trial]), trial
+        if refm is not None:
+            want = M.sim3_se3(refm, "refm_", x)
+            assert all(np.array_equal(a, b) for a, b in zip(got, want)), trial
