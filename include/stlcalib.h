@@ -289,6 +289,45 @@ stl_status_t stl_gpr_hyper(stl_ctx_t *ctx, double *sigma_l, int64_t cap_blocks);
 /* Block counts {plane 2d, pt, pl, gpr 2d} of the last association of this context (waits for it). */
 stl_status_t stl_block_counts(stl_ctx_t *ctx, int64_t n_blocks[4]);
 
+/* ---- several starts: a PROBLEM SET ------------------------------------------------------------------------
+ * Multi-start refinement (refine the best few points of a NOMAD run, or run iba_local from several perturbed initial
+ * extrinsics, iba_local.cpp:145-323,434-460) on ONE context: the context freezes P independent BuildProblems, problem p
+ * associated at its own x0[p], and evaluates candidate b on the problem it names.  stl_associate(x0) is
+ * stl_associate_multi(x0, 1, NULL); every single-problem call keeps its results and meaning on a set of one, and returns
+ * STL_ERR_STATE (naming the multi call) while the set holds more than one problem — stl_associate (or stl_step_batch
+ * with reassociate != 0) freezes a set of one again.
+ * Problem p gives bit for bit what a fresh stl_associate(x0[p]) followed by stl_linearize_batch gives: the same block
+ * counts and the same [62] record, whatever P, whichever problems share the call and however the workspace chunks it.
+ * With a communicator attached the [B][62] / [P][74] record is exchanged once, like the other records; block counts are
+ * this rank's.  Errors: P < 1, a problem index outside [0, P), or a rebuild mask with P different from the size of the
+ * frozen set -> STL_ERR_INVALID; P > STL_MAX_PROBLEMS -> STL_ERR_CAPACITY; variant 1 -> STL_ERR_STATE (as stl_associate).
+ * A failed allocation leaves no set (the next call starts over). */
+#define STL_MAX_PROBLEMS 256   /* = the candidate cap of the evaluation workspace and of the peer-memory record exchange */
+
+/* BuildProblem at x0[p] for p < P (x0 [P][7]).
+ * rebuild == NULL: the set is replaced by P new problems.
+ * rebuild != NULL: P must equal the current set size; only problems with rebuild[p] != 0 are re-associated (at x0[p]); the
+ *   others keep their blocks bit for bit.
+ * The 2-D association of the starts comes from the workspace when the preceding evaluation left exactly those x0 there (as
+ * stl_associate); all rebuilt problems are associated by the same kernel launches, chunk by chunk of the workspace.
+ * With params.gpr_optimize the hyper-parameter fit runs once per rebuilt problem.
+ * n_blocks [P][4] as in stl_associate; NULL = asynchronous (read them with stl_block_counts_multi). */
+stl_status_t stl_associate_multi(stl_ctx_t *ctx, const double *x0, int32_t P, const uint8_t *rebuild, int64_t *n_blocks);
+/* Block counts [P][4] of every problem of the set (waits for the association); cap_problems < P -> STL_ERR_CAPACITY. */
+stl_status_t stl_block_counts_multi(stl_ctx_t *ctx, int64_t *n_blocks, int32_t cap_problems);
+
+/* cost, J^T r, J^T J of candidate b (x [B][7]) on problem problem[b] (NULL: B == P and candidate b on problem b), as
+ * stl_linearize_batch; the _device twin leaves the [B][62] record in DEVICE memory on `stream`. */
+stl_status_t stl_linearize_multi(stl_ctx_t *ctx, const double *x, int32_t B, const int32_t *problem, stl_lin_sums_t *out);
+stl_status_t stl_linearize_multi_device(stl_ctx_t *ctx, const double *x, int32_t B, const int32_t *problem, double *d_out, void *stream);
+
+/* One LM iteration for each of P starts (x [P][7]): BAError sums at x[p], BuildProblem at x[p] for the problems flagged in
+ * rebuild (NULL = all, which makes a new set), linearisation of problem p at x[p]; ONE [P][74] record, exchanged once.
+ * Same bits as stl_eval_batch + stl_associate_multi + stl_linearize_multi.  P = 1 is stl_step_batch(x, 1, rebuild ?
+ * rebuild[0] : 1) with its second-stream overlap; a larger set runs the stages one after another on one stream. */
+stl_status_t stl_step_multi(stl_ctx_t *ctx, const double *x, int32_t P, const uint8_t *rebuild, stl_step_sums_t *out);
+stl_status_t stl_step_multi_device(stl_ctx_t *ctx, const double *x, int32_t P, const uint8_t *rebuild, double *d_out, void *stream);
+
 /* BAError + (optionally) BuildProblem + linearisation in one call — what one LM / g2o iteration at x asks
  * for (iba_local.cpp:434-446 with the BAError value iba_global.cpp:169 logged beside it), or, for a NOMAD
  * poll batch, the cost record and the normal equations of every candidate on the frozen association:

@@ -83,6 +83,25 @@ class Context {
         check(stl_step_batch(ctx_, x, B, reassociate ? 1 : 0, out.data()), "stl_step_batch");
         return out;
     }
+    // several starts on one context (a problem set): BuildProblem at x0[p] for p < P ([P][7]); rebuild (optional [P]) re-associates
+    // only the flagged problems of the current set of P.  Block counts [P][4].
+    std::vector<std::array<int64_t, 4>> associate_multi(const double *x0, int P, const uint8_t *rebuild = nullptr) {
+        std::vector<std::array<int64_t, 4>> n((size_t)P);
+        check(stl_associate_multi(ctx_, x0, P, rebuild, n[0].data()), "stl_associate_multi");
+        return n;
+    }
+    // candidate b (x [B][7]) on problem problem[b] (null: B == P, candidate b on problem b)
+    std::vector<stl_lin_sums_t> linearize_multi(const double *x, int B, const int32_t *problem = nullptr) {
+        std::vector<stl_lin_sums_t> out((size_t)B);
+        check(stl_linearize_multi(ctx_, x, B, problem, out.data()), "stl_linearize_multi");
+        return out;
+    }
+    // one LM iteration of P starts: {eval sums, linearisation} of problem p at x[p], BuildProblem of the flagged problems first
+    std::vector<stl_step_sums_t> step_multi(const double *x, int P, const uint8_t *rebuild = nullptr) {
+        std::vector<stl_step_sums_t> out((size_t)P);
+        check(stl_step_multi(ctx_, x, P, rebuild, out.data()), "stl_step_multi");
+        return out;
+    }
     // keyframes sharded over several GPUs: this context holds shard `rank` of `n_ranks`; `id` comes from
     // stl_comm_unique_id on one rank (handed over by the host program).  Afterwards every call returns the totals.
     void comm_init(const uint8_t id[STL_COMM_ID_BYTES], int rank, int n_ranks) { check(stl_comm_init(ctx_, id, rank, n_ranks), "stl_comm_init"); }
@@ -154,6 +173,23 @@ class LMProblem {
   private:
     Context &ctx_;
     std::array<int64_t, 4> n_{};
+};
+
+// P LMProblems on one context (multi-start refinement): problem p is frozen at its own start.
+class LMProblemSet {
+  public:
+    explicit LMProblemSet(Context &ctx) : ctx_(ctx) {}
+    // X0 [P][7]; rebuild (optional [P]): re-associate only the flagged problems of the current set
+    std::vector<std::array<int64_t, 4>> build(const double *X0, int P, const uint8_t *rebuild = nullptr) {
+        return n_ = ctx_.associate_multi(X0, P, rebuild);
+    }
+    // candidate b (X [B][7]) on problem problem[b] (null: B == P, candidate p on problem p)
+    std::vector<stl_lin_sums_t> evaluate(const double *X, int B, const int32_t *problem = nullptr) { return ctx_.linearize_multi(X, B, problem); }
+    int size() const { return (int)n_.size(); }
+
+  private:
+    Context &ctx_;
+    std::vector<std::array<int64_t, 4>> n_;
 };
 
 }  // namespace stl

@@ -16,6 +16,7 @@ STL_EVAL_NSUMS = 12
 STL_LIN_NSUMS = 62
 STL_STEP_NSUMS = STL_EVAL_NSUMS + STL_LIN_NSUMS
 STL_COMM_ID_BYTES = 128
+STL_MAX_PROBLEMS = 256
 STL_NSTAGES = 8
 STAGE_NAMES = ("assoc2d", "knn3d", "reduce", "linearize", "build", "assoc_lm", "allreduce", "plane_index")
 
@@ -133,6 +134,7 @@ _dp = C.POINTER(C.c_double)
 _u32p = C.POINTER(C.c_uint32)
 _i32p = C.POINTER(C.c_int32)
 _i64p = C.POINTER(C.c_int64)
+_u8p = C.POINTER(C.c_uint8)
 
 # Every symbol include/stlcalib.h declares: name -> (restype, argtypes)
 CALIB_SYMBOLS = {
@@ -156,6 +158,12 @@ CALIB_SYMBOLS = {
     "stl_gpr_hyper": (C.c_int, [_vp, _dp, C.c_int64]),
     "stl_step_batch": (C.c_int, [_vp, _dp, C.c_int32, C.c_int32, C.POINTER(StepSums)]),
     "stl_step_batch_device": (C.c_int, [_vp, _dp, C.c_int32, C.c_int32, _vp, _vp]),
+    "stl_associate_multi": (C.c_int, [_vp, _dp, C.c_int32, _u8p, _i64p]),
+    "stl_block_counts_multi": (C.c_int, [_vp, _i64p, C.c_int32]),
+    "stl_linearize_multi": (C.c_int, [_vp, _dp, C.c_int32, _i32p, C.POINTER(LinSums)]),
+    "stl_linearize_multi_device": (C.c_int, [_vp, _dp, C.c_int32, _i32p, _vp, _vp]),
+    "stl_step_multi": (C.c_int, [_vp, _dp, C.c_int32, _u8p, C.POINTER(StepSums)]),
+    "stl_step_multi_device": (C.c_int, [_vp, _dp, C.c_int32, _u8p, _vp, _vp]),
     "stl_he_linearize": (C.c_int, [_vp, C.POINTER(HeEdges), _dp, C.c_int32, C.POINTER(LinSums), _dp]),
     "stl_calib_linearize": (C.c_int, [_vp, C.POINTER(CalibEdges), _dp, C.c_int32, C.POINTER(LinSums), _dp]),
     "stl_comm_unique_id": (C.c_int, [C.POINTER(C.c_uint8)]),

@@ -32,6 +32,7 @@ class Context:
         self.h = h
         self.device = device
         self.pack = None
+        self.n_problems = 0  # problems of the frozen set, set after each successful call that makes one (associate / step: 1, *_multi: P)
 
     def close(self):
         if getattr(self, "h", None):
@@ -93,10 +94,12 @@ class Context:
         if not wait:
             _check(self.lib, self.h, self.lib.stl_associate(self.h, x0.ctypes.data_as(_dp), None))
             self.n_blocks = None
+            self.n_problems = 1
             return None
         nb = np.zeros(4, np.int64)
         _check(self.lib, self.h, self.lib.stl_associate(self.h, x0.ctypes.data_as(_dp), nb.ctypes.data_as(_abi._i64p)))
         self.n_blocks = nb.copy()
+        self.n_problems = 1
         return nb
 
     def block_counts(self):
@@ -114,6 +117,8 @@ class Context:
         _check(self.lib, self.h, self.lib.stl_step_batch(self.h, x.ctypes.data_as(_dp), B, int(reassociate),
                                                          out.ctypes.data_as(C.POINTER(_abi.StepSums))))
         self.n_blocks = None
+        if reassociate:
+            self.n_problems = 1
         return out
 
     def step_device(self, x, d_out_ptr: int, stream_ptr: int = 0, reassociate: bool = True):
@@ -121,6 +126,82 @@ class Context:
         _check(self.lib, self.h, self.lib.stl_step_batch_device(self.h, x.ctypes.data_as(_dp), x.shape[0], int(reassociate),
                                                                 C.c_void_p(d_out_ptr), C.c_void_p(stream_ptr)))
         self.n_blocks = None
+        if reassociate:
+            self.n_problems = 1
+
+    # -- LM path, several starts (problem set) ---------------------------------------
+    @staticmethod
+    def _mask(rebuild, P):
+        if rebuild is None:
+            return None, None
+        m = np.ascontiguousarray(np.asarray(rebuild).reshape(-1) != 0, dtype=np.uint8)
+        if m.size != P:
+            raise ValueError(f"rebuild has {m.size} entries for {P} starts")
+        return m, m.ctypes.data_as(_abi._u8p)
+
+    @staticmethod
+    def _problems(problem, B):
+        if problem is None:
+            return None, None
+        p = np.ascontiguousarray(np.asarray(problem).reshape(-1), dtype=np.int32)
+        if p.size != B:
+            raise ValueError(f"problem has {p.size} entries for {B} candidates")
+        return p, p.ctypes.data_as(_abi._i32p)
+
+    def associate_multi(self, X0, rebuild=None, wait: bool = True):
+        """BuildProblem at X0[p] for every start p (X0 [P,7]) -> block counts [P,4] (None with wait=False).  rebuild (mask [P]):
+        re-associate only the flagged problems of the current set of P; the others keep their blocks."""
+        X0 = np.ascontiguousarray(np.atleast_2d(X0), dtype=np.float64)
+        P = X0.shape[0]
+        keep, m = self._mask(rebuild, P)
+        nb = np.zeros((P, 4), np.int64)
+        _check(self.lib, self.h, self.lib.stl_associate_multi(self.h, X0.ctypes.data_as(_dp), P, m,
+                                                              nb.ctypes.data_as(_abi._i64p) if wait else None))
+        self.n_blocks = None
+        self.n_problems = P
+        return nb if wait else None
+
+    def block_counts_multi(self) -> np.ndarray:
+        """Block counts [P,4] of the frozen set (waits for its association)."""
+        nb = np.zeros((_abi.STL_MAX_PROBLEMS, 4), np.int64)
+        _check(self.lib, self.h, self.lib.stl_block_counts_multi(self.h, nb.ctypes.data_as(_abi._i64p), _abi.STL_MAX_PROBLEMS))
+        return nb[: self.n_problems].copy()
+
+    def linearize_multi(self, X, problem=None) -> np.ndarray:
+        """Candidate b (X [B,7]) on problem problem[b] (None: B == P, candidate b on problem b) -> [B,62] (host)."""
+        X = np.ascontiguousarray(np.atleast_2d(X), dtype=np.float64)
+        B = X.shape[0]
+        keep, pp = self._problems(problem, B)
+        out = np.empty((B, _abi.STL_LIN_NSUMS), dtype=np.float64)
+        _check(self.lib, self.h, self.lib.stl_linearize_multi(self.h, X.ctypes.data_as(_dp), B, pp,
+                                                              out.ctypes.data_as(C.POINTER(_abi.LinSums))))
+        return out
+
+    def linearize_multi_device(self, X, d_out_ptr: int, problem=None, stream_ptr: int = 0):
+        X = np.ascontiguousarray(np.atleast_2d(X), dtype=np.float64)
+        keep, pp = self._problems(problem, X.shape[0])
+        _check(self.lib, self.h, self.lib.stl_linearize_multi_device(self.h, X.ctypes.data_as(_dp), X.shape[0], pp,
+                                                                     C.c_void_p(d_out_ptr), C.c_void_p(stream_ptr)))
+
+    def step_multi(self, X, rebuild=None) -> np.ndarray:
+        """One LM iteration for each start (X [P,7]): evaluation sums, BuildProblem at X[p] of the flagged problems (None: all,
+        a new set), linearisation of problem p at X[p] -> [P,74] (host)."""
+        X = np.ascontiguousarray(np.atleast_2d(X), dtype=np.float64)
+        P = X.shape[0]
+        keep, m = self._mask(rebuild, P)
+        out = np.empty((P, _abi.STL_STEP_NSUMS), dtype=np.float64)
+        _check(self.lib, self.h, self.lib.stl_step_multi(self.h, X.ctypes.data_as(_dp), P, m, out.ctypes.data_as(C.POINTER(_abi.StepSums))))
+        self.n_blocks = None
+        self.n_problems = P
+        return out
+
+    def step_multi_device(self, X, d_out_ptr: int, rebuild=None, stream_ptr: int = 0):
+        X = np.ascontiguousarray(np.atleast_2d(X), dtype=np.float64)
+        keep, m = self._mask(rebuild, X.shape[0])
+        _check(self.lib, self.h, self.lib.stl_step_multi_device(self.h, X.ctypes.data_as(_dp), X.shape[0], m,
+                                                                C.c_void_p(d_out_ptr), C.c_void_p(stream_ptr)))
+        self.n_blocks = None
+        self.n_problems = X.shape[0]
 
     def gpr_hyper(self):
         """(sigma, l) of the GPR blocks of the last association, block order -> [nG, 2]."""

@@ -40,6 +40,36 @@ constexpr int kLinThreads = 128;
 // All four walk the correspondences that carry a map point (the query list K1 wrote), keyframe by
 // keyframe; list slot = block slot = mp_off[f] + qi.  Traversals are warp-per-item, plane fits thread-per-item.
 // With the plane index only k_lm_plane_a and k_lm_plane_b run (and inside stl_step_batch K2a answers k_lm_knn_b's question).
+// grid (n_kf * sub, lanes): association lane blockIdx.y reads the K1 result at its workspace candidate slot, works in its own
+// scratch and writes the arrays of its problem (lm_lane) — a lane computes exactly what a single association computes.
+
+// Narrows the workspace, the scratch and the problem arrays to association lane blockIdx.y.
+// arg0: lane 0 takes its map from the kernel arguments (lm.lane0 == amap[0], lm_set_lanes) instead of a dependent load
+// (k_lm_plane_b reads amap: the argument copy costs it a register spill)
+__device__ __forceinline__ void lm_lane(const DevPack &pk, DevWork &wk, LmState &lm, bool arg0 = true) {
+    const int2 am = arg0 && blockIdx.y == 0 ? lm.lane0 : lm.amap[blockIdx.y];
+    const long long nk = pk.n_kp_total, F = pk.n_kf, nm = lm.n_slots;
+    const long long wc = am.x, wq = wc * nm;
+    wk.cand += wc;
+    wk.corr_kp += wc * nk; wk.corr_sp += wc * nk; wk.q_corr += wc * nk; wk.q_kpsp += wc * nk;
+    wk.n_corr += wc * F; wk.n_q += wc * F;
+    wk.nn_pos += wq; wk.nn_g2 += wq; wk.nb += wq * kMaxK; wk.nbx += wq; wk.nb_m += wq; wk.nb_last += wq;
+    const long long lo = (long long)blockIdx.y * nm;
+    lm.stage += lo; lm.plane_a += lo * 4; lm.nnb_pos += lo; lm.nbb += lo * kMaxK; lm.nbbx += lo; lm.nbb_m += lo; lm.nbb_last += lo;
+    const long long po = (long long)am.y * lm.slot_stride;
+    lm.slot_kf += po; lm.slot_kp += po; lm.flag2d += po; lm.type3d += po; lm.flag3d += po; lm.flagG += po;
+    lm.geo2d += po * 6; lm.geo3d += po * 9; lm.gpr_nb += po * kMaxK; lm.gpr_m += po;
+    lm.d_counts += am.y * 4;
+}
+
+// clears the flags and counts of the problem of every lane (re-association of part of a set)
+__global__ void k_lm_clear(LmState lm) {
+    const long long po = (long long)lm.amap[blockIdx.y].y * lm.slot_stride, n = lm.slot_stride, ptot = (long long)lm.P * n;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        lm.flags[po + i] = 0; lm.flags[ptot + po + i] = 0; lm.flags[2 * ptot + po + i] = 0; lm.flags[3 * ptot + po + i] = 0;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < 4) lm.d_counts[lm.amap[blockIdx.y].y * 4 + threadIdx.x] = 0;
+}
 
 __device__ __forceinline__ bool lm_frame_active(const DevWork &wk, const DevParams &pr, int f, int &nq) {
     nq = wk.n_q[f];
@@ -61,7 +91,8 @@ __device__ __forceinline__ void lm_map_point(const DevPack &pk, const DevKf &K, 
 // point (:213) or without a covisible observation (:259); neither test depends on the search, so
 // they come first here.
 __global__ void __launch_bounds__(kWarps * 32, STL_LM_MINB)
-k_lm_knn_a(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm) {
+k_lm_knn_a(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
+    lm_lane(pk, wk, lm);
     const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
@@ -100,10 +131,14 @@ k_lm_knn_a(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm) {
 
 // L2: plane at the scan point (iba_local.cpp:218-231) -> 3-D/2-D block; decides whether the 3-D search runs
 __global__ void __launch_bounds__(128)
-k_lm_plane_a(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm) {
+k_lm_plane_a(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
+    lm_lane(pk, wk, lm);
     const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
+    __shared__ int cnt[2];  // plane blocks, GPR blocks of this CTA (one pair of global atomics per CTA)
+    if (threadIdx.x < 2) cnt[threadIdx.x] = 0;
+    __syncthreads();
     const DevKf K = pk.kf[f];
     const ScanView S = make_view(pk, K);
     const bool from_index = pr.plane_index && !pr.use_gpr;  // then k_lm_knn_a did not run: the covisibility test is made here
@@ -135,16 +170,19 @@ k_lm_plane_a(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm)
             double *g = lm.geo2d + cs * 6;
             g[0] = cx; g[1] = cy; g[2] = cz; g[3] = po.n.x; g[4] = po.n.y; g[5] = po.n.z;
             lm.flag2d[cs] = 1;
+            atomicAdd(&cnt[0], 1);
         } else if (pr.use_gpr) {
             // non-planar neighbourhood: IBA_GPRFactor over the neighbour points (iba_local.cpp:272-280);
             // the list is copied because the evaluation workspace is reused by later calls
             for (int t = 0; t < kMaxK; ++t) lm.gpr_nb[slot * kMaxK + t] = wk.nb[slot * kMaxK + t];
             lm.gpr_m[slot] = po.m;
-            lm.slot_mp[cs] = (int)slot;
             lm.flagG[cs] = 1;
+            atomicAdd(&cnt[1], 1);
         }
         lm.stage[slot] = 1;
     }
+    __syncthreads();
+    if (threadIdx.x < 2 && cnt[threadIdx.x] > 0) atomicAdd(lm.d_counts + 3 * threadIdx.x, cnt[threadIdx.x]);  // [0] plane, [3] GPR
 }
 
 // L3: map point -> LiDAR frame with the association extrinsic, 1-NN gate, neighbourhood of that point
@@ -157,8 +195,10 @@ k_lm_plane_a(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm)
 // whose query is not settled that way (no evaluation at hand, near-equidistant neighbours) take turns on the warp-wide
 // exact search, seeded with h or with the associated scan point.
 __global__ void __launch_bounds__(kWarps * 32, STL_LM_MINB)
-k_lm_knn_b(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm, const uint32_t *__restrict__ nn_hint,
-           const float *__restrict__ nn_g2) {
+k_lm_knn_b(const DevPack pk, DevWork wk, const DevParams pr, LmState lm, const bool hints, const bool cert) {
+    lm_lane(pk, wk, lm);
+    const uint32_t *__restrict__ nn_hint = hints ? wk.nn_pos : nullptr;
+    const float *__restrict__ nn_g2 = hints && cert ? wk.nn_g2 : nullptr;
     const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
@@ -273,7 +313,8 @@ __device__ __forceinline__ bool block3d_geometry(const DevPack &pk, const DevPar
 }
 
 __global__ void __launch_bounds__(128)
-k_lm_plane_b(const DevPack pk, const DevWork wk, const DevParams pr, LmState lm) {
+k_lm_plane_b(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
+    lm_lane(pk, wk, lm, false);
     const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
@@ -392,19 +433,32 @@ __device__ __forceinline__ void put_head(const BlockOut &o, long long blk, int t
     o.type[blk] = type; o.kf[blk] = kf; o.kp[blk] = (int32_t)kp; o.nres[blk] = nres;
 }
 
-// grid (chunks, B).  The 3-D/3-D blocks are walked over ALL query slots (no compacted list: the work per block is light, and
-// the association then has no select on the way to the linearisation).
-// WB (stl_eval_blocks) numbers the blocks and therefore walks the compacted list.
+// Start of problem p's run in a concatenated block list: the sum of the counts `which` of problems 0..p-1 (warp 0 of the CTA;
+// integer sums, so the order does not matter)
+__device__ __forceinline__ void lm_list_start(const LmState &lm, int p, int which, int *out) {
+    if (threadIdx.x >= 32) return;
+    int s = 0;
+    for (int q = threadIdx.x; q < p; q += 32) s += lm.d_counts[q * 4 + which];
+    for (int o = 16; o; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+    if (threadIdx.x == 0) *out = s;
+}
+
+// grid (chunks, B): candidate blockIdx.y on problem cprob[blockIdx.y].  The 3-D/3-D blocks are walked over ALL query slots of
+// that problem (no compacted list: the work per block is light, and the association then has no select on the way to the
+// linearisation).  WB (stl_eval_blocks) numbers the blocks and therefore walks the compacted list (problem 0).
 template <bool WB>
 __global__ void __launch_bounds__(kLinThreads)
-k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, double *__restrict__ partial,
-            int partial_stride, const BlockOut bo) {
+k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, const int *__restrict__ cprob,
+            double *__restrict__ partial, int partial_stride, const BlockOut bo) {
     __shared__ LmCand c;
+    __shared__ int list0;
+    const int prob = cprob ? cprob[blockIdx.y] : 0;
     {
         const double *src = reinterpret_cast<const double *>(cands + blockIdx.y);
         double *dst = reinterpret_cast<double *>(&c);
         for (int i = threadIdx.x; i < (int)(sizeof(LmCand) / 8); i += kLinThreads) dst[i] = src[i];
     }
+    lm_list_start(lm, prob, 0, &list0);
     __syncthreads();
     const F7 *cR = reinterpret_cast<const F7 *>(c.R), *ct = reinterpret_cast<const F7 *>(c.t);
     const F7 *cRlc = reinterpret_cast<const F7 *>(c.Rlc), *ctlc = reinterpret_cast<const F7 *>(c.tlc);
@@ -415,11 +469,13 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
     const int C = pk.n_covis;
     const int stride = gridDim.x * kLinThreads, t0 = blockIdx.x * kLinThreads + threadIdx.x;
 
-    // block counts live on the device (written by the selects of the association on this stream): no host round trip
-    const int n2d = lm.d_counts[0];
+    // block counts live on the device (written by the association kernels on this stream): no host round trip
+    const int *counts = lm.d_counts + prob * 4;
+    const int n2d = counts[0];
+    const int *idx2d = lm.idx2d + list0;
     // ---- 3-D/2-D blocks: IBA_PlaneFactor (IBACalib2.hpp:152-184)
     for (int it = t0; it < n2d; it += stride) {
-        const int slot = lm.idx2d[it];
+        const int slot = idx2d[it];  // global slot (problem offset included)
         const int f = lm.slot_kf[slot];
         const uint32_t kp = lm.slot_kp[slot];
         const DevKf &K = pk.kf[f];
@@ -484,7 +540,10 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
     // slots per round, queues the flagged ones in shared memory and evaluates 32 queued blocks at a time (the tail at the end): the
     // lanes stay full although only half of the slots carry a block, and nothing outside this kernel has to compact the list.
     // Which thread sums which block depends on the flags alone, never on the batch size.
-    const long long n3 = WB ? (long long)lm.d_counts[1] : lm.max_blocks;
+    const long long n3 = WB ? (long long)counts[1] : lm.max_blocks;
+    const long long po = (long long)prob * lm.slot_stride;  // the 3-D walk is in problem-local slots
+    const uint8_t *flag3d = lm.flag3d + po, *type3d = lm.type3d + po;
+    const double *geo3d = lm.geo3d + po * 9;
     __shared__ int q3[kLinThreads / 32][64];
     const int lane3 = threadIdx.x & 31, warp3 = threadIdx.x >> 5;
     int qlen = 0;                                                    // warp-uniform
@@ -498,7 +557,7 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             const bool more = base < n3;
             if (more) {
                 const long long sl = base + lane3;
-                const bool on = sl < n3 && lm.flag3d[sl];
+                const bool on = sl < n3 && flag3d[sl];
                 const unsigned mask = __ballot_sync(0xffffffffu, on);
                 if (on) q3[warp3][qlen + __popc(mask & ((1u << lane3) - 1))] = (int)sl;
                 qlen += __popc(mask);
@@ -517,8 +576,8 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             if (mine < 0) continue;
             slot = mine;
         }
-        const double *g = lm.geo3d + slot * 9;
-        const int type = lm.type3d[slot];
+        const double *g = geo3d + slot * 9;
+        const int type = type3d[slot];
         const F7 Ms[3] = {cs7 * g[0], cs7 * g[1], cs7 * g[2]};  // MapPoint * s
         F7 M[3];
         mv3(cRlc, Ms, M);
@@ -536,7 +595,7 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             if (WB) {
                 const long long blk = (long long)n2d + it;
                 put_row(bo, blk, 0, d[0]); put_row(bo, blk, 1, d[1]); put_row(bo, blk, 2, d[2]);
-                put_head(bo, blk, 1, lm.slot_kf[slot], lm.slot_kp[slot], 3);
+                put_head(bo, blk, 1, lm.slot_kf[po + slot], lm.slot_kp[po + slot], 3);
             }
         } else {
             const F7 e = (d[0] * g[6] + d[1] * g[7]) + d[2] * g[8];
@@ -547,7 +606,7 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             if (WB) {
                 const long long blk = (long long)n2d + it;
                 put_row(bo, blk, 0, e);
-                put_head(bo, blk, 2, lm.slot_kf[slot], lm.slot_kp[slot], 1);
+                put_head(bo, blk, 2, lm.slot_kf[po + slot], lm.slot_kp[po + slot], 1);
             }
         }
         A.v[0] += 0.5 * rho0;
@@ -637,28 +696,32 @@ __device__ __forceinline__ D7 shfl7(const D7 &x, int src) {
 // grid (chunks, B), one warp per CTA
 template <bool WB>
 __global__ void __launch_bounds__(32)
-k_linearize_gpr(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, double *__restrict__ partial,
-                int partial_stride, int partial_off, const BlockOut bo) {
+k_linearize_gpr(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, const int *__restrict__ cprob,
+                double *__restrict__ partial, int partial_stride, int partial_off, const BlockOut bo) {
     __shared__ GprSmem S;
     __shared__ LmCand c;
+    __shared__ int list0;
     const int lane = threadIdx.x;
+    const int prob = cprob ? cprob[blockIdx.y] : 0;
     {
         const double *src = reinterpret_cast<const double *>(cands + blockIdx.y);
         double *dst = reinterpret_cast<double *>(&c);
         for (int i = lane; i < (int)(sizeof(LmCand) / 8); i += 32) dst[i] = src[i];
     }
+    lm_list_start(lm, prob, 3, &list0);
     __syncwarp();
+    const int *counts = lm.d_counts + prob * 4;
     Acc A;
 #pragma unroll
     for (int i = 0; i < kLinVals; ++i) A.v[i] = 0.0;
     const int C = pk.n_covis;
-    const int nG = lm.d_counts[3];
+    const int nG = counts[3];
     for (int it = blockIdx.x; it < nG; it += gridDim.x) {
-        const int cs = lm.idxG[it];
+        const int cs = lm.idxG[list0 + it];  // global slot
         const int f = lm.slot_kf[cs];
         const uint32_t kp = lm.slot_kp[cs];
-        const long long gblk = (long long)lm.d_counts[0] + lm.d_counts[1] + it;  // block index in stl_eval_blocks order
-        const long long ms = lm.slot_mp[cs];
+        const long long gblk = (long long)counts[0] + counts[1] + it;  // block index in stl_eval_blocks order
+        const long long ms = cs;
         const int n = lm.gpr_m[ms];
         const DevKf &K = pk.kf[f];
         const double fx = K.fx, fy = K.fy, cx = K.cx, cy = K.cy;
@@ -821,101 +884,155 @@ template <class T> void dfree(T *&p) { if (p) { cudaFree(p); p = nullptr; } }
 
 void lm_free(LmState &lm) {
     dfree(lm.slot_kf); dfree(lm.slot_kp); dfree(lm.flags); dfree(lm.geo2d); dfree(lm.geo3d);
-    dfree(lm.idxG); dfree(lm.slot_mp); dfree(lm.gpr_nb); dfree(lm.gpr_m); dfree(lm.gpr_hyper);
-    dfree(lm.stage); dfree(lm.plane_a); dfree(lm.nnb_pos); dfree(lm.nbb); dfree(lm.nbbx); dfree(lm.nbb_m); dfree(lm.nbb_last);
-    dfree(lm.idx2d); dfree(lm.idx3d); dfree(lm.d_tmp); dfree(lm.partial); dfree(lm.d_cand);
+    dfree(lm.idxG); dfree(lm.gpr_nb); dfree(lm.gpr_m); dfree(lm.gpr_hyper);
+    dfree(lm.amap); dfree(lm.stage); dfree(lm.plane_a); dfree(lm.nnb_pos); dfree(lm.nbb); dfree(lm.nbbx); dfree(lm.nbb_m); dfree(lm.nbb_last);
+    dfree(lm.idx2d); dfree(lm.idx3d); dfree(lm.d_sel); dfree(lm.d_tmp); dfree(lm.partial); dfree(lm.d_cand);
     if (lm.h_cand) cudaFreeHost(lm.h_cand);
     if (lm.h_counts) cudaFreeHost(lm.h_counts);
+    if (lm.h_amap) cudaFreeHost(lm.h_amap);
+    delete[] lm.n_blocks;
     if (lm.h2d_done) cudaEventDestroy(lm.h2d_done);
     if (lm.counts_done) cudaEventDestroy(lm.counts_done);
+    if (lm.amap_done) cudaEventDestroy(lm.amap_done);
     lm = LmState();
 }
 
-// Enqueues BuildProblem on `st` and returns without waiting: the block counts stay on the device
-// (d_counts: plane, 3-D, point-to-point, GPR), where the linearisation kernels read them; a copy lands
-// in pinned host memory behind `counts_done` for callers that want the numbers (lm_block_counts).
-// The buffers of an association (sized by the pack): allocated on the first association, or ahead of it by a caller that
-// wants LmState::nnb_pos / nbb_m filled by K2a.
-cudaError_t lm_reserve(const DevPack &pk, const DevParams &pr, LmState &lm, cudaStream_t st) {
+// The buffers of a set of P problems with `lanes` association lanes (sized by the pack): allocated by the first association, or
+// ahead of it by a caller that wants LmState::nnb_pos / nbb_m filled by K2a.  The per-problem arrays and the lane scratch are
+// high-water marks: reallocated only when more problems / lanes are asked for than they hold (a driver that alternates single
+// steps and sets pays no allocation per switch); a failure frees everything (no half-built set).
+cudaError_t lm_reserve(const DevPack &pk, const DevParams &pr, LmState &lm, int P, int lanes, cudaStream_t st) {
     cudaError_t e;
-#define TRY(x) do { e = (x); if (e != cudaSuccess) return e; } while (0)
+#define TRY(x) do { e = (x); if (e != cudaSuccess) { lm_free(lm); return e; } } while (0)
     // block slots = query slots: one per map-point-carrying keypoint (a twelfth of the keypoints at the KITTI-00 shape), so the
     // flag arrays the selects compact, and the per-block geometry, are that much smaller than one-per-keypoint arrays
     const long long ns = pk.n_mp_total > 0 ? pk.n_mp_total : 1;
-    if (lm.n_slots != ns) {
-        lm_free(lm);  // n_slots stays 0 until every allocation below succeeded: a failure midway starts over next time
-        TRY(cudaMalloc(&lm.slot_kf, 4 * ns)); TRY(cudaMalloc(&lm.slot_kp, 4 * ns));
-        // the four per-slot flag arrays and the counters are one allocation: one memset per association
-        const long long nsa = (ns + 15) / 16 * 16;
-        lm.flags_bytes = (size_t)(4 * nsa + 16);
+    if (lm.n_slots != ns || lm.P_cap < P) {
+        lm_free(lm);  // P_cap stays 0 until every allocation below succeeded: a failure midway starts over next time
+        const long long nsa = (ns + 15) / 16 * 16, n = nsa * P;
+        lm.slot_stride = nsa;
+        TRY(cudaMalloc(&lm.slot_kf, 4 * n)); TRY(cudaMalloc(&lm.slot_kp, 4 * n));
+        // the four per-slot flag arrays and the counters are one allocation: one memset per new set
+        lm.flags_bytes = (size_t)(4 * n + 16 * P);
         TRY(cudaMalloc(&lm.flags, lm.flags_bytes));
-        lm.flag2d = lm.flags; lm.type3d = lm.flags + nsa; lm.flag3d = lm.flags + 2 * nsa; lm.flagG = lm.flags + 3 * nsa;
-        lm.d_counts = reinterpret_cast<int *>(lm.flags + 4 * nsa);
-        TRY(cudaMalloc(&lm.geo2d, 48 * ns)); TRY(cudaMalloc(&lm.geo3d, 72 * ns));
-        TRY(cudaMalloc(&lm.idx2d, 4 * ns)); TRY(cudaMalloc(&lm.idx3d, 4 * ns));
-        const long long nm = pk.n_mp_total > 0 ? pk.n_mp_total : 1;
-        TRY(cudaMalloc(&lm.stage, nm)); TRY(cudaMalloc(&lm.plane_a, 32 * nm)); TRY(cudaMalloc(&lm.nnb_pos, 4 * nm));
-        TRY(cudaMalloc(&lm.nbb, 4 * nm * kMaxK)); TRY(cudaMalloc(&lm.nbbx, sizeof(float4) * nm * kMaxK)); lm.nbbx_stride = (long long)nm; TRY(cudaMalloc(&lm.nbb_m, 4 * nm)); TRY(cudaMalloc(&lm.nbb_last, 8 * nm));
-        TRY(cudaMalloc(&lm.idxG, 4 * ns)); TRY(cudaMalloc(&lm.slot_mp, 4 * ns));
-        if (pr.use_gpr) { TRY(cudaMalloc(&lm.gpr_nb, 4 * nm * kMaxK)); TRY(cudaMalloc(&lm.gpr_m, 4 * nm)); }
+        lm.flag2d = lm.flags; lm.type3d = lm.flags + n; lm.flag3d = lm.flags + 2 * n; lm.flagG = lm.flags + 3 * n;
+        lm.d_counts = reinterpret_cast<int *>(lm.flags + 4 * n);
+        TRY(cudaMalloc(&lm.geo2d, 48 * n)); TRY(cudaMalloc(&lm.geo3d, 72 * n));
+        TRY(cudaMalloc(&lm.idx2d, 4 * n)); TRY(cudaMalloc(&lm.idx3d, 4 * ns)); TRY(cudaMalloc(&lm.idxG, 4 * n));
+        if (pr.use_gpr) { TRY(cudaMalloc(&lm.gpr_nb, 4 * n * kMaxK)); TRY(cudaMalloc(&lm.gpr_m, 4 * n)); }
+        TRY(cudaMalloc(&lm.d_sel, 8));
         size_t tb = 0;
         cub::CountingInputIterator<int> it(0);
-        TRY(cub::DeviceSelect::Flagged(nullptr, tb, it, lm.flag2d, lm.idx2d, lm.d_counts, (int)ns, st));
+        TRY(cub::DeviceSelect::Flagged(nullptr, tb, it, lm.flag2d, lm.idx2d, lm.d_sel, (int)n, st));
         lm.tmp_bytes = tb;
         TRY(cudaMalloc(&lm.d_tmp, tb));
-        TRY(cudaMallocHost(&lm.h_counts, 16));
+        TRY(cudaMallocHost(&lm.h_counts, 16 * (size_t)P));
+        lm.n_blocks = new long long[4 * (size_t)P]();
         TRY(cudaEventCreateWithFlags(&lm.counts_done, cudaEventDisableTiming));
+        TRY(cudaEventCreateWithFlags(&lm.amap_done, cudaEventDisableTiming));
         lm.n_slots = ns;
-        lm.max_blocks = nm;
+        lm.max_blocks = ns;
+        lm.P_cap = P;
+    }
+    if (lanes > lm.lane_cap) {
+        dfree(lm.amap); dfree(lm.stage); dfree(lm.plane_a); dfree(lm.nnb_pos); dfree(lm.nbb); dfree(lm.nbbx); dfree(lm.nbb_m); dfree(lm.nbb_last);
+        if (lm.h_amap) cudaFreeHost(lm.h_amap);
+        lm.h_amap = nullptr;
+        lm.lane_cap = 0;
+        const long long nm = ns * lanes;
+        TRY(cudaMalloc(&lm.amap, sizeof(int2) * lanes)); TRY(cudaMallocHost(&lm.h_amap, sizeof(int2) * lanes));
+        TRY(cudaMalloc(&lm.stage, nm)); TRY(cudaMalloc(&lm.plane_a, 32 * nm)); TRY(cudaMalloc(&lm.nnb_pos, 4 * nm));
+        TRY(cudaMalloc(&lm.nbb, 4 * nm * kMaxK)); TRY(cudaMalloc(&lm.nbbx, sizeof(float4) * nm * kMaxK)); lm.nbbx_stride = nm;
+        TRY(cudaMalloc(&lm.nbb_m, 4 * nm)); TRY(cudaMalloc(&lm.nbb_last, 8 * nm));
+        lm.lane_cap = lanes;
+        // the single association's lane: workspace slot 0, problem 0 (what K2a's folded 1-NN assumes); lm_set_lanes skips the
+        // copy while the first lane stays what h_amap[0] says is on the device
+        lm.h_amap[0] = make_int2(0, 0);
+        TRY(cudaMemcpy(lm.amap, lm.h_amap, sizeof(int2), cudaMemcpyHostToDevice));
     }
 #undef TRY
     return cudaSuccess;
 }
 
-cudaError_t lm_associate(const DevPack &pk, const DevWork &wk, const DevParams &pr, LmState &lm, cudaStream_t st, const uint32_t *nn_hint,
-                         const float *nn_g2, int part, bool nn_folded, bool defer_counts) {
+cudaError_t lm_begin(const DevPack &pk, const DevParams &pr, LmState &lm, int P, bool partial, int lanes, cudaStream_t st) {
+    cudaError_t e = lm_reserve(pk, pr, lm, P, lanes, st);
+    if (e != cudaSuccess) return e;
+    lm.ready = false;
+    lm.clear_lanes = partial;
+    if (!partial) {  // the flag arrays of a set of P are packed for P (the allocation holds P_cap): one memset of what P uses
+        const long long n = lm.slot_stride * P;
+        lm.P = P;
+        lm.flag2d = lm.flags; lm.type3d = lm.flags + n; lm.flag3d = lm.flags + 2 * n; lm.flagG = lm.flags + 3 * n;
+        lm.d_counts = reinterpret_cast<int *>(lm.flags + 4 * n);
+        e = cudaMemsetAsync(lm.flags, 0, (size_t)(4 * n + 16 * P), st);
+    }
+    return e;
+}
+
+cudaError_t lm_set_lanes(LmState &lm, const int2 *lanes, int n, cudaStream_t st) {
+    if (n > lm.lane_cap) return cudaErrorInvalidValue;
+    lm.lane0 = lanes[0];
+    if (n == 1 && lanes[0].x == lm.h_amap[0].x && lanes[0].y == lm.h_amap[0].y) return cudaSuccess;  // already on the device
+    cudaError_t e = cudaEventSynchronize(lm.amap_done);
+    if (e != cudaSuccess) return e;
+    memcpy(lm.h_amap, lanes, sizeof(int2) * n);
+    e = cudaMemcpyAsync(lm.amap, lm.h_amap, sizeof(int2) * n, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaEventRecord(lm.amap_done, st);
+    return e;
+}
+
+// Enqueues BuildProblem of n lanes on `st` and returns without waiting: the block counts stay on the device (d_counts: plane,
+// 3-D, point-to-point, GPR per problem), where the linearisation kernels read them; lm_copy_counts puts a copy in pinned host
+// memory behind `counts_done` for callers that want the numbers (lm_block_counts).
+cudaError_t lm_associate(const DevPack &pk, const DevWork &wk, const DevParams &pr, LmState &lm, int n, cudaStream_t st, bool hints, bool cert,
+                         int part, bool nn_folded) {
     cudaError_t e;
 #define TRY(x) do { e = (x); if (e != cudaSuccess) return e; } while (0)
-    const long long ns = pk.n_mp_total > 0 ? pk.n_mp_total : 1;
-    TRY(lm_reserve(pk, pr, lm, st));
+    const dim3 grid((unsigned)(pk.n_kf * wk.sub), (unsigned)n);
     if (part != 2) {
-    lm.ready = false;
-    lm.sub = wk.sub;
-    TRY(cudaMemsetAsync(lm.flags, 0, lm.flags_bytes, st));
-    if (!(pr.plane_index && !pr.use_gpr))  // with the plane index there is no neighbourhood to search at the scan point
-        k_lm_knn_a<<<(unsigned)(pk.n_kf * lm.sub), kWarps * 32, 0, st>>>(pk, wk, pr, lm);
-    k_lm_plane_a<<<(unsigned)(pk.n_kf * lm.sub), 128, 0, st>>>(pk, wk, pr, lm);
-    TRY(cudaGetLastError());
-    {   // the 3-D/2-D blocks are complete: their dense list (the linearisation walks it) needs nothing of the 3-D search
-        cub::CountingInputIterator<int> it2(0);
-        size_t tb2 = lm.tmp_bytes;
-        TRY(cub::DeviceSelect::Flagged(lm.d_tmp, tb2, it2, lm.flag2d, lm.idx2d, lm.d_counts, (int)ns, st));
-    }
+        lm.ready = false;
+        lm.sub = wk.sub;
+        if (lm.clear_lanes) k_lm_clear<<<dim3((unsigned)((lm.slot_stride + 1023) / 1024 < 64 ? (lm.slot_stride + 1023) / 1024 : 64), (unsigned)n), 256, 0, st>>>(lm);
+        if (!(pr.plane_index && !pr.use_gpr))  // with the plane index there is no neighbourhood to search at the scan point
+            k_lm_knn_a<<<grid, kWarps * 32, 0, st>>>(pk, wk, pr, lm);
+        k_lm_plane_a<<<grid, 128, 0, st>>>(pk, wk, pr, lm);
+        TRY(cudaGetLastError());
     }
     if (part == 1) return cudaSuccess;
-    if (!nn_folded) k_lm_knn_b<<<(unsigned)(pk.n_kf * lm.sub), kWarps * 32, 0, st>>>(pk, wk, pr, lm, nn_hint, nn_g2);  // else K2a has filled nnb_pos / nbb_m
-    k_lm_plane_b<<<(unsigned)(pk.n_kf * lm.sub), 128, 0, st>>>(pk, wk, pr, lm);
+    if (!nn_folded) k_lm_knn_b<<<grid, kWarps * 32, 0, st>>>(pk, wk, pr, lm, hints, cert);  // else K2a has filled nnb_pos / nbb_m
+    k_lm_plane_b<<<grid, 128, 0, st>>>(pk, wk, pr, lm);
     TRY(cudaGetLastError());
+#undef TRY
+    return cudaSuccess;
+}
+
+// the 3-D/2-D blocks are complete after k_lm_plane_a: their dense list (the linearisation walks it) needs nothing of the 3-D
+// search.  ONE select over the flags of all P problems: each problem's run comes out in slot order, and a problem that was not
+// re-associated gets back exactly the run it had
+cudaError_t lm_compact2d(LmState &lm, cudaStream_t st) {
     cub::CountingInputIterator<int> it(0);
+    size_t tb = lm.tmp_bytes;
+    return cub::DeviceSelect::Flagged(lm.d_tmp, tb, it, lm.flag2d, lm.idx2d, lm.d_sel, (int)(lm.slot_stride * lm.P), st);
+}
+
+cudaError_t lm_finish_associate(LmState &lm, bool use_gpr, cudaStream_t st) {
     // the 3-D/3-D blocks are counted by k_lm_plane_b and walked slot by slot by the linearisation: their dense list is only
     // built for stl_eval_blocks (lm_compact3d)
     lm.idx3d_valid = false;
-    if (pr.use_gpr) {
+    if (use_gpr) {
+        cub::CountingInputIterator<int> it(0);
         size_t tb = lm.tmp_bytes;
-        TRY(cub::DeviceSelect::Flagged(lm.d_tmp, tb, it, lm.flagG, lm.idxG, lm.d_counts + 3, (int)ns, st));
-    }
-    TRY(cudaGetLastError());
-    if (!defer_counts) {
-        TRY(cudaMemcpyAsync(lm.h_counts, lm.d_counts, 16, cudaMemcpyDeviceToHost, st));
-        TRY(cudaEventRecord(lm.counts_done, st));
+        const cudaError_t e = cub::DeviceSelect::Flagged(lm.d_tmp, tb, it, lm.flagG, lm.idxG, lm.d_sel + 1, (int)(lm.slot_stride * lm.P), st);
+        if (e != cudaSuccess) return e;
     }
     lm.counts_valid = false;
-    lm.use_gpr = pr.use_gpr != 0;
+    lm.use_gpr = use_gpr;
+    lm.clear_lanes = false;
     lm.ready = true;
     return cudaSuccess;
 }
 
-// Dense list of the 3-D/3-D blocks (slot order), for the numbered walk of stl_eval_blocks.
+// Dense list of the 3-D/3-D blocks of problem 0 (slot order), for the numbered walk of stl_eval_blocks.
 cudaError_t lm_compact3d(const DevPack &pk, LmState &lm, cudaStream_t st) {
     if (lm.idx3d_valid) return cudaSuccess;
     const long long ns = pk.n_mp_total > 0 ? pk.n_mp_total : 1;
@@ -926,10 +1043,9 @@ cudaError_t lm_compact3d(const DevPack &pk, LmState &lm, cudaStream_t st) {
     return e;
 }
 
-// The read-back of the block counts, for a caller that deferred it (lm_associate with defer_counts) to get it out of the
-// way of the linearisation that follows the association on the same stream.
+// The read-back of the block counts of every problem of the set.
 cudaError_t lm_copy_counts(LmState &lm, cudaStream_t st) {
-    cudaError_t e = cudaMemcpyAsync(lm.h_counts, lm.d_counts, 16, cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaMemcpyAsync(lm.h_counts, lm.d_counts, 16 * (size_t)lm.P, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaEventRecord(lm.counts_done, st);
     return e;
 }
@@ -940,26 +1056,26 @@ cudaError_t lm_block_counts(LmState &lm) {
     if (lm.counts_valid) return cudaSuccess;
     cudaError_t e = cudaEventSynchronize(lm.counts_done);
     if (e != cudaSuccess) return e;
-    const int *h = lm.h_counts;
-    lm.n2d = h[0]; lm.n3d = h[1]; lm.nG = lm.use_gpr ? h[3] : 0;
-    const int npt = h[2];
-    lm.n_blocks[0] = lm.n2d; lm.n_blocks[1] = npt; lm.n_blocks[2] = lm.n3d - npt; lm.n_blocks[3] = lm.nG;
+    for (int p = 0; p < lm.P; ++p) {
+        const int *h = lm.h_counts + 4 * p;
+        long long *o = lm.n_blocks + 4 * p;
+        o[0] = h[0]; o[1] = h[2]; o[2] = h[1] - h[2]; o[3] = lm.use_gpr ? h[3] : 0;
+    }
     lm.counts_valid = true;
     return cudaSuccess;
 }
 
 namespace {
-// training data of GPR::fit for GPR block `it`: neighbour j -> (u, v, depth) with the association extrinsic
-// (IBACalib2.hpp:449-457: pt = R p + t; uv = fx pt0 / pt2 + cx, fy pt1 / pt2 + cy), fp64, one thread per neighbour
-__global__ void k_gpr_train(const DevPack pk, const DevWork wk, const LmState lm, double *__restrict__ out /*[nG][32][3]*/, int *__restrict__ out_n) {
+// training data of GPR::fit for GPR block `it` of a problem (list run from l0, nG blocks): neighbour j -> (u, v, depth) with the
+// association extrinsic (IBACalib2.hpp:449-457: pt = R p + t; uv = fx pt0 / pt2 + cx, fy pt1 / pt2 + cy), fp64, one thread per neighbour
+__global__ void k_gpr_train(const DevPack pk, const DevCand *__restrict__ c0, const LmState lm, int l0, double *__restrict__ out /*[nG][32][3]*/,
+                            int *__restrict__ out_n) {
     const int it = blockIdx.x, lane = threadIdx.x;
-    if (it >= lm.d_counts[3]) return;
-    const int cs = lm.idxG[it];
-    const int f = lm.slot_kf[cs];
-    const long long ms = lm.slot_mp[cs];
+    const long long ms = lm.idxG[l0 + it];  // global slot
+    const int f = lm.slot_kf[ms];
     const int n = lm.gpr_m[ms];
     const DevKf &K = pk.kf[f];
-    const DevCand &c = wk.cand[0];
+    const DevCand &c = *c0;
     if (lane == 0) out_n[it] = n;
     double u = 0, v = 0, z = 0;
     if (lane < n) {
@@ -973,29 +1089,30 @@ __global__ void k_gpr_train(const DevPack pk, const DevWork wk, const LmState lm
     double *o = out + ((long long)it * kMaxK + lane) * 3;
     o[0] = u; o[1] = v; o[2] = z;
 }
-__global__ void k_gpr_scatter_hyper(const LmState lm, const double *__restrict__ fitted /*[nG][2]*/, double *__restrict__ hyper) {
+__global__ void k_gpr_scatter_hyper(const LmState lm, int l0, int nG, const double *__restrict__ fitted /*[nG][2]*/, double *__restrict__ hyper) {
     const int it = blockIdx.x * blockDim.x + threadIdx.x;
-    if (it >= lm.d_counts[3]) return;
-    const long long ms = lm.slot_mp[lm.idxG[it]];
+    if (it >= nG) return;
+    const long long ms = lm.idxG[l0 + it];
     hyper[ms * 2] = fitted[it * 2];
     hyper[ms * 2 + 1] = fitted[it * 2 + 1];
 }
-__global__ void k_gpr_gather_hyper(const LmState lm, const DevParams pr, double *__restrict__ out /*[nG][2]*/) {
+__global__ void k_gpr_gather_hyper(const LmState lm, const DevParams pr, int nG, double *__restrict__ out /*[nG][2]*/) {
     const int it = blockIdx.x * blockDim.x + threadIdx.x;
-    if (it >= lm.d_counts[3]) return;
-    const long long ms = lm.slot_mp[lm.idxG[it]];
+    if (it >= nG) return;
+    const long long ms = lm.idxG[it];  // problem 0: its run starts the list
     out[it * 2] = lm.gpr_hyper ? lm.gpr_hyper[ms * 2] : pr.gpr_sigma;
     out[it * 2 + 1] = lm.gpr_hyper ? lm.gpr_hyper[ms * 2 + 1] : pr.gpr_l;
 }
 }  // namespace
 
-cudaError_t lm_fit_gpr_hyper(const DevPack &pk, const DevWork &wk, const DevParams &pr, LmState &lm, cudaStream_t st, int flavour) {
+cudaError_t lm_fit_gpr_hyper(const DevPack &pk, const DevCand *c0, const DevParams &pr, LmState &lm, int prob, cudaStream_t st, int flavour) {
     cudaError_t e = lm_block_counts(lm);
     if (e != cudaSuccess) return e;
-    const int nG = lm.nG;
-    const long long nm = pk.n_mp_total > 0 ? pk.n_mp_total : 1;
+    const int nG = (int)lm.n_blocks[4 * prob + 3];
+    int l0 = 0;
+    for (int q = 0; q < prob; ++q) l0 += (int)lm.n_blocks[4 * q + 3];
     if (!lm.gpr_hyper) {
-        e = cudaMalloc(&lm.gpr_hyper, 16 * nm);
+        e = cudaMalloc(&lm.gpr_hyper, 16 * lm.slot_stride * lm.P_cap);
         if (e != cudaSuccess) return e;
     }
     if (nG == 0) return cudaSuccess;
@@ -1007,7 +1124,7 @@ cudaError_t lm_fit_gpr_hyper(const DevPack &pk, const DevWork &wk, const DevPara
     if (e == cudaSuccess) e = cudaMalloc(&d_n, 4 * (size_t)nG);
     if (e == cudaSuccess) e = cudaMalloc(&d_fit, 16 * (size_t)nG);
     if (e == cudaSuccess) {
-        k_gpr_train<<<nG, kMaxK, 0, st>>>(pk, wk, lm, d_train, d_n);
+        k_gpr_train<<<nG, kMaxK, 0, st>>>(pk, c0, lm, l0, d_train, d_n);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(h_train.data(), d_train, 8 * h_train.size(), cudaMemcpyDeviceToHost, st);
@@ -1030,7 +1147,7 @@ cudaError_t lm_fit_gpr_hyper(const DevPack &pk, const DevWork &wk, const DevPara
         e = cudaMemcpyAsync(d_fit, h_fit.data(), 16 * (size_t)nG, cudaMemcpyHostToDevice, st);
     }
     if (e == cudaSuccess) {
-        k_gpr_scatter_hyper<<<(nG + 127) / 128, 128, 0, st>>>(lm, d_fit, lm.gpr_hyper);
+        k_gpr_scatter_hyper<<<(nG + 127) / 128, 128, 0, st>>>(lm, l0, nG, d_fit, lm.gpr_hyper);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
@@ -1040,46 +1157,53 @@ cudaError_t lm_fit_gpr_hyper(const DevPack &pk, const DevWork &wk, const DevPara
 
 cudaError_t lm_get_gpr_hyper(const DevParams &pr, LmState &lm, double *out, cudaStream_t st) {
     cudaError_t e = lm_block_counts(lm);
-    if (e != cudaSuccess || lm.nG == 0) return e;
+    const int nG = (int)lm.n_blocks[3];
+    if (e != cudaSuccess || nG == 0) return e;
     double *d = nullptr;
-    e = cudaMalloc(&d, 16 * (size_t)lm.nG);
+    e = cudaMalloc(&d, 16 * (size_t)nG);
     if (e != cudaSuccess) return e;
-    k_gpr_gather_hyper<<<(lm.nG + 127) / 128, 128, 0, st>>>(lm, pr, d);
+    k_gpr_gather_hyper<<<(nG + 127) / 128, 128, 0, st>>>(lm, pr, nG, d);
     e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d, 16 * (size_t)lm.nG, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d, 16 * (size_t)nG, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     cudaFree(d);
     return e;
 }
 
-// Sim3Exp / SE3Exp duals of the B parameter vectors, host -> device: the first thing lm_linearize does, or — ahead of it — a
-// caller that has other work to put on the stream in between (the overlapped step)
-cudaError_t lm_stage_candidates(LmState &lm, const double *x, int B, cudaStream_t st) {
+// Sim3Exp / SE3Exp duals of the B parameter vectors and the problem of each, host -> device: the first thing lm_linearize
+// does, or — ahead of it — a caller that has other work to put on the stream in between (the overlapped step)
+cudaError_t lm_stage_candidates(LmState &lm, const double *x, const int *problem, int B, cudaStream_t st) {
     cudaError_t e;
 #define TRY(x) do { e = (x); if (e != cudaSuccess) return e; } while (0)
+    const size_t bytes = (sizeof(LmCand) + sizeof(int)) * (size_t)B;
     if (B > lm.cand_cap) {
         dfree(lm.d_cand);
         if (lm.h_cand) cudaFreeHost(lm.h_cand);
         lm.h_cand = nullptr;
-        TRY(cudaMalloc(&lm.d_cand, sizeof(LmCand) * B));
-        TRY(cudaMallocHost(&lm.h_cand, sizeof(LmCand) * B));
+        lm.cand_cap = 0;
+        TRY(cudaMalloc(&lm.d_cand, bytes));
+        TRY(cudaMallocHost(&lm.h_cand, bytes));
         lm.cand_cap = B;
     }
     LmCand *hc = reinterpret_cast<LmCand *>(lm.h_cand);
+    int *hp = reinterpret_cast<int *>(hc + B);
     if (!lm.h2d_done) TRY(cudaEventCreateWithFlags(&lm.h2d_done, cudaEventDisableTiming));
     TRY(cudaEventSynchronize(lm.h2d_done));
-    for (int b = 0; b < B; ++b) make_lm_candidate(x + (size_t)b * 7, hc + b);
-    TRY(cudaMemcpyAsync(lm.d_cand, hc, sizeof(LmCand) * B, cudaMemcpyHostToDevice, st));
+    for (int b = 0; b < B; ++b) { make_lm_candidate(x + (size_t)b * 7, hc + b); hp[b] = problem ? problem[b] : 0; }
+    TRY(cudaMemcpyAsync(lm.d_cand, hc, bytes, cudaMemcpyHostToDevice, st));
     TRY(cudaEventRecord(lm.h2d_done, st));
 #undef TRY
     return cudaSuccess;
 }
 
-cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, const double *x, int B, double *d_out, cudaStream_t st,
-                         const BlockOut *blocks, int out_stride, const P2pView *p2p, cudaEvent_t before_finish, bool cand_staged) {
+cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, const double *x, const int *problem, int B, double *d_out,
+                         cudaStream_t st, const BlockOut *blocks, int out_stride, const P2pView *p2p, cudaEvent_t before_finish, bool cand_staged) {
     cudaError_t e;
 #define TRY(x) do { e = (x); if (e != cudaSuccess) return e; } while (0)
-    if (!cand_staged) TRY(lm_stage_candidates(lm, x, B, st));
+    if (!cand_staged) TRY(lm_stage_candidates(lm, x, problem, B, st));
+    const LmCand *cands = reinterpret_cast<const LmCand *>(lm.d_cand);
+    // the staged problem index is read only when the caller named problems (stl_*_multi)
+    const int *cprob = problem ? reinterpret_cast<const int *>(cands + B) : nullptr;
     // grids are sized from the host-side upper bound of the block count (one block per map-point-carrying
     // keypoint at most) — never from the counts themselves, so that the chunking, and with it the order
     // of the fp64 sums, is the same whether or not the host has looked at the counts; the kernels read
@@ -1103,14 +1227,14 @@ cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, co
     const BlockOut bo = blocks ? *blocks : BlockOut();
     if (blocks) {
         TRY(lm_compact3d(pk, lm, st));
-        k_linearize<true><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, reinterpret_cast<const LmCand *>(lm.d_cand), lm.partial, stride, bo);
+        k_linearize<true><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
     } else {
-        k_linearize<false><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, reinterpret_cast<const LmCand *>(lm.d_cand), lm.partial, stride, bo);
+        k_linearize<false><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
     }
     TRY(cudaGetLastError());
     if (gchunks > 0) {
-        if (blocks) k_linearize_gpr<true><<<dim3(gchunks, B), 32, 0, st>>>(pk, pr, lm, reinterpret_cast<const LmCand *>(lm.d_cand), lm.partial, stride, chunks, bo);
-        else k_linearize_gpr<false><<<dim3(gchunks, B), 32, 0, st>>>(pk, pr, lm, reinterpret_cast<const LmCand *>(lm.d_cand), lm.partial, stride, chunks, bo);
+        if (blocks) k_linearize_gpr<true><<<dim3(gchunks, B), 32, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, chunks, bo);
+        else k_linearize_gpr<false><<<dim3(gchunks, B), 32, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, chunks, bo);
         TRY(cudaGetLastError());
     }
     if (before_finish) TRY(cudaStreamWaitEvent(st, before_finish, 0));

@@ -12,6 +12,8 @@ mirrors the same interface for Python callers and for the parity tests, on top o
                                  ``f1 f2 C valid_rate`` per candidate
 * :class:`LMProblem`         <- BuildProblem + ceres::Problem::Evaluate (iba_local.cpp:145-323,434-446):
                                  associate at the current estimate, then cost / J^T r / J^T J
+* :class:`LMProblemSet`      <- the same for several starts at once: one ceres::Problem per start,
+                                 all frozen on one context and evaluated by one call
 
 All state (scans, keyframes, index) lives in a :class:`capi.Context`; with several GPUs the
 keyframes are sharded (parallel.py) and the partial sums all-reduced before the epilogue.
@@ -107,6 +109,27 @@ class LMProblem:
         A = H + lam * np.diag(np.maximum(np.diag(H), 1e-12))
         dx = -np.linalg.solve(A, g)
         return np.asarray(x) + dx, cost
+
+
+class LMProblemSet:
+    """P independent :class:`LMProblem` s on one context (multi-start refinement): problem p is frozen at its own start."""
+
+    def __init__(self, ctx: Context, allreduce=None):
+        self.ctx = ctx
+        self.allreduce = allreduce
+        self.n_blocks = None
+
+    def build(self, X0, rebuild=None):
+        """BuildProblem at X0[p] for every start ([P,7]); rebuild (mask [P]) re-associates only the flagged problems."""
+        self.n_blocks = self.ctx.associate_multi(X0, rebuild)
+        return self.n_blocks
+
+    def evaluate(self, X, problem=None):
+        """-> (cost [B], gradient [B,7], JtJ [B,7,7]) of candidate b (X [B,7]) on problem problem[b] (None: candidate p on problem p)."""
+        s = self.ctx.linearize_multi(np.atleast_2d(np.asarray(X, dtype=np.float64)), problem)
+        if self.allreduce is not None:
+            s = self.allreduce(s)
+        return s[:, 0].copy(), s[:, 1:8].copy(), s[:, 8:57].reshape(-1, 7, 7).copy()
 
 
 # ------------------------------------------------------------------------------------------------

@@ -13,6 +13,9 @@ They are NOT a replacement for NOMAD / Ceres; INTEGRATION.md shows how the real 
 * :func:`lm_refine`    — the shape of ``iba_local.cpp:434-460``: outer loop = ``BuildProblem`` at the
   current estimate (association), inner loop = Levenberg-Marquardt on the frozen residual blocks,
   stop when the estimate moved less than ``iba_min_diff``.
+* :func:`lm_refine_multi` — :func:`lm_refine` from several starts in lockstep over a problem set: one
+  ``evaluate`` call per inner iteration for all starts still iterating, one ``build`` per outer iteration
+  for the starts not yet converged.  Start p follows exactly the trajectory of ``lm_refine`` from ``X0[p]``.
 """
 from __future__ import annotations
 
@@ -103,3 +106,61 @@ def lm_refine(problem, x0, max_iba_iter=5, max_num_iterations=30, iba_min_diff=1
         if np.allclose(last, x, rtol=0.0, atol=iba_min_diff):  # allClose(last_sim3_log, sim3_log, iba_min_diff)
             break
     return x, costs
+
+
+def lm_refine_multi(problem_set, X0, max_iba_iter=5, max_num_iterations=30, iba_min_diff=1e-6, lam0=1e-4):
+    """:func:`lm_refine` for P starts at once.  ``problem_set.build(X, rebuild)`` freezes problem p at X[p] for the starts
+    flagged in ``rebuild`` (None: a new set of P); ``problem_set.evaluate(X, problem)`` returns ``(cost [B], g [B,7],
+    H [B,7,7])`` of row b of X on problem ``problem[b]``.  Returns ``(X [P,7], costs per start)``."""
+    X = np.array(np.atleast_2d(X0), dtype=np.float64)
+    P = X.shape[0]
+    costs = [[] for _ in range(P)]
+    outer = np.ones(P, dtype=bool)  # starts whose outer loop goes on
+    for it in range(max_iba_iter):
+        act = np.flatnonzero(outer)
+        if act.size == 0:
+            break
+        last = X.copy()
+        problem_set.build(X, None if it == 0 else outer.astype(np.uint8))
+        lam = np.full(P, lam0)
+        cost, g, H = np.zeros(P), np.zeros((P, 7)), np.zeros((P, 7, 7))
+        c, gg, HH = problem_set.evaluate(X[act], act)
+        cost[act], g[act], H[act] = c, gg, HH
+        inner = outer.copy()  # starts whose inner loop goes on
+        for _ in range(max_num_iterations):
+            todo, steps = [], []
+            for p in np.flatnonzero(inner):
+                D = np.diag(np.maximum(np.diag(H[p]), 1e-12))
+                try:
+                    step = -np.linalg.solve(H[p] + lam[p] * D, g[p])
+                except np.linalg.LinAlgError:
+                    lam[p] *= 10.0
+                    continue
+                todo.append(p)
+                steps.append(step)
+            if not todo:
+                if not inner.any():
+                    break
+                continue
+            todo = np.asarray(todo)
+            Xt = X[todo] + np.asarray(steps)
+            c1, g1, H1 = problem_set.evaluate(Xt, todo)
+            for k, p in enumerate(todo):
+                if np.isfinite(c1[k]) and c1[k] < cost[p]:
+                    X[p] = Xt[k]
+                    rel = (cost[p] - c1[k]) / max(cost[p], 1e-300)
+                    cost[p], g[p], H[p] = c1[k], g1[k], H1[k]
+                    lam[p] = max(lam[p] / 3.0, 1e-12)
+                    if rel < 1e-10:
+                        inner[p] = False
+                else:
+                    lam[p] *= 4.0
+                    if lam[p] > 1e8:
+                        inner[p] = False
+            if not inner.any():
+                break
+        for p in act:
+            costs[p].append(cost[p])
+            if np.allclose(last[p], X[p], rtol=0.0, atol=iba_min_diff):
+                outer[p] = False
+    return X, costs
