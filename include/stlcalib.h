@@ -404,6 +404,42 @@ stl_status_t stl_comm_info(stl_ctx_t *ctx, int32_t *rank, int32_t *n_ranks);
  * STL_NO_P2P=1 forces it).  out[1] = exchanges done through peer memory so far, out[2] = through NCCL. */
 stl_status_t stl_comm_stats(stl_ctx_t *ctx, int64_t out[3]);
 
+/* ---- keyframe selection on the resident pack ---------------------------------------------------------
+ * A context can restrict every call that walks keyframes to a subset of its pack without a second upload: coarse-to-fine
+ * search on every k-th keyframe, a hold-out check, dropping keyframes with moving objects, or the reference's
+ * single-frame caller (iba_single_frame.cpp, keyframe 0 only).
+ *
+ * kf[n]: LOCAL keyframe indices of this context's pack, strictly increasing, inside [0, n_kf); n = 0 (nothing selected) is
+ * allowed (kf must then still be non-null).  kf == NULL selects every keyframe: the default, restored by every stl_upload_pack.
+ * An invalid list returns STL_ERR_INVALID and leaves the selection as it was; without a pack the call returns STL_ERR_STATE; a
+ * CUDA failure returns STL_ERR_CUDA with every keyframe selected.
+ *
+ * While a selection is set, stl_eval_batch, stl_associate(_multi), stl_step_batch, stl_step_multi (and their _device
+ * twins), stl_eval_blocks, the GPR fit, the work counters and the debug getters behave exactly as a context whose pack
+ * holds only the selected keyframes' rows (KeyFramePack.select): the same records, bit for bit, and the same block counts.
+ * Keyframe f keeps its own rows, among them its hand-eye pair (f, f+1) as he_valid bakes it, whether or not f+1 is
+ * selected.  Keyframe indices the library reports (stl_eval_blocks' kf) remain the pack's own.  The debug getters read an
+ * unselected keyframe as empty (n = 0, a zero record); stl_knn3d is unaffected.
+ *
+ * A selection call DROPS the frozen problem set, the reuse of the last evaluation's 2-D association and the batch the
+ * debug getters refer to: stl_linearize_*, stl_eval_blocks, stl_block_counts, stl_gpr_hyper and stl_step_* without
+ * re-association return STL_ERR_STATE until the next association.
+ *
+ * With a communicator attached the indices are local to the rank's shard, and every rank must still make every call (with
+ * n = 0 where it selects nothing); the record exchange is unchanged. */
+stl_status_t stl_select_keyframes(stl_ctx_t *ctx, const int32_t *kf, int32_t n);
+
+/* BAError per keyframe: evaluates B candidates like stl_eval_batch (the same kernels, one workspace chunk at a time) and
+ * returns, for every keyframe of the pack, the 13-value record of stl_debug_frame in its order,
+ * out[B][n_kf][13] = {sum_3d2d, valid_3d2d, cnt_3d2d, sum_he, cnt_he, kept, n_corr, n_queries,
+ *                     sum_3d3d, valid_3d3d, cnt_3d3d, valid_pl, valid_pt}.
+ * Rows of unselected keyframes are zero.  With err_weight[1] <= 1e-10 the 3-D columns hold what the record counts for the
+ * frame (valid_3d3d = cnt_3d3d = kept, the rest 0), so that the rows of a candidate always sum to its stl_eval_batch
+ * record (counters exactly; sums up to the order of the fp64 additions).  There is no exchange: every rank returns its
+ * own keyframes.  Like stl_eval_batch, the call leaves its batch to the debug getters and its 2-D association to a
+ * following stl_associate at one of its candidates. */
+stl_status_t stl_eval_frames(stl_ctx_t *ctx, const double *x, int32_t B, double *out);
+
 /* ---- debug getters (parity tests only) --------------------------------- */
 
 /* 2-D correspondences of keyframe `kf` for the candidate at index `b` of the
@@ -463,7 +499,7 @@ stl_status_t stl_set_stream(stl_ctx_t *ctx, void *stream);
 stl_status_t stl_set_profiling(stl_ctx_t *ctx, int32_t enabled);
 stl_status_t stl_stage_stats(stl_ctx_t *ctx, double ms[STL_NSTAGES], int64_t launches[STL_NSTAGES]);
 
-/* Work counters of the last stl_eval_batch (host-side, summed over b):
+/* Work counters of the last stl_eval_batch or stl_eval_frames (host-side, summed over b):
  * [0] points streamed by K1, [1] 2-D 1-NN queries (= keypoints),
  * [2] 3-D 1-NN queries, [3] 3-D k-NN queries, [4] algorithmic bytes of K1,
  * [5] kernels of this library launched by the context since its creation,

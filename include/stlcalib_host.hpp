@@ -102,6 +102,21 @@ class Context {
         check(stl_step_multi(ctx_, x, P, rebuild, out.data()), "stl_step_multi");
         return out;
     }
+    // keyframe selection on the resident pack (stl_select_keyframes): every later call walks only the local keyframes kf (strictly
+    // increasing; an empty list selects none) as a pack of only those would; select_all() restores the whole pack.  Both drop
+    // the frozen problem set (associate again before linearising).
+    // (an empty vector may have a null data(), which the C-ABI reads as "all keyframes": it is passed a non-null pointer instead)
+    void select_keyframes(const std::vector<int32_t> &kf) {
+        static const int32_t none = 0;
+        check(stl_select_keyframes(ctx_, kf.empty() ? &none : kf.data(), (int32_t)kf.size()), "stl_select_keyframes");
+    }
+    void select_all() { check(stl_select_keyframes(ctx_, nullptr, 0), "stl_select_keyframes"); }
+    // BAError per keyframe: [B][n_kf][13] records of stl_debug_frame's layout (zero rows for unselected keyframes); n_kf = the pack's
+    std::vector<double> eval_frames(const double *x, int B, int n_kf) {
+        std::vector<double> out((size_t)B * (size_t)n_kf * 13);
+        check(stl_eval_frames(ctx_, x, B, out.data()), "stl_eval_frames");
+        return out;
+    }
     // keyframes sharded over several GPUs: this context holds shard `rank` of `n_ranks`; `id` comes from
     // stl_comm_unique_id on one rank (handed over by the host program).  Afterwards every call returns the totals.
     void comm_init(const uint8_t id[STL_COMM_ID_BYTES], int rank, int n_ranks) { check(stl_comm_init(ctx_, id, rank, n_ranks), "stl_comm_init"); }

@@ -32,6 +32,7 @@ class Context:
         self.h = h
         self.device = device
         self.pack = None
+        self.selection = None  # keyframes selected by select_keyframes (None: all)
         self.n_problems = 0  # problems of the frozen set, set after each successful call that makes one (associate / step: 1, *_multi: P)
 
     def close(self):
@@ -56,6 +57,41 @@ class Context:
         cp = pack.as_c()
         _check(self.lib, self.h, self.lib.stl_upload_pack(self.h, C.byref(cp)))
         self.pack = pack
+        self.selection = None  # an upload selects every keyframe again
+
+    def select_keyframes(self, kf=None):
+        """Restrict every call that walks keyframes to the local keyframes `kf` (strictly increasing; [] selects none) of the
+        uploaded pack: results are those of a context holding ``pack.select(kf)``.  None selects all of them again.  Drops the
+        frozen problem set: the linearise calls raise until the next association."""
+        if kf is None:
+            _check(self.lib, self.h, self.lib.stl_select_keyframes(self.h, None, 0))
+            self.selection = None
+        else:
+            k = np.asarray(kf)
+            if k.size == 0:
+                k = k.astype(np.int64).reshape(0)
+            if k.ndim != 1 or k.dtype.kind not in "iu":  # as KeyFramePack.select: no silent truncation of non-integers
+                raise TypeError("select_keyframes: kf must be a 1-D list of integer keyframe indices")
+            k = k.astype(np.int64)
+            if k.size and (k.min() < -2**31 or k.max() >= 2**31):
+                raise ValueError("keyframe index outside the int32 range")
+            k = np.ascontiguousarray(k, dtype=np.int32)
+            buf = k if k.size else np.zeros(1, np.int32)  # an empty selection is a non-null pointer with n = 0 (NULL selects all)
+            _check(self.lib, self.h, self.lib.stl_select_keyframes(self.h, buf.ctypes.data_as(_abi._i32p), int(k.size)))
+            self.selection = k.copy()
+        self.n_blocks = None
+        self.n_problems = 0
+
+    def eval_frames(self, x) -> np.ndarray:
+        """x [B,7] -> the per-keyframe record of BAError [B, n_kf, 13] (the 13 values of :meth:`debug_frame`, in its order) of
+        every keyframe of the pack; rows of unselected keyframes are zero.  Each rank returns its own keyframes."""
+        x = np.ascontiguousarray(np.atleast_2d(x), dtype=np.float64)
+        B = x.shape[0]
+        if self.pack is None:
+            raise _abi.StlError(4, "no pack uploaded")
+        out = np.empty((B, int(self.pack.n_kf), 13), dtype=np.float64)
+        _check(self.lib, self.h, self.lib.stl_eval_frames(self.h, x.ctypes.data_as(_dp), B, out.ctypes.data_as(_dp)))
+        return out
 
     # -- Nomad / iba_func path ---------------------------------------------
     def eval_sums(self, x) -> np.ndarray:

@@ -237,9 +237,9 @@ k_assoc2d(const DevPack pk, const DevWork wk, const DevParams pr, const int B, c
         }
         S.unit = u;
         if (u >= 0) {
-            const int f = u / B;
+            const int i = u / B, f = sel_kf(pk, i);
             const DevKf &K = pk.kf[f];
-            const DevCand &c = wk.cand[u - f * B];
+            const DevCand &c = wk.cand[u - i * B];
             S.new_tab = f != S.cur_f;
             S.cur_f = f;
             if (S.new_tab) {
@@ -302,7 +302,7 @@ k_assoc2d(const DevPack pk, const DevWork wk, const DevParams pr, const int B, c
     __syncthreads();
     const int unit = S.unit;
     if (unit < 0) break;
-    const int f = unit / B, b = unit - f * B;
+    const int fi = unit / B, f = sel_kf(pk, fi), b = unit - fi * B;
     const DevKf K = pk.kf[f];
     const DevCand &c = wk.cand[b];
     const bool new_tab = S.new_tab != 0;
@@ -641,8 +641,8 @@ cudaError_t assoc2d_configure(size_t smem) {
 
 cudaError_t launch_assoc2d(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, size_t smem, int max_kp, int max_tab_bytes,
                            int max_groups, cudaStream_t st, int with_terms) {
-    if (B <= 0 || pk.n_kf <= 0) return cudaSuccess;
-    const long long n_units = (long long)pk.n_kf * B;
+    if (B <= 0 || pk.n_sel <= 0) return cudaSuccess;
+    const long long n_units = (long long)pk.n_sel * B;  // unit = selection position * B + candidate
     if (n_units > 0x7fffffffll || wk.k1_slots <= 0) return cudaErrorInvalidValue;
     // candidates of one keyframe are consecutive units: a chunk keeps the keyframe's tables in shared memory
     const int chunk = B >= 64 ? 8 : (B >= 16 ? 4 : (B >= 4 ? 2 : 1));

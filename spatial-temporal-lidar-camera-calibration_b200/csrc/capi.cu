@@ -46,6 +46,13 @@ struct stl_ctx {
     size_t k1_smem = 0, k1_split_smem = 0;
     bool k1_mono = true;   // the one-kernel K1 (assoc2d.cu); STL_K1_SPLIT=1 selects the three-kernel form (assoc2d_split.cu)
     long long n_pts_total = 0;
+    // keyframe selection (stl_select_keyframes): pk.sel / pk.sel_mp point into these while a subset is selected
+    std::vector<uint8_t> sel_mask;        // [n_kf] 1 = selected
+    int *d_sel = nullptr;                 // [sel_cap]
+    int2 *d_sel_mp = nullptr;             // [sel_cap + 1]
+    int sel_cap = 0;
+    long long sel_pts = 0, sel_kp = 0;    // scan points / keypoints of the selected keyframes (work counters)
+    double *d_frames = nullptr;           // stl_eval_frames: [Bc][n_kf][13] of one workspace chunk
     // workspace
     DevWork wk;
     int wk_cap = 0;
@@ -128,6 +135,9 @@ void free_pack(stl_ctx *c) {
     dfree(p.k1tab); dfree(p.bitmap); dfree(p.grid_start); dfree(p.grid_kp); dfree(p.kp_xy); dfree(p.kp_xyd); dfree(p.kp_mp); dfree(p.Tcw);
     dfree(p.relpose); dfree(p.covis_valid); dfree(p.covis_uv); dfree(p.he_Tc); dfree(p.he_Tl);
     p = DevPack();
+    dfree(c->d_sel); dfree(c->d_sel_mp); dfree(c->d_frames);
+    c->sel_cap = 0;
+    c->sel_mask.clear();
     c->has_pack = false;
 }
 void free_work(stl_ctx *c) {
@@ -137,6 +147,7 @@ void free_work(stl_ctx *c) {
     dfree(w.frame); dfree(w.align); dfree(w.nn_pos); dfree(w.nn_g2); dfree(w.nb); dfree(w.nbx); dfree(w.nb_m); dfree(w.nb_last); dfree(w.dbg_nn); dfree(w.dbg_m); dfree(w.dbg_plane); dfree(w.dbg_dist); dfree(w.dbg_knn); dfree(w.dbg_stats);
     dfree(w.overflow); dfree(w.k1_clk);
     w = DevWork();
+    dfree(c->d_frames);  // sized by the chunk
     c->wk_cap = 0;
     c->dbg_alloc = false;
 }
@@ -296,6 +307,19 @@ stl_status_t ensure_work(stl_ctx *ctx, int B, bool debug) {
     return STL_OK;
 }
 
+// scan points and keypoints an evaluation of B candidates walks (those of the selected keyframes)
+void set_eval_counters(stl_ctx *ctx, int B) {
+    ctx->counters[0] = (double)ctx->sel_pts * B;
+    ctx->counters[1] = (double)ctx->sel_kp * B;
+    ctx->counters[4] = ((double)ctx->sel_pts * 12.0 + (double)ctx->sel_kp * 16.0) * B;
+}
+
+// 3-D 1-NN / k-NN queries of an evaluation whose records count q3 3-D terms (cnt_3d3d summed over the candidates)
+void set_query_counters(stl_ctx *ctx, double q3) {
+    ctx->counters[2] = ctx->params.err_weight[1] > 1e-10 ? q3 : 0.0;
+    ctx->counters[3] = (ctx->params.use_plane && ctx->params.err_weight[1] > 1e-10) ? q3 : 0.0;
+}
+
 // Enqueues the evaluation of B candidates; d_out [B][STL_EVAL_NSUMS] device.
 // exchange: the record of this call is complete after K3 (stl_eval_batch): K3 sums it over the ranks, chunk by chunk, when
 // the peer path is up; *exchanged tells the caller whether that happened (else it runs the NCCL all-reduce)
@@ -330,9 +354,7 @@ stl_status_t enqueue_eval(stl_ctx *ctx, const double *x, int B, double *d_out, c
         ctx->wk_has_nn = true;  // K2a runs for every query of a kept frame and writes its nn_pos
     }
     CK(cudaEventRecord(ctx->h2d_done, st));
-    ctx->counters[0] = (double)ctx->n_pts_total * B;
-    ctx->counters[1] = (double)ctx->pk.n_kp_total * B;
-    ctx->counters[4] = ((double)ctx->n_pts_total * 12.0 + (double)ctx->pk.n_kp_total * 16.0) * B;
+    set_eval_counters(ctx, B);
     ctx->last_x.assign(x, x + (size_t)B * 7);
     ctx->dbg_b = -1;
     return STL_OK;
@@ -453,6 +475,27 @@ stl_status_t need_single(stl_ctx *ctx, const char *call, const char *multi) {
         return fail(ctx, STL_ERR_STATE, "%s: the frozen set holds %d problems; use %s (or stl_associate to freeze one)", call, ctx->lm.P, multi);
     return STL_OK;
 }
+
+// Selection of every keyframe (the state of a new pack): no selection array, the kernels' grids are those of the whole pack
+void select_all(stl_ctx *c) {
+    c->pk.sel = nullptr; c->pk.sel_mp = nullptr;
+    c->pk.n_sel = c->pk.n_kf; c->pk.n_sel_mp = c->pk.n_mp_total;
+    c->sel_mask.assign((size_t)c->pk.n_kf, 1);
+    c->sel_pts = c->n_pts_total; c->sel_kp = c->pk.n_kp_total;
+}
+
+// A new selection invalidates what was computed over the previous one: the frozen problem set (the linearise calls refuse until
+// the next association), the 2-D association reuse and the debug re-evaluation
+void drop_selection_state(stl_ctx *c) {
+    c->lm.ready = false;
+    c->wk_x.clear();
+    c->wk_has_nn = false;
+    c->last_x.clear();
+    c->dbg_b = -1;
+}
+
+// the debug getters read an unselected keyframe as empty
+bool kf_selected(const stl_ctx *c, int kf) { return c->sel_mask[(size_t)kf] != 0; }
 
 stl_status_t run_debug(stl_ctx *ctx, int b) {
     if (!ctx->has_pack) return fail(ctx, STL_ERR_STATE, "no pack uploaded");
@@ -829,6 +872,7 @@ stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *p) {
         ctx->stage_ms[STL_STAGE_PLANE_INDEX] += ms;
         ctx->stage_n[STL_STAGE_PLANE_INDEX] += 1;
     }
+    select_all(ctx);
     ctx->has_pack = true;
     return STL_OK;
 }
@@ -863,8 +907,7 @@ stl_status_t stl_eval_batch(stl_ctx_t *ctx, const double *x, int32_t B, stl_eval
     memcpy(sums, ctx->h_sums, sizeof(double) * STL_EVAL_NSUMS * B);
     double q3 = 0;
     for (int b = 0; b < B; ++b) q3 += sums[b].cnt_3d3d;
-    ctx->counters[2] = ctx->params.err_weight[1] > 1e-10 ? q3 : 0.0;
-    ctx->counters[3] = (ctx->params.use_plane && ctx->params.err_weight[1] > 1e-10) ? q3 : 0.0;
+    set_query_counters(ctx, q3);
     return STL_OK;
 }
 
@@ -892,6 +935,7 @@ stl_status_t stl_debug_corrset(stl_ctx_t *ctx, int32_t b, int32_t kf, uint32_t *
     stl_status_t s = run_debug(ctx, b);
     if (s != STL_OK) return s;
     if (kf < 0 || kf >= ctx->pk.n_kf) return fail(ctx, STL_ERR_INVALID, "keyframe out of range");
+    if (!kf_selected(ctx, kf)) { *n = 0; return STL_OK; }
     int nc = 0;
     CK(cudaMemcpy(&nc, ctx->wk.n_corr + kf, 4, cudaMemcpyDeviceToHost));
     *n = nc;
@@ -909,6 +953,7 @@ stl_status_t stl_debug_align(stl_ctx_t *ctx, int32_t b, int32_t kf, uint32_t *kp
     stl_status_t s = run_debug(ctx, b);
     if (s != STL_OK) return s;
     if (kf < 0 || kf >= ctx->pk.n_kf) return fail(ctx, STL_ERR_INVALID, "keyframe out of range");
+    if (!kf_selected(ctx, kf)) { *n = 0; return STL_OK; }
     int nq = 0;
     CK(cudaMemcpy(&nq, ctx->wk.n_q + kf, 4, cudaMemcpyDeviceToHost));
     *n = nq;
@@ -938,6 +983,7 @@ stl_status_t stl_debug_frame(stl_ctx_t *ctx, int32_t b, int32_t kf, double out[1
     stl_status_t s = run_debug(ctx, b);
     if (s != STL_OK) return s;
     if (kf < 0 || kf >= ctx->pk.n_kf) return fail(ctx, STL_ERR_INVALID, "keyframe out of range");
+    if (!kf_selected(ctx, kf)) { for (int i = 0; i < 13; ++i) out[i] = 0; return STL_OK; }
     FrameRec r;
     CK(cudaMemcpy(&r, ctx->wk.frame + kf, sizeof(r), cudaMemcpyDeviceToHost));
     std::vector<AlignRec> a(ctx->wk.sub);
@@ -959,6 +1005,89 @@ stl_status_t stl_debug_frame(stl_ctx_t *ctx, int32_t b, int32_t kf, double out[1
                 st[4], 100.0 * st[5] / std::max(st[4], 1ull), 100.0 * st[6] / std::max(st[4], 1ull), 100.0 * st[7] / std::max(st[4], 1ull));
     }
     for (auto &x : a) { out[8] += x.s3d; out[9] += x.v3d; out[10] += x.c3d; out[11] += x.vpl; out[12] += x.vpt; }
+    return STL_OK;
+}
+
+stl_status_t stl_select_keyframes(stl_ctx_t *ctx, const int32_t *kf, int32_t n) {
+    if (!ctx) return STL_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!ctx->has_pack) return fail(ctx, STL_ERR_STATE, "stl_upload_pack has not been called");
+    const int F = ctx->pk.n_kf;
+    if (kf) {  // validated completely before anything changes
+        if (n < 0 || n > F) return fail(ctx, STL_ERR_INVALID, "stl_select_keyframes: n = %d is outside [0, n_kf = %d]", n, F);
+        for (int i = 0; i < n; ++i) {
+            if (kf[i] < 0 || kf[i] >= F) return fail(ctx, STL_ERR_INVALID, "stl_select_keyframes: kf[%d] = %d is outside [0, %d)", i, kf[i], F);
+            if (i > 0 && kf[i] <= kf[i - 1]) return fail(ctx, STL_ERR_INVALID, "stl_select_keyframes: the list is not strictly increasing at %d", i);
+        }
+    }
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = acquire_stream(ctx, nullptr);
+    CK(cudaStreamSynchronize(st));  // the kernels already queued read the previous selection arrays
+    drop_selection_state(ctx);
+    // from here on the context selects every keyframe until the new selection is complete on the device: a CUDA failure on the
+    // way leaves it there (never half-switched between two lists)
+    select_all(ctx);
+    if (!kf) return STL_OK;
+    // host tables first; sel_mp[i] = (first slot of position i in the compacted slot range, mp_off - that): k_linearize maps a
+    // compacted slot back
+    std::vector<int2> mp((size_t)n + 1);
+    std::vector<uint8_t> mask((size_t)F, 0);
+    long long slots = 0, pts = 0, kps = 0;
+    for (int i = 0; i < n; ++i) {
+        const DevKf &K = ctx->h_kf[kf[i]];
+        mp[i] = make_int2((int)slots, (int)(K.mp_off - slots));
+        slots += K.n_mp; pts += K.n_pts; kps += K.n_kp;
+        mask[kf[i]] = 1;
+    }
+    mp[n] = make_int2((int)slots, 0);
+    cudaError_t e = cudaSuccess;
+    if (n > ctx->sel_cap || !ctx->d_sel) {
+        dfree(ctx->d_sel); dfree(ctx->d_sel_mp);
+        ctx->sel_cap = 0;
+        const size_t cap = (size_t)std::max(n, 1);
+        e = cudaMalloc(&ctx->d_sel, sizeof(int) * cap);
+        if (e == cudaSuccess) e = cudaMalloc(&ctx->d_sel_mp, sizeof(int2) * (cap + 1));
+        if (e == cudaSuccess) ctx->sel_cap = (int)cap;
+        else { dfree(ctx->d_sel); dfree(ctx->d_sel_mp); }
+    }
+    if (e == cudaSuccess && n > 0) e = cudaMemcpyAsync(ctx->d_sel, kf, sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_sel_mp, mp.data(), sizeof(int2) * ((size_t)n + 1), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(ctx, STL_ERR_CUDA, "stl_select_keyframes: %s (every keyframe stays selected)", cudaGetErrorString(e));
+    ctx->pk.sel = ctx->d_sel; ctx->pk.sel_mp = ctx->d_sel_mp;
+    ctx->pk.n_sel = n; ctx->pk.n_sel_mp = slots;
+    ctx->sel_mask.swap(mask);
+    ctx->sel_pts = pts; ctx->sel_kp = kps;
+    return STL_OK;
+}
+
+stl_status_t stl_eval_frames(stl_ctx_t *ctx, const double *x, int32_t B, double *out) {
+    if (!ctx || !x || !out || B <= 0) return STL_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!ctx->has_pack) return fail(ctx, STL_ERR_STATE, "stl_upload_pack has not been called");
+    CK(cudaSetDevice(ctx->device));
+    stl_status_t s = ensure_work(ctx, B, false);
+    if (s != STL_OK) return s;
+    const int F = ctx->pk.n_kf, Bc = ctx->wk.Bc;
+    const size_t row = (size_t)F * 13;
+    if (!ctx->d_frames) CK(cudaMalloc(&ctx->d_frames, sizeof(double) * row * Bc));
+    cudaStream_t st = acquire_stream(ctx, nullptr);
+    // one workspace chunk at a time: evaluation (no exchange: each rank returns its own keyframes), then the gather of its records
+    for (int c0 = 0; c0 < B; c0 += Bc) {
+        const int nb = std::min(Bc, B - c0);
+        s = enqueue_eval(ctx, x + (size_t)c0 * 7, nb, ctx->d_sums, st, false);
+        if (s != STL_OK) return s;
+        CK(cudaMemsetAsync(ctx->d_frames, 0, sizeof(double) * row * nb, st));
+        CK(launch_frames(ctx->pk, ctx->wk, ctx->dpr, nb, ctx->d_frames, st));
+        ctx->launches += 1;
+        CK(cudaMemcpyAsync(out + row * c0, ctx->d_frames, sizeof(double) * row * nb, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+    set_eval_counters(ctx, B);
+    double q3 = 0;  // cnt_3d3d of the rows: the record's count, exactly (integers)
+    for (size_t r = 0; r < (size_t)B * F; ++r) q3 += out[r * 13 + 10];
+    set_query_counters(ctx, q3);
+    ctx->last_x.assign(x, x + (size_t)B * 7);  // as stl_eval_batch: the debug getters and the 2-D association reuse see this batch
     return STL_OK;
 }
 

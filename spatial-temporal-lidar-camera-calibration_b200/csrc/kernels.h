@@ -34,7 +34,18 @@ struct DevPack {
     float2 *covis_uv = nullptr;      // [n_kp_total][C]
     float *he_Tc = nullptr;          // [n_kf][12]
     double *he_Tl = nullptr;         // [n_kf][12]
+    // keyframe selection (stl_select_keyframes): the kernels walk selection positions i < n_sel, keyframe sel_kf(pk, i), in
+    // the order a pack of only those keyframes would have them.  sel == nullptr: every keyframe (n_sel = n_kf), no extra load.
+    // Workspace records stay indexed by the pack's keyframe ([b][n_kf]): those of unselected keyframes are stale.
+    int n_sel = 0;
+    const int *sel = nullptr;        // [n_sel] selected keyframes, strictly increasing
+    const int2 *sel_mp = nullptr;    // [n_sel + 1] (first compacted map-point slot of position i, mp_off - that): k_linearize's 3-D walk
+    long long n_sel_mp = 0;          // map-point slots of the selected keyframes
 };
+
+#ifdef __CUDACC__
+__device__ __forceinline__ int sel_kf(const DevPack &pk, int i) { return pk.sel ? pk.sel[i] : i; }
+#endif
 
 // Workspace of one candidate chunk (Bc candidates x all keyframes).
 struct DevWork {
@@ -142,6 +153,9 @@ cudaError_t launch_debug_trig(const double *d_x, int n, double *d_acos, double *
 // p2p (optional): the kernel also exchanges and sums each candidate's record over the ranks (p2p.cuh)
 cudaError_t launch_reduce(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, double *d_out, cudaStream_t st, int out_stride = 0,
                           const P2pView *p2p = nullptr);
+// stl_eval_frames: the per-keyframe records (stl_debug_frame's 13 values) of the selected keyframes of B candidates,
+// d_out [B][n_kf][13] (rows of unselected keyframes untouched)
+cudaError_t launch_frames(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, double *d_out, cudaStream_t st);
 
 // ---- N4 (calib.cu): hand-eye initialisation edges and calibration-BA edges; HOST in, HOST out, synchronous
 }  // namespace stl

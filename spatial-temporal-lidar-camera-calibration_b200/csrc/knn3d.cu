@@ -57,7 +57,7 @@ k_nn_knn(const DevPack pk, const DevWork wk, const DevParams pr, const int B, co
     const int sub = wk.sub;
     const int j = blockIdx.x % sub;
     const int bf = blockIdx.x / sub;
-    const int f = bf / B, b = bf - f * B;
+    const int fi = bf / B, f = sel_kf(pk, fi), b = bf - fi * B;
     const int nq = wk.n_q[(long long)b * pk.n_kf + f];
     if (nq <= 0) return;
     const int lane = threadIdx.x & 31;
@@ -169,7 +169,7 @@ k_plane_dist(const DevPack pk, const DevWork wk, const DevParams pr, const int B
     const int sub = wk.sub;
     const int j = blockIdx.x % sub;
     const int bf = blockIdx.x / sub;
-    const int f = bf / B, b = bf - f * B;
+    const int fi = bf / B, f = sel_kf(pk, fi), b = bf - fi * B;
     const long long rec = (long long)b * pk.n_kf + f;
     const int nq = wk.n_q[rec];
     double s3d = 0, v3d = 0, c3d = 0, vpl = 0, vpt = 0;
@@ -324,16 +324,17 @@ cudaError_t launch_debug_trig(const double *d_x, int n, double *d_acos, double *
 
 cudaError_t launch_align3d(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, int debug, cudaStream_t st, cudaEvent_t after_traversal,
                            uint32_t *lm_pos, int *lm_m) {
-    if (B <= 0 || pk.n_kf <= 0) return cudaSuccess;
+    if (B <= 0) return cudaSuccess;
+    if (pk.n_sel <= 0) return after_traversal ? cudaEventRecord(after_traversal, st) : cudaSuccess;
     // queries a warp draws at a time: the per-query preamble runs one query per lane, the searches one after another — a long
-    // batch is cheap in instructions and long in latency, so small keyframe shards (one wave of CTAs) get the short one
-    int batch = (long long)pk.n_kf * B >= 600 ? 8 : 4;
+    // batch is cheap in instructions and long in latency, so small keyframe shards or selections (one wave of CTAs) get the short one
+    int batch = (long long)pk.n_sel * B >= 600 ? 8 : 4;
     if (const char *e = getenv("STL_K2_BATCH")) batch = std::max(1, std::min(32, atoi(e)));
-    k_nn_knn<<<(unsigned)(pk.n_kf * B * wk.sub), kWarps * 32, 0, st>>>(pk, wk, pr, B, batch, lm_pos, lm_m);
+    k_nn_knn<<<(unsigned)(pk.n_sel * B * wk.sub), kWarps * 32, 0, st>>>(pk, wk, pr, B, batch, lm_pos, lm_m);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     if (after_traversal && (e = cudaEventRecord(after_traversal, st)) != cudaSuccess) return e;
-    k_plane_dist<<<(unsigned)(pk.n_kf * B * wk.sub), kPlaneThreads, 0, st>>>(pk, wk, pr, B, debug);
+    k_plane_dist<<<(unsigned)(pk.n_sel * B * wk.sub), kPlaneThreads, 0, st>>>(pk, wk, pr, B, debug);
     return cudaGetLastError();
 }
 

@@ -40,7 +40,7 @@ constexpr int kLinThreads = 128;
 // All four walk the correspondences that carry a map point (the query list K1 wrote), keyframe by
 // keyframe; list slot = block slot = mp_off[f] + qi.  Traversals are warp-per-item, plane fits thread-per-item.
 // With the plane index only k_lm_plane_a and k_lm_plane_b run (and inside stl_step_batch K2a answers k_lm_knn_b's question).
-// grid (n_kf * sub, lanes): association lane blockIdx.y reads the K1 result at its workspace candidate slot, works in its own
+// grid (n_sel * sub, lanes) over the keyframe selection (DevPack::sel; all keyframes without one): association lane blockIdx.y reads the K1 result at its workspace candidate slot, works in its own
 // scratch and writes the arrays of its problem (lm_lane) — a lane computes exactly what a single association computes.
 
 // Narrows the workspace, the scratch and the problem arrays to association lane blockIdx.y.
@@ -93,7 +93,7 @@ __device__ __forceinline__ void lm_map_point(const DevPack &pk, const DevKf &K, 
 __global__ void __launch_bounds__(kWarps * 32, STL_LM_MINB)
 k_lm_knn_a(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
     lm_lane(pk, wk, lm);
-    const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
+    const int j = blockIdx.x % lm.sub, f = sel_kf(pk, blockIdx.x / lm.sub);
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -133,7 +133,7 @@ k_lm_knn_a(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
 __global__ void __launch_bounds__(128)
 k_lm_plane_a(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
     lm_lane(pk, wk, lm);
-    const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
+    const int j = blockIdx.x % lm.sub, f = sel_kf(pk, blockIdx.x / lm.sub);
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
     __shared__ int cnt[2];  // plane blocks, GPR blocks of this CTA (one pair of global atomics per CTA)
@@ -199,7 +199,7 @@ k_lm_knn_b(const DevPack pk, DevWork wk, const DevParams pr, LmState lm, const b
     lm_lane(pk, wk, lm);
     const uint32_t *__restrict__ nn_hint = hints ? wk.nn_pos : nullptr;
     const float *__restrict__ nn_g2 = hints && cert ? wk.nn_g2 : nullptr;
-    const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
+    const int j = blockIdx.x % lm.sub, f = sel_kf(pk, blockIdx.x / lm.sub);
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
     const int lane = threadIdx.x & 31;
@@ -315,7 +315,7 @@ __device__ __forceinline__ bool block3d_geometry(const DevPack &pk, const DevPar
 __global__ void __launch_bounds__(128)
 k_lm_plane_b(const DevPack pk, DevWork wk, const DevParams pr, LmState lm) {
     lm_lane(pk, wk, lm, false);
-    const int j = blockIdx.x % lm.sub, f = blockIdx.x / lm.sub;
+    const int j = blockIdx.x % lm.sub, f = sel_kf(pk, blockIdx.x / lm.sub);
     int nq;
     if (!lm_frame_active(wk, pr, f, nq)) return;
     const DevKf K = pk.kf[f];
@@ -443,6 +443,18 @@ __device__ __forceinline__ void lm_list_start(const LmState &lm, int p, int whic
     if (threadIdx.x == 0) *out = s;
 }
 
+// Problem-local slot of slot v of the selection's compacted slot range (DevPack::sel_mp): with a keyframe selection the 3-D walk
+// runs over the selected keyframes' slots only, grouped 32 at a time as a pack of those keyframes groups them, so that every
+// thread sums the blocks it would sum there
+__device__ __forceinline__ int sel_slot(const DevPack &pk, int v) {
+    int lo = 0, hi = pk.n_sel;  // sel_mp[lo].x <= v < sel_mp[hi].x
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (pk.sel_mp[mid].x <= v) lo = mid; else hi = mid;
+    }
+    return v + pk.sel_mp[lo].y;
+}
+
 // grid (chunks, B): candidate blockIdx.y on problem cprob[blockIdx.y].  The 3-D/3-D blocks are walked over ALL query slots of
 // that problem (no compacted list: the work per block is light, and the association then has no select on the way to the
 // linearisation).  WB (stl_eval_blocks) numbers the blocks and therefore walks the compacted list (problem 0).
@@ -540,7 +552,7 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
     // slots per round, queues the flagged ones in shared memory and evaluates 32 queued blocks at a time (the tail at the end): the
     // lanes stay full although only half of the slots carry a block, and nothing outside this kernel has to compact the list.
     // Which thread sums which block depends on the flags alone, never on the batch size.
-    const long long n3 = WB ? (long long)counts[1] : lm.max_blocks;
+    const long long n3 = WB ? (long long)counts[1] : (pk.sel ? pk.n_sel_mp : lm.max_blocks);
     const long long po = (long long)prob * lm.slot_stride;  // the 3-D walk is in problem-local slots
     const uint8_t *flag3d = lm.flag3d + po, *type3d = lm.type3d + po;
     const double *geo3d = lm.geo3d + po * 9;
@@ -557,9 +569,10 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             const bool more = base < n3;
             if (more) {
                 const long long sl = base + lane3;
-                const bool on = sl < n3 && flag3d[sl];
+                const int rs = pk.sel && sl < n3 ? sel_slot(pk, (int)sl) : (int)sl;
+                const bool on = sl < n3 && flag3d[rs];
                 const unsigned mask = __ballot_sync(0xffffffffu, on);
-                if (on) q3[warp3][qlen + __popc(mask & ((1u << lane3) - 1))] = (int)sl;
+                if (on) q3[warp3][qlen + __popc(mask & ((1u << lane3) - 1))] = rs;
                 qlen += __popc(mask);
                 base += stride;
                 __syncwarp();
@@ -988,17 +1001,19 @@ cudaError_t lm_associate(const DevPack &pk, const DevWork &wk, const DevParams &
                          int part, bool nn_folded) {
     cudaError_t e;
 #define TRY(x) do { e = (x); if (e != cudaSuccess) return e; } while (0)
-    const dim3 grid((unsigned)(pk.n_kf * wk.sub), (unsigned)n);
+    const dim3 grid((unsigned)(pk.n_sel * wk.sub), (unsigned)n);  // selection positions: unselected keyframes keep the cleared flags
     if (part != 2) {
         lm.ready = false;
         lm.sub = wk.sub;
         if (lm.clear_lanes) k_lm_clear<<<dim3((unsigned)((lm.slot_stride + 1023) / 1024 < 64 ? (lm.slot_stride + 1023) / 1024 : 64), (unsigned)n), 256, 0, st>>>(lm);
-        if (!(pr.plane_index && !pr.use_gpr))  // with the plane index there is no neighbourhood to search at the scan point
-            k_lm_knn_a<<<grid, kWarps * 32, 0, st>>>(pk, wk, pr, lm);
-        k_lm_plane_a<<<grid, 128, 0, st>>>(pk, wk, pr, lm);
+        if (pk.n_sel > 0) {
+            if (!(pr.plane_index && !pr.use_gpr))  // with the plane index there is no neighbourhood to search at the scan point
+                k_lm_knn_a<<<grid, kWarps * 32, 0, st>>>(pk, wk, pr, lm);
+            k_lm_plane_a<<<grid, 128, 0, st>>>(pk, wk, pr, lm);
+        }
         TRY(cudaGetLastError());
     }
-    if (part == 1) return cudaSuccess;
+    if (part == 1 || pk.n_sel == 0) return cudaSuccess;  // an empty selection: no blocks
     if (!nn_folded) k_lm_knn_b<<<grid, kWarps * 32, 0, st>>>(pk, wk, pr, lm, hints, cert);  // else K2a has filled nnb_pos / nbb_m
     k_lm_plane_b<<<grid, 128, 0, st>>>(pk, wk, pr, lm);
     TRY(cudaGetLastError());
@@ -1208,13 +1223,13 @@ cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, co
     // keypoint at most) — never from the counts themselves, so that the chunking, and with it the order
     // of the fp64 sums, is the same whether or not the host has looked at the counts; the kernels read
     // the exact counts from the device
-    const long long work = lm.max_blocks;
+    const long long work = pk.sel ? (pk.n_sel_mp > 0 ? pk.n_sel_mp : 1) : lm.max_blocks;  // a selection: what a pack of it would have
     long long chunks_ll = (work + kLinThreads * 2 - 1) / (kLinThreads * 2);
     // at most ONE wave of CTAs per candidate (2 CTAs of 255 registers per SM): 296 chunks measured 0.134 ms against 0.140 (592),
     // 0.163 (444: a wave and a half) and 0.157 (1184) at the KITTI-00 shape, and the finishing kernel sums four times fewer partials
     static const int kChunkCap = getenv("STL_LIN_CHUNKS") ? atoi(getenv("STL_LIN_CHUNKS")) : 148 * 2;
     int chunks = (int)(chunks_ll < 1 ? 1 : (chunks_ll > kChunkCap ? kChunkCap : chunks_ll));
-    const long long gwork = lm.use_gpr ? lm.max_blocks : 0;
+    const long long gwork = lm.use_gpr ? work : 0;
     long long gchunks_ll = gwork > 0 ? (gwork + 3) / 4 : 0;
     int gchunks = (int)(gchunks_ll > 148 * 8 ? 148 * 8 : gchunks_ll);
     const int stride = chunks + gchunks;

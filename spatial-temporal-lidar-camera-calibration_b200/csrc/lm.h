@@ -81,7 +81,7 @@ cudaError_t lm_begin(const DevPack &pk, const DevParams &pr, LmState &lm, int P,
 // Association lanes of the next lm_associate: lane j associates problem lanes[j].y from the K1 result (correspondences) at
 // workspace candidate slot lanes[j].x
 cudaError_t lm_set_lanes(LmState &lm, const int2 *lanes, int n, cudaStream_t st);
-// BuildProblem of the n lanes set by lm_set_lanes, all in the same launches (grid (n_kf * sub, n)).
+// BuildProblem of the n lanes set by lm_set_lanes, all in the same launches (grid (n_sel * sub, n): the selected keyframes).
 // hints: the workspace holds, at each lane's candidate slot, the 1-NN position an evaluation at the SAME extrinsic found for each
 // map point (DevWork::nn_pos) and, with cert, its lower bound of the squared distance to any other scan point (nn_g2): they
 // seed, or settle, the 3-D search.

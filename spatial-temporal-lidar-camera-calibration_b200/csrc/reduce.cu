@@ -17,7 +17,9 @@ __global__ void __launch_bounds__(kT) k_reduce(const DevPack pk, const DevWork w
     double v[STL_EVAL_NSUMS];
 #pragma unroll
     for (int i = 0; i < STL_EVAL_NSUMS; ++i) v[i] = 0;
-    for (int f = threadIdx.x; f < F; f += kT) {
+    // selection positions: the partial sums have the order of a pack holding only the selected keyframes
+    for (int i = threadIdx.x; i < pk.n_sel; i += kT) {
+        const int f = sel_kf(pk, i);
         const FrameRec r = wk.frame[(long long)b * F + f];
         v[0] += r.s2d; v[2] += r.she; v[3] += r.che; v[4] += r.c2d; v[5] += r.v2d; v[10] += r.kept; v[11] += r.ncorr;
         if (pr.w1 <= 1e-10) {  // iba_global.cpp:214-219: no 3-D term, one "valid" count per kept frame
@@ -46,12 +48,42 @@ __global__ void __launch_bounds__(kT) k_reduce(const DevPack pk, const DevWork w
     if (P.n > 1) p2p_allreduce_record(P, b, out + (long long)b * out_stride + P.off);  // keyframes sharded over GPUs: sum the shards here
 }
 
+// stl_eval_frames: one thread per selected (keyframe, candidate) folds FrameRec + AlignRec[sub] into the 13 values of
+// stl_debug_frame, in its order; with err_weight[1] <= 1e-10 the 3-D columns take k_reduce's "one valid count per kept frame"
+// instead, so that the rows of a candidate sum to its record.  out: [B][n_kf][13]; rows of unselected keyframes are not written.
+__global__ void __launch_bounds__(kT) k_frames(const DevPack pk, const DevWork wk, const DevParams pr, const int B, double *__restrict__ out) {
+    const long long t = (long long)blockIdx.x * kT + threadIdx.x;
+    if (t >= (long long)pk.n_sel * B) return;
+    const int i = (int)(t / B), b = (int)(t - (long long)i * B);
+    const long long rec = (long long)b * pk.n_kf + sel_kf(pk, i);
+    const FrameRec r = wk.frame[rec];
+    double *o = out + rec * 13;
+    o[0] = r.s2d; o[1] = r.v2d; o[2] = r.c2d; o[3] = r.she; o[4] = r.che; o[5] = r.kept; o[6] = r.ncorr; o[7] = r.nq;
+    double s3d = 0, v3d = 0, c3d = 0, vpl = 0, vpt = 0;
+    if (pr.w1 <= 1e-10) {
+        v3d = r.kept; c3d = r.kept;
+    } else {
+        for (int j = 0; j < wk.sub; ++j) {
+            const AlignRec a = wk.align[rec * wk.sub + j];
+            s3d += a.s3d; v3d += a.v3d; c3d += a.c3d; vpl += a.vpl; vpt += a.vpt;
+        }
+    }
+    o[8] = s3d; o[9] = v3d; o[10] = c3d; o[11] = vpl; o[12] = vpt;
+}
+
 }  // namespace
 
 cudaError_t launch_reduce(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, double *d_out, cudaStream_t st, int out_stride,
                           const P2pView *p2p) {
     if (B <= 0) return cudaSuccess;
     k_reduce<<<B, kT, 0, st>>>(pk, wk, pr, d_out, out_stride > 0 ? out_stride : STL_EVAL_NSUMS, p2p ? *p2p : P2pView());
+    return cudaGetLastError();
+}
+
+cudaError_t launch_frames(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, double *d_out, cudaStream_t st) {
+    const long long n = (long long)pk.n_sel * B;
+    if (n <= 0) return cudaSuccess;
+    k_frames<<<(unsigned)((n + kT - 1) / kT), kT, 0, st>>>(pk, wk, pr, B, d_out);
     return cudaGetLastError();
 }
 

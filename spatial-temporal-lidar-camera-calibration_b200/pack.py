@@ -113,6 +113,39 @@ class KeyFramePack:
             covis_valid=self.covis_valid[begin:end], covis_uv=self.covis_uv[k0:k1],
             he_Tc=self.he_Tc[begin:end], he_Tl=self.he_Tl[begin:end], he_valid=self.he_valid[begin:end])
 
+    def select(self, kf) -> "KeyFramePack":
+        """The keyframes ``kf`` (strictly increasing indices into this pack) as a self-contained pack: ``shard`` for any
+        index list, ``shard(b, e) == select(range(b, e))``.
+
+        Every keyframe keeps its own rows, its hand-eye pair (f, f+1) included as ``he_valid`` bakes it, whether or not f+1
+        is selected.  It is what a context computes over this pack after ``Context.select_keyframes(kf)``."""
+        k = np.asarray(kf)
+        if k.size == 0:
+            k = k.astype(np.int64).reshape(0)
+        if k.ndim != 1 or k.dtype.kind not in "iu":
+            raise TypeError("select: kf must be a 1-D list of integer keyframe indices")
+        k = k.astype(np.int64)
+        if k.size and (k[0] < 0 or k[-1] >= self.n_kf):
+            raise ValueError(f"select: keyframe indices must lie in [0, {self.n_kf})")
+        if np.any(np.diff(k) <= 0):
+            raise ValueError("select: keyframe indices must be strictly increasing")
+
+        def rows(off):  # row indices of the selected keyframes and their new offsets
+            n = off[k + 1] - off[k]
+            new_off = np.concatenate(([0], np.cumsum(n))).astype(np.int64)
+            return np.repeat(off[k] - new_off[:-1], n) + np.arange(new_off[-1], dtype=np.int64), new_off
+
+        pts, so = rows(self.scan_offset)
+        kps, ko = rows(self.kp_offset)
+        return KeyFramePack(
+            n_kf=int(k.size), n_covis=self.n_covis,
+            scan_offset=so, scan_xyz=self.scan_xyz[pts],
+            intrinsics=self.intrinsics[k], image_wh=self.image_wh[k],
+            kp_offset=ko, kp_xy=self.kp_xy[kps], kp_mappoint=self.kp_mappoint[kps],
+            Tcw=self.Tcw[k], covis_relpose=self.covis_relpose[k],
+            covis_valid=self.covis_valid[k], covis_uv=self.covis_uv[kps],
+            he_Tc=self.he_Tc[k], he_Tl=self.he_Tl[k], he_valid=self.he_valid[k])
+
     def to_npz_dict(self) -> dict:
         d = {f.name: getattr(self, f.name) for f in fields(self) if f.name not in ("n_kf", "n_covis")}
         d["n_kf"] = np.int64(self.n_kf)

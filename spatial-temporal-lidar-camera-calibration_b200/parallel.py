@@ -27,6 +27,20 @@ def shard_bounds(n_kf: int, world: int, rank: int) -> tuple[int, int]:
     return begin, begin + base + (1 if rank < rem else 0)
 
 
+def local_selection(global_kf, begin: int, end: int) -> np.ndarray:
+    """The part of a global keyframe selection that falls in the shard [begin, end), as the LOCAL indices
+    ``Context.select_keyframes`` takes on that rank (empty where the rank holds none of it: the rank still makes the call)."""
+    g = np.asarray(global_kf)
+    if g.size == 0:
+        g = g.astype(np.int64).reshape(0)
+    if g.ndim != 1 or g.dtype.kind not in "iu":
+        raise TypeError("local_selection: global_kf must be a 1-D list of integer keyframe indices")
+    g = g.astype(np.int64)
+    if np.any(np.diff(g) <= 0) or (g.size and g[0] < 0):
+        raise ValueError("local_selection: global keyframe indices must be non-negative and strictly increasing")
+    return (g[(g >= begin) & (g < end)] - begin).astype(np.int32)
+
+
 def attach_communicator(ctx, rank: int, world: int, exchange=None, id_file: str | None = None, timeout_s: float = 120.0):
     """Attaches an NCCL communicator of `world` ranks to `ctx` (which must hold keyframe shard `rank`).
 
