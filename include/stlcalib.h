@@ -213,7 +213,20 @@ int32_t stl_abi_version(void);
 
 /* Copies the pack to HBM and builds the per-scan 3-D index (replaces the
  * KDTree3D-per-scan build, iba_global.cpp:362-367).  May be called again to
- * replace the pack. */
+ * replace the pack.
+ *
+ * Size limits.  A scan holds at most 2^20 points, an image at most 16384 px
+ * per side and a keyframe at most 65535 keypoints, but the binding rule is
+ * tighter: the K1 tables of the largest keyframe must fit the device's opt-in
+ * shared memory per block.  They take 26 B per keypoint (pixel, grid slot,
+ * map-point bit, per-keypoint best match) plus the 2 px keypoint bitmap
+ * (4 B x ceil((ceil(W/2) + 3) / 32) words x (ceil(H/2) + 3) rows), the 8 px
+ * cell grid (2 B per cell) and 2.25 B per 128 points of the largest scan.
+ * Measured on an NVIDIA B200 (227 KB opt-in shared memory, 1000 W power
+ * limit), 2 keyframes of ~38 k-point scans: 1241 x 376 admits 7694 keypoints,
+ * 1920 x 1080 admits 3782; a 3840 x 2160 image admits none (its bitmap alone
+ * is 264 KB).  A pack over the limit is refused with STL_ERR_CAPACITY and the
+ * previously uploaded pack stays in place. */
 stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *pack);
 
 /* ---- Nomad / iba_func path ------------------------------------------- */

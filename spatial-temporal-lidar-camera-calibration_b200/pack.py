@@ -90,7 +90,13 @@ class KeyFramePack:
                  "covis_relpose": F * Cc * 12, "covis_valid": F * Cc, "covis_uv": nk * Cc * 2}
         kw = {}
         for name, _ in _abi.Pack._fields_[2:]:
-            a = np.ctypeslib.as_array(getattr(p, name), shapes[name])
+            ptr = getattr(p, name)
+            if not ptr:  # stl_pack_t allows NULL for empty members (no keypoints, n_covis = 0)
+                if sizes.get(name, 1) != 0:
+                    raise ValueError(f"stl_pack_t.{name} is NULL")
+                kw[name] = np.zeros(0, _SPEC[name])
+                continue
+            a = np.ctypeslib.as_array(ptr, shapes[name])
             a = a[: sizes.get(name, a.size)]
             kw[name] = a.copy() if copy else a
         return cls(n_kf=F, n_covis=Cc, **kw)
