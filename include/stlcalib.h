@@ -225,9 +225,41 @@ int32_t stl_abi_version(void);
  * Measured on an NVIDIA B200 (227 KB opt-in shared memory, 1000 W power
  * limit), 2 keyframes of ~38 k-point scans: 1241 x 376 admits 7694 keypoints,
  * 1920 x 1080 admits 3782; a 3840 x 2160 image admits none (its bitmap alone
- * is 264 KB).  A pack over the limit is refused with STL_ERR_CAPACITY and the
- * previously uploaded pack stays in place. */
+ * is 264 KB).  By default a pack over the limit is refused with
+ * STL_ERR_CAPACITY and the previously uploaded pack stays in place; with
+ * stl_allow_oversize_keyframes(ctx, 1) it is accepted (see there), and only
+ * the 65535-keypoint, 16384 px and 2^20-point limits remain. */
 stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *pack);
+
+/* Oversize keyframes.  allow = 1 lets the NEXT stl_upload_pack accept keyframes
+ * whose K1 tables do not fit the shared memory of the one-kernel K1; they run
+ * on a banded three-kernel K1 whose shared memory does not grow with the image
+ * (DESIGN.md §3 "Oversize keyframes"), with bit for bit the results the
+ * one-kernel K1 would give.  allow = 0 (the default) refuses such a pack as
+ * before.  The call does not touch the resident pack; allow other than 0 / 1
+ * -> STL_ERR_INVALID.
+ *
+ * Routing rule.  The one-kernel K1 keeps a "fitting" set of keyframes whose
+ * maxima of keypoints, table bytes and 128-point groups fit the opt-in limit
+ * (a sum of maxima, not a maximum of sums).  Keyframes leave that set
+ * largest-first, by the shared memory each would need alone (ties: the lower
+ * index first), until the set's maxima fit; those that left are the oversize
+ * keyframes.  With none the fitting set is the whole pack and nothing changes.
+ *
+ * Cost: each band of bitmap rows (floor(4096 / words per row) rows, at most
+ * 16 KB) streams the scan cells that can project into it, and the K1 keeps its
+ * per-keypoint tables, survivors and matches in a workspace sized per
+ * (candidate, oversize keyframe): 16 B per keypoint, and per keyframe
+ * S = max(4096, min(2 n_kp rounded up to 256, padded scan points)) survivor
+ * slots of 4 B and 2 S match slots of 16 B.  A unit that finds more survivors
+ * than S falls back to the exact pass over every point (correct, slower;
+ * work counter [6]). */
+stl_status_t stl_allow_oversize_keyframes(stl_ctx_t *ctx, int32_t allow);
+
+/* Local keyframes of the resident pack that run on the oversize path, in
+ * increasing order: up to `cap` of them into kf (may be NULL), their count in
+ * *n (even if > cap).  No pack -> STL_ERR_STATE. */
+stl_status_t stl_oversize_keyframes(stl_ctx_t *ctx, int32_t *kf, int32_t cap, int32_t *n);
 
 /* ---- Nomad / iba_func path ------------------------------------------- */
 

@@ -111,6 +111,16 @@ class Context {
         check(stl_select_keyframes(ctx_, kf.empty() ? &none : kf.data(), (int32_t)kf.size()), "stl_select_keyframes");
     }
     void select_all() { check(stl_select_keyframes(ctx_, nullptr, 0), "stl_select_keyframes"); }
+    // oversize keyframes (stl_allow_oversize_keyframes): read by the next upload; the resident pack is not touched
+    void allow_oversize_keyframes(bool allow) { check(stl_allow_oversize_keyframes(ctx_, allow ? 1 : 0), "stl_allow_oversize_keyframes"); }
+    // local keyframes of the resident pack on the oversize path, increasing
+    std::vector<int32_t> oversize_keyframes() {
+        int32_t n = 0;
+        check(stl_oversize_keyframes(ctx_, nullptr, 0, &n), "stl_oversize_keyframes");
+        std::vector<int32_t> kf((size_t)n);
+        if (n > 0) check(stl_oversize_keyframes(ctx_, kf.data(), n, &n), "stl_oversize_keyframes");
+        return kf;
+    }
     // BAError per keyframe: [B][n_kf][13] records of stl_debug_frame's layout (zero rows for unselected keyframes); n_kf = the pack's
     std::vector<double> eval_frames(const double *x, int B, int n_kf) {
         std::vector<double> out((size_t)B * (size_t)n_kf * 13);

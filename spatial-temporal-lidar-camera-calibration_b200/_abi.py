@@ -172,6 +172,8 @@ CALIB_SYMBOLS = {
     "stl_comm_stats": (C.c_int, [_vp, _i64p]),
     "stl_select_keyframes": (C.c_int, [_vp, _i32p, C.c_int32]),
     "stl_eval_frames": (C.c_int, [_vp, _dp, C.c_int32, _dp]),
+    "stl_allow_oversize_keyframes": (C.c_int, [_vp, C.c_int32]),
+    "stl_oversize_keyframes": (C.c_int, [_vp, _i32p, C.c_int32, _i32p]),
     "stl_debug_corrset": (C.c_int, [_vp, C.c_int32, C.c_int32, _u32p, _u32p, C.c_int32, _i32p]),
     "stl_debug_align": (C.c_int, [_vp, C.c_int32, C.c_int32, _u32p, _u32p, _i32p, _i32p, _dp, _u32p,
                                   C.c_int32, _i32p]),

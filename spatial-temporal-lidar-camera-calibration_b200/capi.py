@@ -82,6 +82,22 @@ class Context:
         self.n_blocks = None
         self.n_problems = 0
 
+    def allow_oversize_keyframes(self, flag: bool):
+        """Let the next :meth:`upload` accept keyframes whose K1 tables do not fit the one-kernel K1's shared memory (4K
+        images, many keypoints); they run on the banded three-kernel K1 with the same results.  False (the default) refuses
+        such a pack.  The resident pack is not touched."""
+        if not (isinstance(flag, (bool, np.bool_)) or (isinstance(flag, (int, np.integer)) and flag in (0, 1))):
+            raise TypeError("allow_oversize_keyframes: flag must be a bool (or 0 / 1)")
+        _check(self.lib, self.h, self.lib.stl_allow_oversize_keyframes(self.h, 1 if flag else 0))
+
+    def oversize_keyframes(self) -> np.ndarray:
+        """Local keyframes of the resident pack that run on the oversize path, increasing (int32)."""
+        n = C.c_int32(0)
+        _check(self.lib, self.h, self.lib.stl_oversize_keyframes(self.h, None, 0, C.byref(n)))
+        out = np.zeros(max(n.value, 1), dtype=np.int32)
+        _check(self.lib, self.h, self.lib.stl_oversize_keyframes(self.h, out.ctypes.data_as(_abi._i32p), int(out.size), C.byref(n)))
+        return out[: n.value].copy()
+
     def eval_frames(self, x) -> np.ndarray:
         """x [B,7] -> the per-keyframe record of BAError [B, n_kf, 13] (the 13 values of :meth:`debug_frame`, in its order) of
         every keyframe of the pack; rows of unselected keyframes are zero.  Each rank returns its own keyframes."""

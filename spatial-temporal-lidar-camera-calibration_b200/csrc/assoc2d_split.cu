@@ -1,17 +1,21 @@
-// assoc2d_split.cu — K1 as three kernels (selected by STL_K1_SPLIT=1; the default is the one-kernel form, assoc2d.cu).
-// Status: bit-identical results (the whole GPU suite passes with it), but 13 % SLOWER than the one-kernel form at the
-// KITTI-00 shape — k_stream 0.152 ms (instruction-bound, 80 % issue), k_exact 0.213 ms and k_corr 0.137 ms (both bound by
-// chains of dependent L2 / DRAM round trips at 23 % issue), against 0.447 ms in one kernel.  What would make it win is
-// listed in profiles/r02_negative_results.txt.
+// assoc2d_split.cu — K1 as three kernels, for the keyframes whose K1 tables do not fit the one-kernel K1's shared memory
+// (stl_allow_oversize_keyframes; STL_K1_OVERSIZE=all or STL_K1_SPLIT=1 route every keyframe here).  Nothing it keeps in
+// shared memory grows with the image: the stream holds one BAND of the keypoint bitmap (kK1BandWords), and the exact and
+// correspondence passes keep their per-keypoint tables in global memory.
+// Status: bit-identical results to the one-kernel form (assoc2d.cu), but 13 % SLOWER than it at the KITTI-00 shape when
+// routed there — k_stream 0.152 ms (instruction-bound, 80 % issue), k_exact 0.213 ms and k_corr 0.137 ms (both bound by
+// chains of dependent L2 / DRAM round trips at 23 % issue), against 0.447 ms in one kernel (profiles/r02_negative_results.txt).
 //
 // Same result as k_assoc2d (assoc2d.cu), i.e. per (candidate, keyframe):
 //   TransformPointCloud + FindProjectCorrespondences   include/pointcloud.h:82-86, src/examples/iba_global.cpp:55-96
 //   frame gate, hand-eye term, covisible term           src/examples/iba_global.cpp:203,264-276,291-328
 // but every phase runs on the grid shape that suits it:
-//   K1a k_stream   S CTAs per unit stream the scan (SoA float4 loads, 12 B/point) through the float32 pre-cull and the
-//                  keypoint bitmap — nothing else lives in the CTA (bitmap + group list + a local survivor list, ~25 KB
-//                  of shared memory), so six CTAs fit an SM and the stream runs at HBM speed.  Survivors (1-2 % of the
-//                  points) go to a per-unit list in global memory (L2).
+//   K1a k_stream   bands x S CTAs per unit stream the scan (SoA float4 loads, 12 B/point) through the float32 pre-cull and
+//                  the keypoint bitmap.  A CTA holds one band of bitmap rows, culls the KD cells with the v-range of its
+//                  band, and tests a point's bit only when the point's cell row falls in its band (the bitmap is dilated
+//                  by max_pixel_dist + 0.25 px, so every point is decided in exactly one band; the z < zmin slab goes to
+//                  the exact pass from band 0).  Band + group list + a local survivor list stay under ~49 KB of shared
+//                  memory, so four CTAs fit an SM.  Survivors (1-2 % of the points) go to a per-unit list in global memory.
 //   K1b k_exact    one THREAD per survivor: the reference's exact fp64 projection, the keypoints of the 8 px grid cells
 //                  around it, atomicMin of the squared distance per keypoint on a table in global memory (L2 atomics),
 //                  every match appended to the unit's match list.
@@ -38,7 +42,7 @@ constexpr int kCorrThreads = 256;
 // two of its threads, so that STL_K1_SPLIT=1 changes no bit of the record
 constexpr int kTermLanes = 512;
 static_assert(kTermLanes == 2 * kCorrThreads, "k_corr plays two threads of the one-kernel K1 each");
-constexpr int kLocalSurv = kK1SurvCap;  // survivors a stream CTA can hold (flushed once, at its end)
+constexpr int kLocalSurv = kK1SurvCap;  // survivors a stream CTA holds in shared memory (flushed once, at its end; beyond: straight to the unit's list)
 constexpr unsigned long long kNoKey = 0xffffffffffffffffull;
 
 struct Fast {  // float32 projection rows, error bounds and the culling half-spaces of one (candidate, keyframe)
@@ -111,34 +115,56 @@ struct UnitCnt { int n_surv, n_match, overflow, pad; };
 // ------------------------------------------------------------------------------------------------ K1a
 struct StreamSmem {
     Fast F;
-    int n_groups, next_group, n_local, overflow, flush_base;
+    int n_groups, next_group, n_local, flush_base;
 };
 
-// grid: ((keyframe * B + candidate) * S + sub)
+// The cull of band [r0, r1) of bitmap rows: cell row cv = floor(v / kBmCell) + 1 covers v in [kBmCell (cv - 1), kBmCell cv), so
+// the band's points have v in [kBmCell (r0 - 1), kBmCell (r1 - 1)); the v half-spaces are moved to that range widened by one
+// cell on either side, the margin the image range itself has (-kBmCell, H + kBmCell).  The first and last band keep the
+// image's own bounds; the thresholds stay those of the slab z <= zmin (conservative for every band, exact for band 0).
+__device__ void narrow_to_band(Fast &S, int r0, int r1, int rows) {
+    const float rzx = S.mz[0], rzy = S.mz[1], rzz = S.mz[2], rzw = S.mz[3];
+    if (r0 > 0) {
+        const float vl = (float)(kBmCell * (r0 - 2));
+        S.plane[3] = make_float4(S.mv[0] - vl * rzx, S.mv[1] - vl * rzy, S.mv[2] - vl * rzz, S.mv[3] - vl * rzw);
+    }
+    if (r1 < rows) {
+        const float vh = fminf((float)(kBmCell * r1), S.v_hi);
+        S.plane[4] = make_float4(vh * rzx - S.mv[0], vh * rzy - S.mv[1], vh * rzz - S.mv[2], vh * rzw - S.mv[3]);
+    }
+}
+
+// grid: ((unit * max_bands + band) * S + sub), unit = oversize selection position * B + candidate; CTAs of bands the
+// keyframe does not have leave at once
 __global__ void __launch_bounds__(kStreamThreads, 6)
-k_stream(const DevPack pk, const DevWork wk, const int B, const int S_sub) {
+k_stream(const DevPack pk, const DevWork wk, const int B, const int S_sub, const int max_bands) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int sub = blockIdx.x % S_sub, unit = blockIdx.x / S_sub;
-    const int fi = unit / B, f = sel_kf(pk, fi), b = unit - fi * B;
-    const DevKf K = pk.kf[f];
+    const int sub = blockIdx.x % S_sub, ub = blockIdx.x / S_sub, band = ub % max_bands, unit = ub / max_bands;
+    const int oi = unit / B, b = unit - oi * B, o = pk.ov_sel[oi];
+    const OvKf O = pk.ov[o];
+    if (band >= O.n_bands) return;
+    const DevKf K = pk.kf[O.f];
     const DevCand &c = wk.cand[b];
+    const int wpr = K.bm_wpr, band_rows = k1_band_rows(wpr), r0 = band * band_rows, r1 = min(r0 + band_rows, K.bm_rows);
     StreamSmem &S = *reinterpret_cast<StreamSmem *>(smem_raw);
     unsigned char *p = smem_raw + ((sizeof(StreamSmem) + 15) & ~size_t(15));
-    uint32_t *bm = reinterpret_cast<uint32_t *>(p); p += 4 * (size_t)K.bm_wpr * K.bm_rows;
+    // the band's words, then the lists: at most min(band_rows, bm_rows) rows, as assoc2d_split_smem_bytes is given
+    uint32_t *bm = reinterpret_cast<uint32_t *>(p); p += 4 * (size_t)wpr * min(band_rows, K.bm_rows);
     uint32_t *surv = reinterpret_cast<uint32_t *>(p); p += 4 * (size_t)kLocalSurv;
     unsigned short *groups = reinterpret_cast<unsigned short *>(p);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const long long urec = (long long)b * pk.n_kf + f;
-    UnitCnt *cnt = reinterpret_cast<UnitCnt *>(wk.k1_cnt) + urec;
-    uint32_t *gsurv = wk.k1_surv + urec * kK1SurvCap;
+    UnitCnt *cnt = reinterpret_cast<UnitCnt *>(wk.k1_cnt) + (long long)b * pk.n_ov + o;
+    uint32_t *gsurv = wk.k1_surv + (long long)b * pk.n_ov_surv + O.surv_off;
+    const int surv_cap = O.surv_cap;
 
     if (tid == 0) {
         make_fast(K, c, S.F);
-        S.n_groups = 0; S.next_group = 0; S.n_local = 0; S.overflow = 0; S.flush_base = 0;
+        narrow_to_band(S.F, r0, r1, K.bm_rows);
+        S.n_groups = 0; S.next_group = 0; S.n_local = 0; S.flush_base = 0;
     }
     {
-        const uint32_t *bmg = pk.bitmap + K.bm_off;
-        const int nw = K.bm_wpr * K.bm_rows;
+        const uint32_t *bmg = pk.bitmap + K.bm_off + (long long)r0 * wpr;
+        const int nw = (r1 - r0) * wpr;
         for (int i = tid; i < nw; i += kStreamThreads) bm[i] = bmg[i];
     }
     __syncthreads();
@@ -169,7 +195,8 @@ k_stream(const DevPack pk, const DevWork wk, const int B, const int S_sub) {
         const float mv0 = F.mv[0], mv1 = F.mv[1], mv2 = F.mv[2], mv3 = F.mv[3];
         const float mz0 = F.mz[0], mz1 = F.mz[1], mz2 = F.mz[2], mz3 = F.mz[3];
         const float zmin = F.zmin, u_hi = F.u_hi, v_hi = F.v_hi, lo = -(float)kBmCell, ezs = F.ez, ubu = F.ub_u, ubv = F.ub_v;
-        const int wpr = K.bm_wpr, cu_max = K.bm_wpr * 32 - 1, cv_max = K.bm_rows - 1;
+        const int cu_max = wpr * 32 - 1, cv_max = K.bm_rows - 1;
+        const bool slab = band == 0;  // the z < zmin slab is passed to the exact pass by the first band only
         const float4 *X = reinterpret_cast<const float4 *>(pk.px + K.pt_off);
         const float4 *Y = reinterpret_cast<const float4 *>(pk.py + K.pt_off);
         const float4 *Z = reinterpret_cast<const float4 *>(pk.pz + K.pt_off);
@@ -206,9 +233,9 @@ k_stream(const DevPack pk, const DevWork wk, const int B, const int S_sub) {
                         const float inv = __frcp_rn(zc);
                         const int cu = min(max((int)floorf(uz * inv * (1.0f / kBmCell)) + 1, 0), cu_max);
                         const int cv = min(max((int)floorf(vz * inv * (1.0f / kBmCell)) + 1, 0), cv_max);
-                        pass = (bm[cv * wpr + (cu >> 5)] >> (cu & 31)) & 1u;
+                        pass = cv >= r0 && cv < r1 && ((bm[(cv - r0) * wpr + (cu >> 5)] >> (cu & 31)) & 1u);
                     }
-                } else if (zc > -ezs) {
+                } else if (slab && zc > -ezs) {
                     pass = fabsf(uz) <= ubu && fabsf(vz) <= ubv;
                 }
                 pm |= (pass ? 1u : 0u) << e;
@@ -228,8 +255,13 @@ k_stream(const DevPack pk, const DevWork wk, const int B, const int S_sub) {
 #pragma unroll
                 for (int e = 0; e < 4; ++e)
                     if ((pm >> e) & 1u) {
-                        if (pos < kLocalSurv) surv[pos] = (uint32_t)(i * 4 + e);
-                        else S.overflow = 1;
+                        if (pos < kLocalSurv) {
+                            surv[pos] = (uint32_t)(i * 4 + e);
+                        } else {  // the CTA's list is full: straight to the unit's list
+                            const int g = atomicAdd(&cnt->n_surv, 1);
+                            if (g < surv_cap) gsurv[g] = (uint32_t)(i * 4 + e);
+                            else atomicExch(&cnt->overflow, 1);
+                        }
                         ++pos;
                     }
             }
@@ -242,12 +274,12 @@ k_stream(const DevPack pk, const DevWork wk, const int B, const int S_sub) {
     if (tid == 0) {
         const int base = atomicAdd(&cnt->n_surv, nl);
         S.flush_base = base;
-        if (S.overflow || base + nl > kK1SurvCap) atomicExch(&cnt->overflow, 1);
+        if (base + nl > surv_cap) atomicExch(&cnt->overflow, 1);
     }
     __syncthreads();
     const int fb = S.flush_base;
     for (int s = tid; s < nl; s += kStreamThreads)
-        if (fb + s < kK1SurvCap) gsurv[fb + s] = surv[s];
+        if (fb + s < surv_cap) gsurv[fb + s] = surv[s];
 }
 
 // ------------------------------------------------------------------------------------------------ K1b
@@ -269,7 +301,7 @@ __device__ __forceinline__ bool exact_project(const DevCand &c, double fx, doubl
 // PASS 1: atomicMin of the squared distance per keypoint + match list; PASS 2 (match list overflowed): ties by recomputation
 template <int PASS>
 __device__ __forceinline__ void exact_point(const DevPack &pk, const DevKf &K, const DevCand &c, const DevParams &pr, unsigned long long *best_d2,
-                                            unsigned long long *best_key, uint32_t si, ulonglong2 *__restrict__ matches, int *n_match) {
+                                            unsigned long long *best_key, uint32_t si, ulonglong2 *__restrict__ matches, int *n_match, int match_cap) {
     const long long g = K.pt_off + si;
     const float xf = pk.px[g], yf = pk.py[g], zf = pk.pz[g];
     double u, v;
@@ -295,7 +327,7 @@ __device__ __forceinline__ void exact_point(const DevPack &pk, const DevKf &K, c
                 if (PASS == 1) {
                     atomicMin(&best_d2[k], bits);
                     const int slot = atomicAdd(n_match, 1);
-                    if (slot < kK1MatchCap) matches[slot] = make_ulonglong2(bits, ((unsigned long long)k << 32) | si);
+                    if (slot < match_cap) matches[slot] = make_ulonglong2(bits, ((unsigned long long)k << 32) | si);
                 } else if (bits == __ldcg(&best_d2[k])) {
                     atomicMin(&best_key[k], ((unsigned long long)pk.orig[g] << 32) | si);
                 }
@@ -308,20 +340,20 @@ __device__ __forceinline__ void exact_point(const DevPack &pk, const DevKf &K, c
 __global__ void __launch_bounds__(kExactThreads)
 k_exact(const DevPack pk, const DevWork wk, const DevParams pr, const int B) {
     const int unit = blockIdx.x;
-    const int fi = unit / B, f = sel_kf(pk, fi), b = unit - fi * B;
-    const long long urec = (long long)b * pk.n_kf + f;
-    UnitCnt *cnt = reinterpret_cast<UnitCnt *>(wk.k1_cnt) + urec;
-    const DevKf K = pk.kf[f];
+    const int oi = unit / B, b = unit - oi * B, o = pk.ov_sel[oi];
+    const OvKf O = pk.ov[o];
+    UnitCnt *cnt = reinterpret_cast<UnitCnt *>(wk.k1_cnt) + (long long)b * pk.n_ov + o;
+    const DevKf K = pk.kf[O.f];
     const bool ovf = cnt->overflow != 0;
-    const int ns = ovf ? K.n_pts : min(cnt->n_surv, kK1SurvCap);
+    const int ns = ovf ? K.n_pts : min(cnt->n_surv, O.surv_cap);
     const int first = blockIdx.y * kExactThreads + threadIdx.x;
     if (first >= ns) return;
     const DevCand &c = wk.cand[b];
-    const uint32_t *gsurv = wk.k1_surv + urec * kK1SurvCap;
-    unsigned long long *best_d2 = wk.k1_best_d2 + (long long)b * pk.n_kp_total + K.kp_off;
-    ulonglong2 *matches = wk.k1_match + urec * kK1MatchCap;
+    const uint32_t *gsurv = wk.k1_surv + (long long)b * pk.n_ov_surv + O.surv_off;
+    unsigned long long *best_d2 = wk.k1_best_d2 + (long long)b * pk.n_ov_kp + O.kp_off;
+    ulonglong2 *matches = wk.k1_ov_match + (long long)b * pk.n_ov_match + O.match_off;
     for (int s = first; s < ns; s += gridDim.y * kExactThreads)
-        exact_point<1>(pk, K, c, pr, best_d2, nullptr, ovf ? (uint32_t)s : gsurv[s], matches, &cnt->n_match);
+        exact_point<1>(pk, K, c, pr, best_d2, nullptr, ovf ? (uint32_t)s : gsurv[s], matches, &cnt->n_match, O.match_cap);
 }
 
 // ------------------------------------------------------------------------------------------------ K1c
@@ -357,15 +389,17 @@ __global__ void __launch_bounds__(kCorrThreads)
 k_corr(const DevPack pk, const DevWork wk, const DevParams pr, const int B, const int with_terms) {
     __shared__ CorrSmem S;
     const int unit = blockIdx.x;
-    const int fi = unit / B, f = sel_kf(pk, fi), b = unit - fi * B;
-    const long long urec = (long long)b * pk.n_kf + f;
-    UnitCnt *cnt = reinterpret_cast<UnitCnt *>(wk.k1_cnt) + urec;
+    const int oi = unit / B, b = unit - oi * B, o = pk.ov_sel[oi];
+    const OvKf O = pk.ov[o];
+    const int f = O.f;
+    const long long urec = (long long)b * pk.n_kf + f;  // the records every K1 writes
+    UnitCnt *cnt = reinterpret_cast<UnitCnt *>(wk.k1_cnt) + (long long)b * pk.n_ov + o;
     const DevKf K = pk.kf[f];
     const DevCand &c = wk.cand[b];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    unsigned long long *best_d2 = wk.k1_best_d2 + (long long)b * pk.n_kp_total + K.kp_off;
-    unsigned long long *best_key = wk.k1_best_key + (long long)b * pk.n_kp_total + K.kp_off;
-    const ulonglong2 *matches = wk.k1_match + urec * kK1MatchCap;
+    unsigned long long *best_d2 = wk.k1_best_d2 + (long long)b * pk.n_ov_kp + O.kp_off;
+    unsigned long long *best_key = wk.k1_best_key + (long long)b * pk.n_ov_kp + O.kp_off;
+    const ulonglong2 *matches = wk.k1_ov_match + (long long)b * pk.n_ov_match + O.match_off;
     const int C = pk.n_covis;
     if (tid >= 32 && tid < 32 + C) {
         const int j = tid - 32;
@@ -378,7 +412,7 @@ k_corr(const DevPack pk, const DevWork wk, const DevParams pr, const int B, cons
 
     // ---- ties: among the recorded matches, the ones at the minimum compete on (original index, position)
     const int nm = cnt->n_match;
-    if (nm <= kK1MatchCap) {
+    if (nm <= O.match_cap) {
         for (int i = tid; i < nm; i += kCorrThreads) {
             const ulonglong2 m = matches[i];
             const uint32_t k = (uint32_t)(m.y >> 32), si = (uint32_t)(m.y & 0xffffffffu);
@@ -386,10 +420,10 @@ k_corr(const DevPack pk, const DevWork wk, const DevParams pr, const int B, cons
         }
     } else {  // match list overflowed: recompute
         const bool ovf = cnt->overflow != 0;
-        const int ns = ovf ? K.n_pts : min(cnt->n_surv, kK1SurvCap);
-        const uint32_t *gsurv = wk.k1_surv + urec * kK1SurvCap;
+        const int ns = ovf ? K.n_pts : min(cnt->n_surv, O.surv_cap);
+        const uint32_t *gsurv = wk.k1_surv + (long long)b * pk.n_ov_surv + O.surv_off;
         for (int s = tid; s < ns; s += kCorrThreads)
-            exact_point<2>(pk, K, c, pr, best_d2, best_key, ovf ? (uint32_t)s : gsurv[s], nullptr, nullptr);
+            exact_point<2>(pk, K, c, pr, best_d2, best_key, ovf ? (uint32_t)s : gsurv[s], nullptr, nullptr, 0);
     }
     __threadfence_block();
     __syncthreads();
@@ -499,8 +533,8 @@ k_corr(const DevPack pk, const DevWork wk, const DevParams pr, const int B, cons
 
 }  // namespace
 
-size_t assoc2d_split_smem_bytes(int max_bm_words, int max_groups) {
-    return ((sizeof(StreamSmem) + 15) & ~size_t(15)) + (size_t)max_bm_words * 4 + (size_t)kLocalSurv * 4 + 2 * (size_t)max_groups + 16;
+size_t assoc2d_split_smem_bytes(int max_band_words, int max_groups) {
+    return ((sizeof(StreamSmem) + 15) & ~size_t(15)) + (size_t)max_band_words * 4 + (size_t)kLocalSurv * 4 + 2 * (size_t)max_groups + 16;
 }
 
 cudaError_t assoc2d_split_configure(size_t smem) {
@@ -517,24 +551,27 @@ cudaError_t assoc2d_split_configure(size_t smem) {
     return e;
 }
 
-cudaError_t launch_assoc2d_split(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, size_t smem, int max_pts, cudaStream_t st,
-                                 int with_terms) {
-    if (B <= 0 || pk.n_sel <= 0) return cudaSuccess;
-    const long long units = (long long)pk.n_sel * B;  // unit = selection position * B + candidate
-    // per-unit counters (indexed by the pack's keyframe) and the per-keypoint tables start empty (all-ones = "no value": larger
+cudaError_t launch_assoc2d_split(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, size_t smem, int max_bands, int max_surv_cap,
+                                 cudaStream_t st, int with_terms) {
+    if (B <= 0 || pk.n_ov_sel <= 0) return cudaSuccess;
+    const long long units = (long long)pk.n_ov_sel * B;  // unit = oversize selection position * B + candidate
+    // per-unit counters and the per-keypoint tables (indexed by oversize ordinal) start empty (all-ones = "no value": larger
     // than any distance / key)
-    cudaError_t e = cudaMemsetAsync(wk.k1_cnt, 0, sizeof(UnitCnt) * (size_t)pk.n_kf * B, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(wk.k1_best_d2, 0xff, 8 * (size_t)pk.n_kp_total * B, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(wk.k1_best_key, 0xff, 8 * (size_t)pk.n_kp_total * B, st);
+    cudaError_t e = cudaMemsetAsync(wk.k1_cnt, 0, sizeof(UnitCnt) * (size_t)pk.n_ov * B, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(wk.k1_best_d2, 0xff, 8 * (size_t)pk.n_ov_kp * B, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(wk.k1_best_key, 0xff, 8 * (size_t)pk.n_ov_kp * B, st);
     if (e != cudaSuccess) return e;
-    // few units (a keyframe shard of a multi-GPU run, one candidate): more CTAs per unit keep the SMs busy
+    // few (unit, band) pairs (a keyframe shard of a multi-GPU run, one candidate): more CTAs per pair keep the SMs busy
+    const long long ub = units * max_bands;
     int S_sub = 2;
-    while (S_sub < 8 && units * S_sub < 148 * 6 * 2) S_sub *= 2;
+    while (S_sub < 8 && ub * S_sub < 148 * 6 * 2) S_sub *= 2;
     if (const char *e2 = getenv("STL_K1_SUB")) S_sub = max(1, min(8, atoi(e2)));  // diagnostic
-    k_stream<<<(unsigned)(units * S_sub), kStreamThreads, smem, st>>>(pk, wk, B, S_sub);
-    // survivors are 1-2 % of the points: two chunks of 256 threads cover the usual unit, the loop the rest
-    (void)max_pts;
-    k_exact<<<dim3((unsigned)units, 4), kExactThreads, 0, st>>>(pk, wk, pr, B);
+    if (ub * S_sub > 0x7fffffffll) return cudaErrorInvalidValue;
+    k_stream<<<(unsigned)(ub * S_sub), kStreamThreads, smem, st>>>(pk, wk, B, S_sub, max_bands);
+    // survivors are 1-2 % of the points: four chunks of 256 threads cover the usual unit (kK1SurvCap), one more per
+    // 1024 survivor slots the larger ones, the loop the rest
+    const int ychunks = max(4, min(32, (max_surv_cap + 1023) / 1024));
+    k_exact<<<dim3((unsigned)units, ychunks), kExactThreads, 0, st>>>(pk, wk, pr, B);
     k_corr<<<(unsigned)units, kCorrThreads, 0, st>>>(pk, wk, pr, B, with_terms);
     return cudaGetLastError();
 }

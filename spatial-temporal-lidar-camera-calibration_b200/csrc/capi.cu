@@ -42,9 +42,19 @@ struct stl_ctx {
     float adj_r2 = 0.f;  // squared radius of the leaf adjacency lists, rounded up (0: none)
     DevPack pk;
     std::vector<DevKf> h_kf;
-    int max_kp = 0, max_bm_words = 0, max_tab = 0, max_groups = 0, n_sm = 0;
+    int max_kp = 0, max_tab = 0, max_groups = 0, n_sm = 0;  // maxima over the fitting keyframes (the one-kernel K1's shared memory)
     size_t k1_smem = 0, k1_split_smem = 0;
-    bool k1_mono = true;   // the one-kernel K1 (assoc2d.cu); STL_K1_SPLIT=1 selects the three-kernel form (assoc2d_split.cu)
+    // K1 routing (DESIGN §3 "Oversize keyframes"): the one-kernel K1 (assoc2d.cu) runs the fitting keyframes, the banded
+    // three-kernel K1 (assoc2d_split.cu) the oversize ones (pk.ov); STL_K1_OVERSIZE=all / STL_K1_SPLIT=1 route every keyframe there
+    bool allow_oversize = false;   // stl_allow_oversize_keyframes: read by the next upload
+    int n_fit = 0;                 // fitting keyframes of the pack
+    std::vector<int> ov_kf;        // oversize keyframes of the pack, increasing (position = oversize ordinal)
+    OvKf *d_ov = nullptr;          // [n_ov]
+    int *d_route = nullptr;        // [2][n_kf]: the fitting keyframes, then the oversize ordinals, of the whole pack
+    int *d_route_sel = nullptr;    // [2][n_kf]: the same lists restricted to the current selection
+    const int *fit_sel = nullptr;  // the one-kernel K1's keyframe list (into d_route or d_route_sel); unused without oversize keyframes
+    int n_fit_sel = 0;
+    int ov_max_bands = 0, ov_max_surv = 0;
     long long n_pts_total = 0;
     // keyframe selection (stl_select_keyframes): pk.sel / pk.sel_mp point into these while a subset is selected
     std::vector<uint8_t> sel_mask;        // [n_kf] 1 = selected
@@ -136,6 +146,8 @@ void free_pack(stl_ctx *c) {
     dfree(p.relpose); dfree(p.covis_valid); dfree(p.covis_uv); dfree(p.he_Tc); dfree(p.he_Tl);
     p = DevPack();
     dfree(c->d_sel); dfree(c->d_sel_mp); dfree(c->d_frames);
+    dfree(c->d_ov); dfree(c->d_route); dfree(c->d_route_sel);
+    c->ov_kf.clear(); c->n_fit = 0; c->fit_sel = nullptr; c->n_fit_sel = 0;
     c->sel_cap = 0;
     c->sel_mask.clear();
     c->has_pack = false;
@@ -143,7 +155,7 @@ void free_pack(stl_ctx *c) {
 void free_work(stl_ctx *c) {
     DevWork &w = c->wk;
     dfree(w.cand); dfree(w.corr_kp); dfree(w.corr_pt); dfree(w.corr_sp); dfree(w.q_corr); dfree(w.q_kpsp); dfree(w.n_corr); dfree(w.n_q);
-    dfree(w.k1_ticket); dfree(w.k1_rec); dfree(w.k1_match); dfree(w.k1_surv); dfree(w.k1_cnt); dfree(w.k1_best_d2); dfree(w.k1_best_key);
+    dfree(w.k1_ticket); dfree(w.k1_rec); dfree(w.k1_match); dfree(w.k1_ov_match); dfree(w.k1_surv); dfree(w.k1_cnt); dfree(w.k1_best_d2); dfree(w.k1_best_key);
     dfree(w.frame); dfree(w.align); dfree(w.nn_pos); dfree(w.nn_g2); dfree(w.nb); dfree(w.nbx); dfree(w.nb_m); dfree(w.nb_last); dfree(w.dbg_nn); dfree(w.dbg_m); dfree(w.dbg_plane); dfree(w.dbg_dist); dfree(w.dbg_knn); dfree(w.dbg_stats);
     dfree(w.overflow); dfree(w.k1_clk);
     w = DevWork();
@@ -228,7 +240,8 @@ stl_status_t ensure_work(stl_ctx *ctx, int B, bool debug) {
     if (ctx->wk_cap == 0) {
         size_t free_b = 0, total_b = 0;
         CK(cudaMemGetInfo(&free_b, &total_b));
-        const size_t per_cand = (size_t)pk.n_kp_total * 24 + (size_t)pk.n_mp_total * (20 * kMaxK + 16) + (size_t)pk.n_kf * (sizeof(FrameRec) + 4 * sizeof(AlignRec) + 24 + (ctx->k1_mono ? 0 : sizeof(ulonglong2) * kK1MatchCap + 4 * kK1SurvCap)) + (size_t)pk.n_kp_total * 16 + sizeof(DevCand);
+        // (the three-kernel K1's survivors and matches: only those of the oversize keyframes)
+        const size_t per_cand = (size_t)pk.n_kp_total * 24 + (size_t)pk.n_mp_total * (20 * kMaxK + 16) + (size_t)pk.n_kf * (sizeof(FrameRec) + 4 * sizeof(AlignRec) + 24) + (size_t)pk.n_ov_match * sizeof(ulonglong2) + (size_t)pk.n_ov_surv * 4 + (size_t)pk.n_kp_total * 16 + sizeof(DevCand);
         size_t budget = std::min<size_t>((size_t)12 << 30, free_b / 4);
         int cap = (int)std::max<size_t>(1, std::min<size_t>(budget / std::max<size_t>(per_cand, 1), 256));
         if (const char *e = getenv("STL_MAX_CHUNK")) cap = std::max(1, std::min(cap, atoi(e)));  // tests: force the multi-chunk path
@@ -248,15 +261,18 @@ stl_status_t ensure_work(stl_ctx *ctx, int B, bool debug) {
             A_(w.cand, sizeof(DevCand) * cap);
             A_(w.corr_kp, 4 * nk); A_(w.corr_pt, 4 * nk); A_(w.corr_sp, 4 * nk); A_(w.q_corr, 4 * nk); A_(w.q_kpsp, 8 * nk);
             A_(w.n_corr, 4 * nf); A_(w.n_q, 4 * nf);
-            if (ctx->k1_mono) {  // persistent K1: scratch per resident CTA, not per unit
+            if (ctx->n_fit > 0) {  // persistent K1: scratch per resident CTA, not per unit
                 w.k1_slots = 2 * std::max(ctx->n_sm, 1);
                 A_(w.k1_match, sizeof(ulonglong2) * kK1MatchCap * (size_t)w.k1_slots);
                 A_(w.k1_rec, sizeof(float4) * kK1SurvCap * (size_t)w.k1_slots);
                 A_(w.k1_ticket, 8);
                 e = cudaMemsetAsync(w.k1_ticket, 0, 8, ctx->last_stream); if (e != cudaSuccess) return e;
-            } else {
-                A_(w.k1_match, sizeof(ulonglong2) * kK1MatchCap * nf);
-                A_(w.k1_surv, 4 * (size_t)kK1SurvCap * nf); A_(w.k1_cnt, 16 * nf); A_(w.k1_best_d2, 8 * nk); A_(w.k1_best_key, 8 * nk);
+            }
+            if (pk.n_ov > 0) {  // three-kernel K1: per (candidate, oversize keyframe)
+                const size_t c = (size_t)cap;
+                A_(w.k1_ov_match, sizeof(ulonglong2) * (size_t)pk.n_ov_match * c); A_(w.k1_surv, 4 * (size_t)pk.n_ov_surv * c);
+                A_(w.k1_cnt, 16 * (size_t)pk.n_ov * c);
+                A_(w.k1_best_d2, 8 * (size_t)std::max<long long>(pk.n_ov_kp, 1) * c); A_(w.k1_best_key, 8 * (size_t)std::max<long long>(pk.n_ov_kp, 1) * c);
             }
             A_(w.frame, sizeof(FrameRec) * nf); A_(w.align, sizeof(AlignRec) * nf * w.sub);
             A_(w.nn_pos, 4 * nm); A_(w.nn_g2, 4 * nm); A_(w.nb, 4 * nm * kMaxK); A_(w.nbx, sizeof(float4) * nm * kMaxK); A_(w.nb_m, 4 * nm); A_(w.nb_last, 8 * nm);
@@ -307,6 +323,23 @@ stl_status_t ensure_work(stl_ctx *ctx, int B, bool debug) {
     return STL_OK;
 }
 
+// K1 kernels one pass launches (work counter [5]): the one-kernel K1 when the pack has a fitting keyframe, the three of the
+// banded K1 when it has an oversize one
+int k1_launches(const stl_ctx *c) { return (c->n_fit > 0 ? 1 : 0) + (c->pk.n_ov > 0 ? 3 : 0); }
+
+// K1 over the selected keyframes of nb candidates: the one-kernel K1 over the fitting ones (the pack's own selection when no
+// keyframe is oversize), the banded three-kernel K1 over the oversize ones; both write the same per-keyframe records
+stl_status_t launch_k1(stl_ctx *ctx, int nb, cudaStream_t st, int with_terms) {
+    if (ctx->n_fit > 0) {
+        DevPack fit = ctx->pk;
+        if (fit.n_ov > 0) { fit.sel = ctx->fit_sel; fit.n_sel = ctx->n_fit_sel; }
+        CK(launch_assoc2d(fit, ctx->wk, ctx->dpr, nb, ctx->k1_smem, ctx->max_kp, ctx->max_tab, ctx->max_groups, st, with_terms));
+    }
+    if (ctx->pk.n_ov > 0)
+        CK(launch_assoc2d_split(ctx->pk, ctx->wk, ctx->dpr, nb, ctx->k1_split_smem, ctx->ov_max_bands, ctx->ov_max_surv, st, with_terms));
+    return STL_OK;
+}
+
 // scan points and keypoints an evaluation of B candidates walks (those of the selected keyframes)
 void set_eval_counters(stl_ctx *ctx, int B) {
     ctx->counters[0] = (double)ctx->sel_pts * B;
@@ -335,10 +368,8 @@ stl_status_t enqueue_eval(stl_ctx *ctx, const double *x, int B, double *d_out, c
     for (int c0 = 0; c0 < B; c0 += Bc) {
         const int nb = std::min(Bc, B - c0);
         CK(cudaMemcpyAsync(ctx->wk.cand, ctx->h_cand + c0, sizeof(DevCand) * nb, cudaMemcpyHostToDevice, st));
-        { StageTimer t(ctx, STL_STAGE_ASSOC2D, st);
-          if (ctx->k1_mono) CK(launch_assoc2d(ctx->pk, ctx->wk, ctx->dpr, nb, ctx->k1_smem, ctx->max_kp, ctx->max_tab, ctx->max_groups, st));
-          else CK(launch_assoc2d_split(ctx->pk, ctx->wk, ctx->dpr, nb, ctx->k1_split_smem, 0, st)); }
-        ctx->launches += ctx->k1_mono ? 0 : 2;
+        { StageTimer t(ctx, STL_STAGE_ASSOC2D, st); s = launch_k1(ctx, nb, st, 1); if (s != STL_OK) return s; }
+        ctx->launches += k1_launches(ctx) - 1;
         if (marks) CK(cudaEventRecord(ctx->ev_k1, st));
         { StageTimer t(ctx, STL_STAGE_KNN3D, st); CK(launch_align3d(ctx->pk, ctx->wk, ctx->dpr, nb, debug ? 1 : 0, st, marks ? ctx->ev_k2a : nullptr,
                                                                             marks ? ctx->lm.nnb_pos : nullptr, marks ? ctx->lm.nbb_m : nullptr)); }
@@ -426,10 +457,8 @@ stl_status_t enqueue_associate(stl_ctx *ctx, const double *x0, int P, const uint
             CK(cudaMemcpyAsync(ctx->wk.cand, hc, sizeof(DevCand) * nb, cudaMemcpyHostToDevice, st));
             CK(cudaEventRecord(ctx->h2d_done, st));
             // 2-D association at x0 (FindProjectCorrespondences, iba_local.cpp:191): K1 without the cost terms
-            { StageTimer t(ctx, STL_STAGE_ASSOC2D, st);
-              if (ctx->k1_mono) CK(launch_assoc2d(pk, ctx->wk, ctx->dpr, nb, ctx->k1_smem, ctx->max_kp, ctx->max_tab, ctx->max_groups, st, 0));
-              else CK(launch_assoc2d_split(pk, ctx->wk, ctx->dpr, nb, ctx->k1_split_smem, 0, st, 0)); }
-            ctx->launches += ctx->k1_mono ? 1 : 3;
+            { StageTimer t(ctx, STL_STAGE_ASSOC2D, st); s = launch_k1(ctx, nb, st, 0); if (s != STL_OK) return s; }
+            ctx->launches += k1_launches(ctx);
             ctx->wk_has_nn = false;
         }
         e = lm_set_lanes(lm, lanes.data(), nb, st);
@@ -480,6 +509,8 @@ stl_status_t need_single(stl_ctx *ctx, const char *call, const char *multi) {
 void select_all(stl_ctx *c) {
     c->pk.sel = nullptr; c->pk.sel_mp = nullptr;
     c->pk.n_sel = c->pk.n_kf; c->pk.n_sel_mp = c->pk.n_mp_total;
+    c->fit_sel = c->d_route; c->n_fit_sel = c->n_fit;
+    c->pk.ov_sel = c->d_route ? c->d_route + c->pk.n_kf : nullptr; c->pk.n_ov_sel = c->pk.n_ov;
     c->sel_mask.assign((size_t)c->pk.n_kf, 1);
     c->sel_pts = c->n_pts_total; c->sel_kp = c->pk.n_kp_total;
 }
@@ -611,7 +642,7 @@ stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *p) {
     std::vector<DevKf> &hk = hk_new;
     hk.assign(F, DevKf());
     long long pt = 0, nodes = 0, bmw = 0, gcells = 0, mp_total = 0, tab_total = 0;
-    int max_kp = 0, max_bm = 0, max_tab = 0;
+    int max_kp = 0, max_tab = 0;
     for (int f = 0; f < F; ++f) {
         DevKf &K = hk[f];
         const long long n = p->scan_offset[f + 1] - p->scan_offset[f];
@@ -651,21 +682,67 @@ stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *p) {
         mp_total += K.n_mp;
         K.pmax = 1.f;
         max_kp = std::max(max_kp, K.n_kp);
-        max_bm = std::max(max_bm, K.bm_wpr * K.bm_rows);
     }
     const long long NK = p->kp_offset[F];
     int max_cells = 0, max_groups = 0;
     for (int f = 0; f < F; ++f) { max_cells = std::max(max_cells, hk[f].gw * hk[f].gh); max_groups = std::max(max_groups, hk[f].n_pad / 128); }
     if (max_kp > 65535) return fail(ctx, STL_ERR_CAPACITY, "more than 65535 keypoints in a keyframe");
-    const size_t k1_smem_new = assoc2d_smem_bytes(max_kp, max_tab, max_groups);
     int smem_optin = 0;
     CK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
-    if (k1_smem_new > (size_t)smem_optin)
-        return fail(ctx, STL_ERR_CAPACITY, "K1 needs %zu B of shared memory (%d keypoints); device limit %d", k1_smem_new, max_kp, smem_optin);
-    CK(assoc2d_configure(k1_smem_new));
-    const size_t k1_split_new = assoc2d_split_smem_bytes(max_bm, max_groups);
-    if (k1_split_new > (size_t)smem_optin) return fail(ctx, STL_ERR_CAPACITY, "K1a needs %zu B of shared memory; device limit %d", k1_split_new, smem_optin);
-    CK(assoc2d_split_configure(k1_split_new));
+    // ---- K1 routing (stlcalib.h, stl_allow_oversize_keyframes): keyframes leave the one-kernel K1's set largest-first (by their
+    // own assoc2d_smem_bytes, ties: lower index first) until the set's maxima fit the opt-in limit; with no keyframe out this is
+    // the check of a pack without oversize keyframes
+    std::vector<int> order(F);
+    std::vector<size_t> own(F);
+    for (int f = 0; f < F; ++f) { order[f] = f; own[f] = assoc2d_smem_bytes(hk[f].n_kp, hk[f].tab_bytes, hk[f].n_pad / 128); }
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return own[a] > own[b]; });
+    std::vector<int> sfx_kp(F + 1, 0), sfx_tab(F + 1, 0), sfx_gr(F + 1, 0);  // maxima over order[r..F)
+    for (int r = F - 1; r >= 0; --r) {
+        const DevKf &K = hk[order[r]];
+        sfx_kp[r] = std::max(sfx_kp[r + 1], K.n_kp); sfx_tab[r] = std::max(sfx_tab[r + 1], K.tab_bytes); sfx_gr[r] = std::max(sfx_gr[r + 1], K.n_pad / 128);
+    }
+    int n_out = 0;
+    while (n_out < F && assoc2d_smem_bytes(sfx_kp[n_out], sfx_tab[n_out], sfx_gr[n_out]) > (size_t)smem_optin) ++n_out;
+    if (n_out > 0 && !ctx->allow_oversize)
+        return fail(ctx, STL_ERR_CAPACITY, "K1 needs %zu B of shared memory (%d keypoints); device limit %d", assoc2d_smem_bytes(max_kp, max_tab, max_groups),
+                    max_kp, smem_optin);
+    const char *route_env = getenv("STL_K1_OVERSIZE");
+    if ((route_env && strcmp(route_env, "all") == 0) || getenv("STL_K1_SPLIT")) n_out = F;  // diagnostic: every keyframe on the banded K1
+    const int n_fit_new = F - n_out;
+    size_t k1_smem_new = 0;
+    if (n_fit_new > 0) {
+        k1_smem_new = assoc2d_smem_bytes(sfx_kp[n_out], sfx_tab[n_out], sfx_gr[n_out]);
+        CK(assoc2d_configure(k1_smem_new));
+    }
+    // the oversize keyframes, increasing, and their workspace slices (OvKf)
+    std::vector<uint8_t> is_ov((size_t)F, 0);
+    for (int r = 0; r < n_out; ++r) is_ov[order[r]] = 1;
+    std::vector<int> ov_new;
+    std::vector<OvKf> hov;
+    long long ov_kp = 0, ov_surv = 0, ov_match = 0;
+    int ov_bands = 0, ov_surv_max = 0, ov_band_words = 0, ov_groups = 0;
+    for (int f = 0; f < F; ++f) {
+        if (!is_ov[f]) continue;
+        const DevKf &K = hk[f];
+        OvKf o;
+        o.f = f;
+        o.surv_cap = (int)std::max<long long>(kK1SurvCap, std::min<long long>(((2ll * K.n_kp + 255) / 256) * 256, K.n_pad));
+        o.match_cap = 2 * o.surv_cap;
+        const int rows = k1_band_rows(K.bm_wpr);
+        o.n_bands = (K.bm_rows + rows - 1) / rows;
+        o.kp_off = ov_kp; o.surv_off = ov_surv; o.match_off = ov_match;
+        ov_kp += K.n_kp; ov_surv += o.surv_cap; ov_match += o.match_cap;
+        ov_bands = std::max(ov_bands, o.n_bands); ov_surv_max = std::max(ov_surv_max, o.surv_cap);
+        ov_band_words = std::max(ov_band_words, std::min(rows, K.bm_rows) * K.bm_wpr); ov_groups = std::max(ov_groups, K.n_pad / 128);
+        ov_new.push_back(f);
+        hov.push_back(o);
+    }
+    size_t k1_split_new = 0;
+    if (n_out > 0) {
+        k1_split_new = assoc2d_split_smem_bytes(ov_band_words, ov_groups);
+        if (k1_split_new > (size_t)smem_optin) return fail(ctx, STL_ERR_CAPACITY, "K1a needs %zu B of shared memory; device limit %d", k1_split_new, smem_optin);
+        CK(assoc2d_split_configure(k1_split_new));
+    }
 
     // ---- from here on the previous state is gone
     free_work(ctx);
@@ -673,10 +750,12 @@ stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *p) {
     lm_free(ctx->lm);
     ctx->h_kf.swap(hk_new);
     std::vector<DevKf> &hk2 = ctx->h_kf;
-    ctx->max_kp = max_kp; ctx->max_bm_words = max_bm; ctx->max_tab = max_tab; ctx->max_groups = max_groups;
+    ctx->max_kp = sfx_kp[n_out]; ctx->max_tab = sfx_tab[n_out]; ctx->max_groups = sfx_gr[n_out];
     CK(cudaDeviceGetAttribute(&ctx->n_sm, cudaDevAttrMultiProcessorCount, ctx->device));
     ctx->k1_smem = k1_smem_new; ctx->k1_split_smem = k1_split_new;
-    ctx->k1_mono = getenv("STL_K1_SPLIT") == nullptr;
+    ctx->n_fit = n_fit_new;
+    ctx->ov_kf.swap(ov_new);
+    ctx->ov_max_bands = ov_bands; ctx->ov_max_surv = ov_surv_max;
     cudaStream_t st = acquire_stream(ctx, nullptr);
     struct Scope {  // events and the raw-scan scratch are released on every exit path
         cudaEvent_t ev0 = nullptr, ev1 = nullptr; float *d_raw = nullptr; BuildScratch scr;
@@ -804,6 +883,19 @@ stl_status_t stl_upload_pack(stl_ctx_t *ctx, const stl_pack_t *p) {
     }
     CK(cudaMemcpyAsync(pk.he_Tc, p->he_Tc, 48 * (size_t)F, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(pk.he_Tl, p->he_Tl, 96 * (size_t)F, cudaMemcpyHostToDevice, st));
+    if (!hov.empty()) {  // the oversize descriptors and the routing lists of the whole pack
+        const int n_ov = (int)hov.size();
+        pk.n_ov = n_ov; pk.n_ov_kp = ov_kp; pk.n_ov_surv = ov_surv; pk.n_ov_match = ov_match;
+        CK(cudaMalloc(&ctx->d_ov, sizeof(OvKf) * (size_t)n_ov));
+        CK(cudaMemcpyAsync(ctx->d_ov, hov.data(), sizeof(OvKf) * (size_t)n_ov, cudaMemcpyHostToDevice, st));
+        pk.ov = ctx->d_ov;
+        std::vector<int> route((size_t)2 * F, 0);
+        for (int f = 0, i = 0; f < F; ++f) if (!is_ov[f]) route[i++] = f;
+        for (int o = 0; o < n_ov; ++o) route[(size_t)F + o] = o;
+        CK(cudaMalloc(&ctx->d_route, sizeof(int) * 2 * (size_t)F));
+        CK(cudaMalloc(&ctx->d_route_sel, sizeof(int) * 2 * (size_t)F));
+        CK(cudaMemcpyAsync(ctx->d_route, route.data(), sizeof(int) * 2 * (size_t)F, cudaMemcpyHostToDevice, st));
+    }
     CK(cudaStreamSynchronize(st));
 
     // ---- scans: chunked upload + index build
@@ -1052,12 +1144,46 @@ stl_status_t stl_select_keyframes(stl_ctx_t *ctx, const int32_t *kf, int32_t n) 
     }
     if (e == cudaSuccess && n > 0) e = cudaMemcpyAsync(ctx->d_sel, kf, sizeof(int) * (size_t)n, cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_sel_mp, mp.data(), sizeof(int2) * ((size_t)n + 1), cudaMemcpyHostToDevice, st);
+    // with oversize keyframes: the selected fitting keyframes and the ordinals of the selected oversize ones, as for the pack
+    int n_fit_sel = 0, n_ov_sel = 0;
+    if (ctx->pk.n_ov > 0) {
+        std::vector<int> route((size_t)2 * F, 0);
+        for (int i = 0; i < n; ++i) {
+            const auto it = std::lower_bound(ctx->ov_kf.begin(), ctx->ov_kf.end(), kf[i]);
+            if (it != ctx->ov_kf.end() && *it == kf[i]) route[(size_t)F + n_ov_sel++] = (int)(it - ctx->ov_kf.begin());
+            else route[n_fit_sel++] = kf[i];
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(ctx->d_route_sel, route.data(), sizeof(int) * 2 * (size_t)F, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // route is host memory of this scope
+    }
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return fail(ctx, STL_ERR_CUDA, "stl_select_keyframes: %s (every keyframe stays selected)", cudaGetErrorString(e));
     ctx->pk.sel = ctx->d_sel; ctx->pk.sel_mp = ctx->d_sel_mp;
     ctx->pk.n_sel = n; ctx->pk.n_sel_mp = slots;
+    if (ctx->pk.n_ov > 0) {
+        ctx->fit_sel = ctx->d_route_sel; ctx->n_fit_sel = n_fit_sel;
+        ctx->pk.ov_sel = ctx->d_route_sel + F; ctx->pk.n_ov_sel = n_ov_sel;
+    }
     ctx->sel_mask.swap(mask);
     ctx->sel_pts = pts; ctx->sel_kp = kps;
+    return STL_OK;
+}
+
+stl_status_t stl_allow_oversize_keyframes(stl_ctx_t *ctx, int32_t allow) {
+    if (!ctx) return STL_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (allow != 0 && allow != 1) return fail(ctx, STL_ERR_INVALID, "stl_allow_oversize_keyframes: allow = %d is neither 0 nor 1", allow);
+    ctx->allow_oversize = allow != 0;
+    return STL_OK;
+}
+
+stl_status_t stl_oversize_keyframes(stl_ctx_t *ctx, int32_t *kf, int32_t cap, int32_t *n) {
+    if (!ctx || !n || cap < 0) return STL_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!ctx->has_pack) return fail(ctx, STL_ERR_STATE, "stl_upload_pack has not been called");
+    *n = (int32_t)ctx->ov_kf.size();
+    const int m = std::min(*n, cap);
+    if (kf) for (int i = 0; i < m; ++i) kf[i] = ctx->ov_kf[(size_t)i];
     return STL_OK;
 }
 

@@ -9,6 +9,20 @@
 
 namespace stl {
 
+// A keyframe on the banded three-kernel K1 (assoc2d_split.cu): an oversize keyframe (stl_allow_oversize_keyframes), or any
+// keyframe under STL_K1_OVERSIZE=all.  Its slices of the three-kernel K1's workspace, which is indexed by oversize ordinal
+// o (position in DevPack::ov) and laid out per candidate b as [b][n_ov] counters, [b][n_ov_kp] per-keypoint tables,
+// [b][n_ov_surv] survivors and [b][n_ov_match] matches.
+struct OvKf {
+    int f;               // pack keyframe
+    int surv_cap;        // survivor slots of one (candidate, keyframe) unit: max(kK1SurvCap, min(2 n_kp rounded up to 256, n_pad))
+    int match_cap;       // match slots of one unit: 2 * surv_cap
+    int n_bands;         // k_stream bands: ceil(bm_rows / k1_band_rows(bm_wpr))
+    long long kp_off;    // first slot of its keypoints in [n_ov_kp]
+    long long surv_off;  // first slot of its survivors in [n_ov_surv]
+    long long match_off; // first slot of its matches in [n_ov_match]
+};
+
 // Device-resident pack (all pointers are device memory owned by the context).
 struct DevPack {
     int n_kf = 0, n_covis = 0;
@@ -41,6 +55,12 @@ struct DevPack {
     const int *sel = nullptr;        // [n_sel] selected keyframes, strictly increasing
     const int2 *sel_mp = nullptr;    // [n_sel + 1] (first compacted map-point slot of position i, mp_off - that): k_linearize's 3-D walk
     long long n_sel_mp = 0;          // map-point slots of the selected keyframes
+    // three-kernel K1: the keyframes it serves (OvKf) and, for a launch, the ordinals of the selected ones, increasing
+    int n_ov = 0;
+    const OvKf *ov = nullptr;        // [n_ov]
+    long long n_ov_kp = 0, n_ov_surv = 0, n_ov_match = 0;
+    int n_ov_sel = 0;
+    const int *ov_sel = nullptr;     // [n_ov_sel]
 };
 
 #ifdef __CUDACC__
@@ -81,12 +101,13 @@ struct DevWork {
     int k1_slots = 0;
     int *k1_ticket = nullptr;        // [2] next chunk of units, CTAs that have left (the last one re-arms both)
     float4 *k1_rec = nullptr;        // [k1_slots][kK1SurvCap] (x, y, z, sorted position) of the points that passed the pre-cull
-    ulonglong2 *k1_match = nullptr;  // [k1_slots][8192] (one-kernel K1) or [Bc][n_kf][8192] (three-kernel K1): matches of the exact pass
-    // three-kernel K1 (assoc2d_split.cu)
-    uint32_t *k1_surv = nullptr;              // [Bc][n_kf][kK1SurvCap] sorted positions that passed the pre-cull
-    int *k1_cnt = nullptr;                    // [Bc][n_kf][4] survivors, matches, overflow flag, pad
-    unsigned long long *k1_best_d2 = nullptr; // [Bc][n_kp_total] bits of the smallest squared pixel distance per keypoint
-    unsigned long long *k1_best_key = nullptr;// [Bc][n_kp_total] (original index << 32 | position) of the point that owns it
+    ulonglong2 *k1_match = nullptr;  // [k1_slots][8192] matches of the exact pass
+    // three-kernel K1 (assoc2d_split.cu), indexed by oversize ordinal (OvKf)
+    ulonglong2 *k1_ov_match = nullptr;        // [Bc][n_ov_match] matches of the exact pass
+    uint32_t *k1_surv = nullptr;              // [Bc][n_ov_surv] sorted positions that passed the pre-cull
+    int *k1_cnt = nullptr;                    // [Bc][n_ov][4] survivors, matches, overflow flag, pad
+    unsigned long long *k1_best_d2 = nullptr; // [Bc][n_ov_kp] bits of the smallest squared pixel distance per keypoint
+    unsigned long long *k1_best_key = nullptr;// [Bc][n_ov_kp] (original index << 32 | position) of the point that owns it
     long long *k1_clk = nullptr;  // optional [units][8] phase clocks of K1 (diagnostic, STL_K1_CLK=1)
     int *overflow = nullptr;      // K1 survivor-list overflow counter (diagnostic)
 };
@@ -122,18 +143,26 @@ cudaError_t build_plane_index(const DevPack &pk, const DevKf *h_kf, int kf_begin
 
 constexpr int kK1SurvCap = 4096;   // survivors of the float32 pre-cull a (candidate, keyframe) unit may list
 constexpr int kK1MatchCap = 8192;  // (keypoint, point) matches a unit may record between the exact pass and the tie pass
+// Bands of the three-kernel K1's stream (DESIGN §3 "Oversize keyframes"): band j of a keyframe holds bitmap rows
+// [j R, min((j + 1) R, bm_rows)) with R = k1_band_rows(bm_wpr), so that a band's words stay within kK1BandWords (16 KB)
+// whatever the image size
+constexpr int kK1BandWords = 4096;
+__host__ __device__ inline int k1_band_rows(int bm_wpr) { return bm_wpr >= kK1BandWords ? 1 : kK1BandWords / bm_wpr; }
 
-// ---- K1 (assoc2d.cu: one persistent kernel, the default; assoc2d_split.cu: stream / exact / correspondence kernels, STL_K1_SPLIT=1) ----
+// ---- K1 (assoc2d.cu: one persistent kernel over the keyframes whose tables fit its shared memory; assoc2d_split.cu: banded
+// stream / exact / correspondence kernels over the oversize keyframes DevPack::ov_sel) ----
 size_t assoc2d_smem_bytes(int max_kp, int max_tab_bytes, int max_groups);
 cudaError_t assoc2d_configure(size_t smem);
 // with_terms = 0: correspondences only (the association pass of the LM path needs neither the covisible
 // re-projection term nor the hand-eye term)
 cudaError_t launch_assoc2d(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, size_t smem, int max_kp, int max_tab_bytes,
                            int max_groups, cudaStream_t st, int with_terms = 1);
-size_t assoc2d_split_smem_bytes(int max_bm_words, int max_groups);
+// max_band_words: the largest band (rows * bm_wpr) of the served keyframes, at most kK1BandWords
+size_t assoc2d_split_smem_bytes(int max_band_words, int max_groups);
 cudaError_t assoc2d_split_configure(size_t smem);
-cudaError_t launch_assoc2d_split(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, size_t smem, int max_pts, cudaStream_t st,
-                                 int with_terms = 1);
+// max_bands / max_surv_cap: maxima of OvKf::n_bands / surv_cap over DevPack::ov
+cudaError_t launch_assoc2d_split(const DevPack &pk, const DevWork &wk, const DevParams &pr, int B, size_t smem, int max_bands, int max_surv_cap,
+                                 cudaStream_t st, int with_terms = 1);
 
 // ---- K2 (knn3d.cu) ---------------------------------------------------------------
 // K2a (traversal: 1-NN + k-NN, warp per query) then K2b (plane fit + distance, thread per query)
