@@ -12,7 +12,7 @@
 //        IBA_PlaneFactor::operator()     include/IBACalib2.hpp:152-184 (g2o twin IBACalib.hpp:103-140)
 //        Point2Point_Factor              include/IBACalib2.hpp:570-584
 //        Point2Plane_Factor              include/IBACalib2.hpp:611-625
-//      with forward-mode duals (dual.cuh), ceres::HuberLoss + Corrector semantics
+//      with the Jet evaluation's values and chain-rule partials (linrow.cuh), ceres::HuberLoss + Corrector semantics
 //      (iba_local.cpp:263,291; rho'' <= 0 => residual and Jacobian scaled by sqrt(rho')),
 //      and reduces cost, J^T r and the 7x7 J^T J in fp64 (warp shuffles, fixed order).
 #include <cub/cub.cuh>
@@ -21,6 +21,7 @@
 #include "dual.cuh"
 #include "gprfit.hpp"
 #include "knn.cuh"
+#include "linrow.cuh"
 #include "lm.h"
 
 namespace stl {
@@ -348,30 +349,6 @@ struct Acc {
     double v[kLinVals];
 };
 
-// D7 with the PARTIALS formed by fused multiply-adds (the values keep the reference's separate multiply and add, so costs
-// and the robust-kernel branch are bit-identical to the plain-D7 evaluation; a partial differs from the Jet's by one
-// rounding, 1e-16 relative, on these well-conditioned blocks).  Same layout as D7: the candidate's Sim3Exp duals are read
-// as F7.  Used by k_linearize only — the GPR blocks (cond ~1e12) stay on D7, operation for operation.
-struct F7 {
-    double a;
-    double v[7];
-};
-static_assert(sizeof(F7) == sizeof(D7), "F7 views D7 storage");
-__device__ __forceinline__ F7 f7_const(double x) { F7 r; r.a = x; for (int i = 0; i < 7; ++i) r.v[i] = 0.0; return r; }
-__device__ __forceinline__ F7 operator+(const F7 &f, const F7 &g) { F7 r; r.a = f.a + g.a; for (int i = 0; i < 7; ++i) r.v[i] = f.v[i] + g.v[i]; return r; }
-__device__ __forceinline__ F7 operator-(const F7 &f, const F7 &g) { F7 r; r.a = f.a - g.a; for (int i = 0; i < 7; ++i) r.v[i] = f.v[i] - g.v[i]; return r; }
-__device__ __forceinline__ F7 operator*(const F7 &f, const F7 &g) { F7 r; r.a = f.a * g.a; for (int i = 0; i < 7; ++i) r.v[i] = fma(f.a, g.v[i], f.v[i] * g.a); return r; }
-__device__ __forceinline__ F7 operator/(const F7 &f, const F7 &g) {
-    F7 r;
-    const double gi = 1.0 / g.a, q = f.a * gi;
-    r.a = q;
-    for (int i = 0; i < 7; ++i) r.v[i] = fma(-q, g.v[i], f.v[i]) * gi;
-    return r;
-}
-__device__ __forceinline__ F7 operator*(const F7 &f, double c) { F7 r; r.a = f.a * c; for (int i = 0; i < 7; ++i) r.v[i] = f.v[i] * c; return r; }
-__device__ __forceinline__ F7 operator+(const F7 &f, double c) { F7 r = f; r.a = f.a + c; return r; }
-__device__ __forceinline__ F7 operator-(const F7 &f, double c) { F7 r = f; r.a = f.a - c; return r; }
-
 __device__ __forceinline__ void huber(double sq, double delta, double &rho0, double &sr) {
     if (sq > delta * delta) {  // ceres::HuberLoss::Evaluate
         const double r = sqrt(sq);
@@ -401,11 +378,8 @@ __device__ __forceinline__ void mv3(const D7 *M, const D7 *p, D7 *o) {
 #pragma unroll
     for (int i = 0; i < 3; ++i) o[i] = (M[i * 3] * p[0] + M[i * 3 + 1] * p[1]) + M[i * 3 + 2] * p[2];
 }
-__device__ __forceinline__ void mv3(const F7 *M, const F7 *p, F7 *o) {
-#pragma unroll
-    for (int i = 0; i < 3; ++i) o[i] = (M[i * 3] * p[0] + M[i * 3 + 1] * p[1]) + M[i * 3 + 2] * p[2];
-}
-__device__ __forceinline__ void accumulate(Acc &A, const F7 &e, double sr) {
+// k_linearize's rows (linrow.cuh): J^T r and J^T J by fused multiply-adds
+__device__ __forceinline__ void accumulate(Acc &A, const Row7 &e, double sr) {
     const double r = sr * e.a;
     double J[7];
 #pragma unroll
@@ -443,6 +417,16 @@ __device__ __forceinline__ void lm_list_start(const LmState &lm, int p, int whic
     if (threadIdx.x == 0) *out = s;
 }
 
+// x, re-read: the address carries an offset of zero the compiler cannot see through, so loads from x inside a loop are not
+// hoisted out of it.  k_linearize reads its candidate tables (~190 doubles, shared memory) through this once per block: kept in
+// registers across the block loops they spill.
+template <class T>
+__device__ __forceinline__ const T &reread(const T &x) {
+    int z;
+    asm volatile("mov.b32 %0, 0;" : "=r"(z));
+    return *reinterpret_cast<const T *>(reinterpret_cast<const char *>(&x) + z);
+}
+
 // Problem-local slot of slot v of the selection's compacted slot range (DevPack::sel_mp): with a keyframe selection the 3-D walk
 // runs over the selected keyframes' slots only, grouped 32 at a time as a pack of those keyframes groups them, so that every
 // thread sums the blocks it would sum there
@@ -458,23 +442,23 @@ __device__ __forceinline__ int sel_slot(const DevPack &pk, int v) {
 // grid (chunks, B): candidate blockIdx.y on problem cprob[blockIdx.y].  The 3-D/3-D blocks are walked over ALL query slots of
 // that problem (no compacted list: the work per block is light, and the association then has no select on the way to the
 // linearisation).  WB (stl_eval_blocks) numbers the blocks and therefore walks the compacted list (problem 0).
-template <bool WB>
-__global__ void __launch_bounds__(kLinThreads)
+// MINB: resident CTAs per SM the registers must allow (lm_linearize); the two forms compute the same bits.
+template <bool WB, int MINB>
+__global__ void __launch_bounds__(kLinThreads, MINB)
 k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, const int *__restrict__ cprob,
             double *__restrict__ partial, int partial_stride, const BlockOut bo) {
     __shared__ LmCand c;
+    __shared__ double W[9][7];  // candidate table of the 3-D/3-D partials (linrow.cuh)
     __shared__ int list0;
     const int prob = cprob ? cprob[blockIdx.y] : 0;
     {
         const double *src = reinterpret_cast<const double *>(cands + blockIdx.y);
         double *dst = reinterpret_cast<double *>(&c);
         for (int i = threadIdx.x; i < (int)(sizeof(LmCand) / 8); i += kLinThreads) dst[i] = src[i];
+        lin_table(cands[blockIdx.y], W, threadIdx.x, kLinThreads);
     }
     lm_list_start(lm, prob, 0, &list0);
     __syncthreads();
-    const F7 *cR = reinterpret_cast<const F7 *>(c.R), *ct = reinterpret_cast<const F7 *>(c.t);
-    const F7 *cRlc = reinterpret_cast<const F7 *>(c.Rlc), *ctlc = reinterpret_cast<const F7 *>(c.tlc);
-    const F7 &cs7 = *reinterpret_cast<const F7 *>(&c.s);
     Acc A;
 #pragma unroll
     for (int i = 0; i < kLinVals; ++i) A.v[i] = 0.0;
@@ -488,23 +472,18 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
     // ---- 3-D/2-D blocks: IBA_PlaneFactor (IBACalib2.hpp:152-184)
     for (int it = t0; it < n2d; it += stride) {
         const int slot = idx2d[it];  // global slot (problem offset included)
+        const LmCand &cb = reread(c);
         const int f = lm.slot_kf[slot];
         const uint32_t kp = lm.slot_kp[slot];
         const DevKf &K = pk.kf[f];
         const double fx = K.fx, fy = K.fy, cx = K.cx, cy = K.cy;
         const float2 kxy = pk.kp_xy[K.kp_off + kp];
-        const double *g = lm.geo2d + (long long)slot * 6;
-        const F7 p0[3] = {f7_const(g[0]), f7_const(g[1]), f7_const(g[2])}, n0[3] = {f7_const(g[3]), f7_const(g[4]), f7_const(g[5])};
-        F7 p0c[3], n0c[3];
-        mv3(cR, p0, p0c);
+        double g[6];
 #pragma unroll
-        for (int i = 0; i < 3; ++i) p0c[i] = p0c[i] + ct[i];
-        mv3(cR, n0, n0c);
+        for (int i = 0; i < 6; ++i) g[i] = lm.geo2d[(long long)slot * 6 + i];
         const double Cxz = ((double)kxy.x - cx) / fx, Cyz = ((double)kxy.y - cy) / fy;
-        const F7 num = (n0c[0] * p0c[0] + n0c[1] * p0c[1]) + n0c[2] * p0c[2];
-        const F7 den = (n0c[0] * Cxz + n0c[1] * Cyz) + n0c[2];
-        const F7 Z0 = num / den;
-        const F7 P0[3] = {Z0 * Cxz, Z0 * Cyz, Z0};
+        double Z0, dZ[7];
+        p2_depth(cb, g, Cxz, Cyz, Z0, dZ);
         // pass 1: squared norm of the block (values only) for the robust kernel
         double sq = 0.0;
         int nres = 0;
@@ -514,9 +493,7 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             if (isnan(uv.x)) continue;
             const float *rp = pk.relpose + ((long long)f * C + s) * 12;
             double P1[3];
-#pragma unroll
-            for (int i = 0; i < 3; ++i)
-                P1[i] = (((double)rp[i * 4] * P0[0].a + (double)rp[i * 4 + 1] * P0[1].a) + (double)rp[i * 4 + 2] * P0[2].a) + (double)rp[i * 4 + 3] * c.s.a;
+            p2_point(cb, rp, Z0, Cxz, Cyz, P1);
             const double eu = (fx * P1[0] / P1[2] + cx) - (double)uv.x, ev = (fy * P1[1] / P1[2] + cy) - (double)uv.y;
             sq += eu * eu;
             sq += ev * ev;
@@ -527,19 +504,17 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
         A.v[0] += 0.5 * rho0;
         A.v[36] += 1.0;
         A.v[39] += (double)nres;
-        // pass 2: duals
+        // pass 2: the rows with their partials
         int wrow = 0;
         for (int s = 0; s < C; ++s) {
             if (!pk.covis_valid[f * C + s]) continue;
             const float2 uv = pk.covis_uv[(K.kp_off + kp) * C + s];
             if (isnan(uv.x)) continue;
             const float *rp = pk.relpose + ((long long)f * C + s) * 12;
-            F7 P1[3];
-#pragma unroll
-            for (int i = 0; i < 3; ++i)
-                P1[i] = ((P0[0] * (double)rp[i * 4] + P0[1] * (double)rp[i * 4 + 1]) + P0[2] * (double)rp[i * 4 + 2]) + cs7 * (double)rp[i * 4 + 3];
-            const F7 eu = ((P1[0] * fx) / P1[2] + cx) - (double)uv.x;
-            const F7 ev = ((P1[1] * fy) / P1[2] + cy) - (double)uv.y;
+            double P1[3];
+            p2_point(cb, rp, Z0, Cxz, Cyz, P1);
+            Row7 eu, ev;
+            p2_rows(cb, rp, P1, dZ, Cxz, Cyz, fx, fy, cx, cy, uv.x, uv.y, eu, ev);
             accumulate(A, eu, sr);
             accumulate(A, ev, sr);
             if (WB) { put_row(bo, it, wrow, eu); put_row(bo, it, wrow + 1, ev); wrow += 2; }
@@ -589,29 +564,28 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             if (mine < 0) continue;
             slot = mine;
         }
-        const double *g = geo3d + slot * 9;
         const int type = type3d[slot];
-        const F7 Ms[3] = {cs7 * g[0], cs7 * g[1], cs7 * g[2]};  // MapPoint * s
-        F7 M[3];
-        mv3(cRlc, Ms, M);
+        const LmCand &cb = reread(c);
+        const double (*Wb)[7] = reread(W);
+        double g[9], d[3];
 #pragma unroll
-        for (int i = 0; i < 3; ++i) M[i] = M[i] + ctlc[i];
-        const F7 d[3] = {M[0] - g[3], M[1] - g[4], M[2] - g[5]};
+        for (int i = 0; i < 9; ++i) g[i] = geo3d[slot * 9 + i];
+        p3_values(cb, g, d);
         double rho0, sr;
         if (type == 1) {
-            huber((d[0].a * d[0].a + d[1].a * d[1].a) + d[2].a * d[2].a, pr.delta3d, rho0, sr);
-            accumulate(A, d[0], sr);
-            accumulate(A, d[1], sr);
-            accumulate(A, d[2], sr);
+            huber((d[0] * d[0] + d[1] * d[1]) + d[2] * d[2], pr.delta3d, rho0, sr);
+            const long long blk = (long long)n2d + it;
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                const Row7 e = p3_point_row(cb, Wb, g, d, i);
+                accumulate(A, e, sr);
+                if (WB) put_row(bo, blk, i, e);
+            }
             A.v[37] += 1.0;
             A.v[39] += 3.0;
-            if (WB) {
-                const long long blk = (long long)n2d + it;
-                put_row(bo, blk, 0, d[0]); put_row(bo, blk, 1, d[1]); put_row(bo, blk, 2, d[2]);
-                put_head(bo, blk, 1, lm.slot_kf[po + slot], lm.slot_kp[po + slot], 3);
-            }
+            if (WB) put_head(bo, blk, 1, lm.slot_kf[po + slot], lm.slot_kp[po + slot], 3);
         } else {
-            const F7 e = (d[0] * g[6] + d[1] * g[7]) + d[2] * g[8];
+            const Row7 e = p3_plane_row(cb, Wb, g, d);
             huber(e.a * e.a, pr.delta3d, rho0, sr);
             accumulate(A, e, sr);
             A.v[38] += 1.0;
@@ -1225,8 +1199,10 @@ cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, co
     // the exact counts from the device
     const long long work = pk.sel ? (pk.n_sel_mp > 0 ? pk.n_sel_mp : 1) : lm.max_blocks;  // a selection: what a pack of it would have
     long long chunks_ll = (work + kLinThreads * 2 - 1) / (kLinThreads * 2);
-    // at most ONE wave of CTAs per candidate (2 CTAs of 255 registers per SM): 296 chunks measured 0.134 ms against 0.140 (592),
-    // 0.163 (444: a wave and a half) and 0.157 (1184) at the KITTI-00 shape, and the finishing kernel sums four times fewer partials
+    // at most ONE wave of CTAs per candidate at 2 CTAs per SM: 296 chunks measured 0.134 ms against 0.140 (592), 0.163 (444: a
+    // wave and a half) and 0.157 (1184) at the KITTI-00 shape, and the finishing kernel sums four times fewer partials.  444 chunks at
+    // 3 CTAs per SM take 0.853 ms per step against 0.869 (296 at 2 CTAs per SM), but the chunk count sets the order of the fp64
+    // sums: changing it changes the cost's last bits
     static const int kChunkCap = getenv("STL_LIN_CHUNKS") ? atoi(getenv("STL_LIN_CHUNKS")) : 148 * 2;
     int chunks = (int)(chunks_ll < 1 ? 1 : (chunks_ll > kChunkCap ? kChunkCap : chunks_ll));
     const long long gwork = lm.use_gpr ? work : 0;
@@ -1242,9 +1218,15 @@ cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, co
     const BlockOut bo = blocks ? *blocks : BlockOut();
     if (blocks) {
         TRY(lm_compact3d(pk, lm, st));
-        k_linearize<true><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
+        k_linearize<true, 1><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
+    } else if ((long long)chunks * B <= 148 * 2) {
+        // one candidate (the step): one wave at two CTAs per SM, which a third CTA slot would leave unused; unbounded, the
+        // kernel takes 222 registers without spills (0.114 against 0.120 ms at 168 registers with 128 B of spills)
+        k_linearize<false, 1><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
     } else {
-        k_linearize<false><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
+        // a batch (the poll): several waves, three CTAs per SM at 168 registers (13.7 ms per 256-candidate poll against 14.0
+        // at four CTAs per SM)
+        k_linearize<false, 3><<<dim3(chunks, B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, lm.partial, stride, bo);
     }
     TRY(cudaGetLastError());
     if (gchunks > 0) {
