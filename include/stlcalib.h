@@ -366,6 +366,28 @@ stl_status_t stl_block_counts_multi(stl_ctx_t *ctx, int64_t *n_blocks, int32_t c
 stl_status_t stl_linearize_multi(stl_ctx_t *ctx, const double *x, int32_t B, const int32_t *problem, stl_lin_sums_t *out);
 stl_status_t stl_linearize_multi_device(stl_ctx_t *ctx, const double *x, int32_t B, const int32_t *problem, double *d_out, void *stream);
 
+/* Normal equations per keyframe: for candidate b (x [B][7]) on problem problem[b] (NULL: every candidate on problem 0, which
+ * needs a frozen set of one, as stl_linearize_batch), out[b][f] is the stl_lin_sums_t of the frozen blocks of keyframe f
+ * alone: cost, J^T r, J^T J and the block / residual counts, with the Huber correction of stl_linearize_batch.
+ * For leave-one-keyframe-out or k-fold checks of an LM refinement, per-keyframe observability (the spectrum of H_f), or
+ * dropping keyframes whose cost dominates.
+ *   Layout: out is [B][n_kf] rows, n_kf = this context's pack.  Rows of unselected keyframes are zero, and so is the row of
+ *     a keyframe without blocks.
+ *   Sum: the rows of a candidate sum to its stl_linearize_multi record; block and residual counts exactly, cost, J^T r and
+ *     J^T J up to the order of the fp64 additions.  Every block's values and partials come from the same device code as
+ *     the record's; only the summation order differs.
+ *   Row independence (bitwise): a row depends only on its keyframe's blocks and the candidate, whatever B, the other
+ *     candidates and problems of the call, the current selection (as long as f is selected) and the keyframe shard
+ *     holding f.
+ *   Errors: those of stl_linearize_multi.  No association, or a selection call since the last one -> STL_ERR_STATE (so is
+ *     variant 1, which has no association); problem == NULL with a set of more than one problem -> STL_ERR_STATE; a
+ *     problem index outside [0, P), or a null or non-positive argument -> STL_ERR_INVALID.
+ *   No exchange: with a communicator attached each rank returns the rows of its own keyframes and makes no collective call,
+ *     as stl_eval_frames.
+ * Its kernels count in work counter [5] (launches) and, with profiling on, are timed under STL_STAGE_LINEARIZE.  Device
+ * scratch of 8 (41 + 41 use_gpr + 62) bytes per (candidate, keyframe) is kept with the context and grows on demand. */
+stl_status_t stl_linearize_frames(stl_ctx_t *ctx, const double *x, int32_t B, const int32_t *problem, stl_lin_sums_t *out);
+
 /* One LM iteration for each of P starts (x [P][7]): BAError sums at x[p], BuildProblem at x[p] for the problems flagged in
  * rebuild (NULL = all, which makes a new set), linearisation of problem p at x[p]; ONE [P][74] record, exchanged once.
  * Same bits as stl_eval_batch + stl_associate_multi + stl_linearize_multi.  P = 1 is stl_step_batch(x, 1, rebuild ?

@@ -96,6 +96,13 @@ class Context {
         check(stl_linearize_multi(ctx_, x, B, problem, out.data()), "stl_linearize_multi");
         return out;
     }
+    // normal equations per keyframe: [B][n_kf] rows (n_kf = the pack's), row f of candidate b = keyframe f's blocks alone on
+    // problem problem[b] (null: every candidate on problem 0, a set of one); zero rows for unselected keyframes
+    std::vector<stl_lin_sums_t> linearize_frames(const double *x, int B, int n_kf, const int32_t *problem = nullptr) {
+        std::vector<stl_lin_sums_t> out((size_t)B * (size_t)n_kf);
+        check(stl_linearize_frames(ctx_, x, B, problem, out.data()), "stl_linearize_frames");
+        return out;
+    }
     // one LM iteration of P starts: {eval sums, linearisation} of problem p at x[p], BuildProblem of the flagged problems first
     std::vector<stl_step_sums_t> step_multi(const double *x, int P, const uint8_t *rebuild = nullptr) {
         std::vector<stl_step_sums_t> out((size_t)P);

@@ -162,6 +162,7 @@ CALIB_SYMBOLS = {
     "stl_block_counts_multi": (C.c_int, [_vp, _i64p, C.c_int32]),
     "stl_linearize_multi": (C.c_int, [_vp, _dp, C.c_int32, _i32p, C.POINTER(LinSums)]),
     "stl_linearize_multi_device": (C.c_int, [_vp, _dp, C.c_int32, _i32p, _vp, _vp]),
+    "stl_linearize_frames": (C.c_int, [_vp, _dp, C.c_int32, _i32p, C.POINTER(LinSums)]),
     "stl_step_multi": (C.c_int, [_vp, _dp, C.c_int32, _u8p, C.POINTER(StepSums)]),
     "stl_step_multi_device": (C.c_int, [_vp, _dp, C.c_int32, _u8p, _vp, _vp]),
     "stl_he_linearize": (C.c_int, [_vp, C.POINTER(HeEdges), _dp, C.c_int32, C.POINTER(LinSums), _dp]),

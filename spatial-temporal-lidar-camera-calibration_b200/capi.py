@@ -229,6 +229,23 @@ class Context:
                                                               out.ctypes.data_as(C.POINTER(_abi.LinSums))))
         return out
 
+    def linearize_frames(self, X, problem=None) -> np.ndarray:
+        """Normal equations per keyframe: candidate b (X [B,7]) on problem problem[b] (None: every candidate on problem 0, which
+        needs a frozen set of one) -> [B, n_kf, 62] (host), row f = the :meth:`linearize_multi` record of keyframe f's blocks
+        alone.  The rows of a candidate sum to its record; rows of unselected keyframes are zero.  Each rank returns its own
+        keyframes (no exchange)."""
+        X = np.ascontiguousarray(np.atleast_2d(X), dtype=np.float64)
+        if X.ndim != 2 or X.shape[1] != 7 or X.shape[0] == 0:
+            raise ValueError(f"linearize_frames: X must be [B, 7] with B >= 1, got shape {X.shape}")
+        B = X.shape[0]
+        keep, pp = self._problems(problem, B)
+        if self.pack is None:
+            raise _abi.StlError(4, "no pack uploaded")
+        out = np.empty((B, int(self.pack.n_kf), _abi.STL_LIN_NSUMS), dtype=np.float64)
+        _check(self.lib, self.h, self.lib.stl_linearize_frames(self.h, X.ctypes.data_as(_dp), B, pp,
+                                                               out.ctypes.data_as(C.POINTER(_abi.LinSums))))
+        return out
+
     def linearize_multi_device(self, X, d_out_ptr: int, problem=None, stream_ptr: int = 0):
         X = np.ascontiguousarray(np.atleast_2d(X), dtype=np.float64)
         keep, pp = self._problems(problem, X.shape[0])

@@ -1281,6 +1281,31 @@ stl_status_t stl_linearize_multi(stl_ctx_t *ctx, const double *x, int32_t B, con
     return STL_OK;
 }
 
+stl_status_t stl_linearize_frames(stl_ctx_t *ctx, const double *x, int32_t B, const int32_t *problem, stl_lin_sums_t *out) {
+    if (!ctx || !x || !out || B <= 0) return STL_ERR_INVALID;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    std::vector<int> prob;
+    if (problem) {
+        const stl_status_t s = check_problems(ctx, B, problem, prob);
+        if (s != STL_OK) return s;
+    } else {  // every candidate on problem 0, as stl_linearize_batch
+        if (!ctx->lm.ready) return fail(ctx, STL_ERR_STATE, "stl_associate has not been called");
+        if (need_single(ctx, "stl_linearize_frames without problem indices", "stl_linearize_frames with problem indices") != STL_OK)
+            return STL_ERR_STATE;
+    }
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = acquire_stream(ctx, nullptr);
+    double *d_rows = nullptr;
+    cudaError_t e;
+    // no exchange: every rank returns the rows of its own keyframes
+    { StageTimer t(ctx, STL_STAGE_LINEARIZE, st); e = lm_linearize_frames(ctx->pk, ctx->dpr, ctx->lm, x, problem ? prob.data() : nullptr, B, &d_rows, st); }
+    if (e != cudaSuccess) return fail(ctx, STL_ERR_CUDA, "linearize_frames: %s", cudaGetErrorString(e));
+    ctx->launches += ctx->pk.n_sel > 0 ? 2 + (ctx->lm.use_gpr ? 1 : 0) : 0;  // k_linearize (frames), (k_linearize_gpr,) k_lin_frames_finish
+    CK(cudaMemcpyAsync(out, d_rows, sizeof(double) * STL_LIN_NSUMS * (size_t)B * (size_t)ctx->pk.n_kf, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return STL_OK;
+}
+
 // One LM iteration for each of P starts.  P = 1 is stl_step_batch(x, 1, rebuild ? rebuild[0] : 1) (overlapped); a larger set runs
 // the stages one after another on the caller's stream, chunk by chunk of the workspace: evaluation of the chunk's starts, then
 // BuildProblem of its flagged problems, reusing the correspondences and the 1-NN the evaluation has just left in the workspace;

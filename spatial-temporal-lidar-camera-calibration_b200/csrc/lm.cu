@@ -439,11 +439,29 @@ __device__ __forceinline__ int sel_slot(const DevPack &pk, int v) {
     return v + pk.sel_mp[lo].y;
 }
 
+
+// First position in the sorted run l[0, n) whose value is >= v
+__device__ __forceinline__ int lower_pos(const int *__restrict__ l, int n, long long v) {
+    int lo = 0, hi = n;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (l[mid] < v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
 // grid (chunks, B): candidate blockIdx.y on problem cprob[blockIdx.y].  The 3-D/3-D blocks are walked over ALL query slots of
 // that problem (no compacted list: the work per block is light, and the association then has no select on the way to the
 // linearisation).  WB (stl_eval_blocks) numbers the blocks and therefore walks the compacted list (problem 0).
 // MINB: resident CTAs per SM the registers must allow (lm_linearize); the two forms compute the same bits.
-template <bool WB, int MINB>
+// FR (stl_linearize_frames): per-keyframe rows, grid (ceil(n_sel / 4), B).  Warp w of CTA x sums the blocks of selection position
+// x * 4 + w alone, the four warps sharing the candidate tables: its 3-D/2-D blocks are the keyframe's run of the problem's idx2d
+// list (slot order, found by binary search for the keyframe's slot bounds), lane l taking the run's blocks l, l + 32, ...; its
+// 3-D/3-D blocks come from the queue walk below over the keyframe's own slots [mp_off, mp_off + n_mp), 32 per round; the warp's
+// shuffle tree makes the row, written at partial[blockIdx.y][position] (partial_stride = n_sel).  Which lane sums which block,
+// and the order of the sum, so depend on the keyframe's blocks alone: not on B, the other candidates, the selection, the problem
+// set or the shard holding the keyframe.
+template <bool WB, int MINB, bool FR = false>
 __global__ void __launch_bounds__(kLinThreads, MINB)
 k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, const int *__restrict__ cprob,
             double *__restrict__ partial, int partial_stride, const BlockOut bo) {
@@ -459,16 +477,27 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
     }
     lm_list_start(lm, prob, 0, &list0);
     __syncthreads();
+    const int fpos = FR ? (int)(blockIdx.x * (kLinThreads / 32) + (threadIdx.x >> 5)) : 0;  // FR: the warp's selection position
+    if (FR && fpos >= pk.n_sel) return;  // whole warps; FR has no CTA barrier below
     Acc A;
 #pragma unroll
     for (int i = 0; i < kLinVals; ++i) A.v[i] = 0.0;
     const int C = pk.n_covis;
-    const int stride = gridDim.x * kLinThreads, t0 = blockIdx.x * kLinThreads + threadIdx.x;
+    const int stride = FR ? 32 : gridDim.x * kLinThreads;
+    long long s0 = 0, s1 = 0;  // FR: the keyframe's problem-local slots
+    if (FR) {
+        const DevKf &Kf = pk.kf[sel_kf(pk, fpos)];
+        s0 = Kf.mp_off;
+        s1 = Kf.mp_off + Kf.n_mp;
+    }
 
     // block counts live on the device (written by the association kernels on this stream): no host round trip
     const int *counts = lm.d_counts + prob * 4;
-    const int n2d = counts[0];
+    const int n2d_all = counts[0];
     const int *idx2d = lm.idx2d + list0;
+    const long long pg = (long long)prob * lm.slot_stride;
+    const int t0 = FR ? lower_pos(idx2d, n2d_all, pg + s0) + (int)(threadIdx.x & 31) : blockIdx.x * kLinThreads + threadIdx.x;
+    const int n2d = FR ? lower_pos(idx2d, n2d_all, pg + s1) : n2d_all;
     // ---- 3-D/2-D blocks: IBA_PlaneFactor (IBACalib2.hpp:152-184)
     for (int it = t0; it < n2d; it += stride) {
         const int slot = idx2d[it];  // global slot (problem offset included)
@@ -527,14 +556,14 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
     // slots per round, queues the flagged ones in shared memory and evaluates 32 queued blocks at a time (the tail at the end): the
     // lanes stay full although only half of the slots carry a block, and nothing outside this kernel has to compact the list.
     // Which thread sums which block depends on the flags alone, never on the batch size.
-    const long long n3 = WB ? (long long)counts[1] : (pk.sel ? pk.n_sel_mp : lm.max_blocks);
+    const long long n3 = FR ? s1 : WB ? (long long)counts[1] : (pk.sel ? pk.n_sel_mp : lm.max_blocks);
     const long long po = (long long)prob * lm.slot_stride;  // the 3-D walk is in problem-local slots
     const uint8_t *flag3d = lm.flag3d + po, *type3d = lm.type3d + po;
     const double *geo3d = lm.geo3d + po * 9;
     __shared__ int q3[kLinThreads / 32][64];
     const int lane3 = threadIdx.x & 31, warp3 = threadIdx.x >> 5;
     int qlen = 0;                                                    // warp-uniform
-    long long base = (long long)blockIdx.x * kLinThreads + warp3 * 32;  // first slot of this warp's next round
+    long long base = FR ? s0 : (long long)blockIdx.x * kLinThreads + warp3 * 32;  // first slot of this warp's next round
     for (long long it = t0;; it += stride) {
         long long slot = it;
         if (WB) {
@@ -544,7 +573,7 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
             const bool more = base < n3;
             if (more) {
                 const long long sl = base + lane3;
-                const int rs = pk.sel && sl < n3 ? sel_slot(pk, (int)sl) : (int)sl;
+                const int rs = !FR && pk.sel && sl < n3 ? sel_slot(pk, (int)sl) : (int)sl;
                 const bool on = sl < n3 && flag3d[rs];
                 const unsigned mask = __ballot_sync(0xffffffffu, on);
                 if (on) q3[warp3][qlen + __popc(mask & ((1u << lane3) - 1))] = rs;
@@ -599,15 +628,20 @@ k_linearize(const DevPack pk, const DevParams pr, const LmState lm, const LmCand
         A.v[0] += 0.5 * rho0;
     }
 
-    // ---- CTA reduction (fixed order)
+    // ---- CTA reduction (fixed order); FR: the warp's row
     __shared__ double red[kLinThreads / 32][kLinVals];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
     for (int i = 0; i < kLinVals; ++i) {
         double x = A.v[i];
         for (int o = 16; o; o >>= 1) x += __shfl_down_sync(0xffffffffu, x, o);
-        if (lane == 0) red[warp][i] = x;
+        if (FR) {
+            if (lane == 0) partial[((long long)blockIdx.y * partial_stride + fpos) * kLinVals + i] = x;
+        } else if (lane == 0) {
+            red[warp][i] = x;
+        }
     }
+    if (FR) return;
     __syncthreads();
     if (threadIdx.x < kLinVals) {
         double x = 0.0;
@@ -680,8 +714,10 @@ __device__ __forceinline__ D7 shfl7(const D7 &x, int src) {
     return r;
 }
 
-// grid (chunks, B), one warp per CTA
-template <bool WB>
+// grid (chunks, B), one warp per CTA.  FR (stl_linearize_frames): grid (n_sel, B), CTA x walks, in list order, the run of
+// selection position x's keyframe in the problem's GPR list and writes its row at partial[blockIdx.y][x] (partial_stride = n_sel,
+// partial_off = 0): the row's sum order depends on that keyframe's blocks alone.
+template <bool WB, bool FR = false>
 __global__ void __launch_bounds__(32)
 k_linearize_gpr(const DevPack pk, const DevParams pr, const LmState lm, const LmCand *__restrict__ cands, const int *__restrict__ cprob,
                 double *__restrict__ partial, int partial_stride, int partial_off, const BlockOut bo) {
@@ -703,7 +739,15 @@ k_linearize_gpr(const DevPack pk, const DevParams pr, const LmState lm, const Lm
     for (int i = 0; i < kLinVals; ++i) A.v[i] = 0.0;
     const int C = pk.n_covis;
     const int nG = counts[3];
-    for (int it = blockIdx.x; it < nG; it += gridDim.x) {
+    int it0 = blockIdx.x, it1 = nG, step = gridDim.x;
+    if (FR) {  // the keyframe's slots [mp_off, mp_off + n_mp) of problem prob
+        const DevKf &Kf = pk.kf[sel_kf(pk, blockIdx.x)];
+        const long long po = (long long)prob * lm.slot_stride;
+        it0 = lower_pos(lm.idxG + list0, nG, po + Kf.mp_off);
+        it1 = lower_pos(lm.idxG + list0, nG, po + Kf.mp_off + Kf.n_mp);
+        step = 1;
+    }
+    for (int it = it0; it < it1; it += step) {
         const int cs = lm.idxG[list0 + it];  // global slot
         const int f = lm.slot_kf[cs];
         const uint32_t kp = lm.slot_kp[cs];
@@ -839,6 +883,15 @@ k_linearize_gpr(const DevPack pk, const DevParams pr, const LmState lm, const Lm
         partial[((long long)blockIdx.y * partial_stride + partial_off + blockIdx.x) * kLinVals + i] = red[i];
 }
 
+// Position in the kLinVals packed sums (cost, g[7], the upper triangle of H by rows, counts) of value v of the STL_LIN_NSUMS
+// record (cost, g[7], H[7][7] full, counts)
+__device__ __forceinline__ int lin_packed(int v) {
+    if (v < 8) return v;
+    if (v >= 57) return v - 21;
+    const int i = (v - 8) / 7, j = (v - 8) % 7, a = i < j ? i : j, b = i < j ? j : i;
+    return 8 + a * 7 - a * (a - 1) / 2 + (b - a);
+}
+
 // one CTA per candidate: sums the per-CTA partials in order and expands H to the full symmetric 7x7
 // one CTA of 1024 threads per candidate: warp w sums values w, w+32 over the chunks (lane-strided partial
 // sums, then a shuffle tree: a fixed order, so the result is reproducible)
@@ -853,16 +906,20 @@ k_lin_finish(const double *__restrict__ partial, int nchunks, double *__restrict
         if (lane == 0) tot[v] = x;
     }
     __syncthreads();
-    if (threadIdx.x == 0) {
-        double *o = out + (long long)b * out_stride;
-        o[0] = tot[0];
-        for (int a = 0; a < 7; ++a) o[1 + a] = tot[1 + a];
-        int h = 8;
-        for (int a = 0; a < 7; ++a)
-            for (int c = a; c < 7; ++c) { o[8 + a * 7 + c] = tot[h]; o[8 + c * 7 + a] = tot[h]; ++h; }
-        o[57] = tot[36]; o[58] = tot[37]; o[59] = tot[38]; o[60] = tot[39]; o[61] = tot[40];
-    }
+    if (threadIdx.x < STL_LIN_NSUMS) out[(long long)b * out_stride + threadIdx.x] = tot[lin_packed(threadIdx.x)];
     if (P.n > 1) p2p_allreduce_record(P, b, out + (long long)b * out_stride + P.off);  // keyframes sharded over GPUs: sum the shards here
+}
+
+// per-keyframe rows: one thread per value of out[b][sel_kf(pos)][STL_LIN_NSUMS] = plane / point row + GPR row (in that order)
+__global__ void k_lin_frames_finish(const DevPack pk, const double *__restrict__ rows, const double *__restrict__ rows_gpr, int B,
+                                    double *__restrict__ out /*[B][n_kf][STL_LIN_NSUMS]*/) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)B * pk.n_sel * STL_LIN_NSUMS) return;
+    const int v = (int)(i % STL_LIN_NSUMS);
+    const long long r = i / STL_LIN_NSUMS;  // b * n_sel + pos
+    const int b = (int)(r / pk.n_sel), pos = (int)(r % pk.n_sel);
+    const long long src = r * kLinVals + lin_packed(v);
+    out[((long long)b * pk.n_kf + sel_kf(pk, pos)) * STL_LIN_NSUMS + v] = rows_gpr ? rows[src] + rows_gpr[src] : rows[src];
 }
 
 template <class T> void dfree(T *&p) { if (p) { cudaFree(p); p = nullptr; } }
@@ -873,7 +930,7 @@ void lm_free(LmState &lm) {
     dfree(lm.slot_kf); dfree(lm.slot_kp); dfree(lm.flags); dfree(lm.geo2d); dfree(lm.geo3d);
     dfree(lm.idxG); dfree(lm.gpr_nb); dfree(lm.gpr_m); dfree(lm.gpr_hyper);
     dfree(lm.amap); dfree(lm.stage); dfree(lm.plane_a); dfree(lm.nnb_pos); dfree(lm.nbb); dfree(lm.nbbx); dfree(lm.nbb_m); dfree(lm.nbb_last);
-    dfree(lm.idx2d); dfree(lm.idx3d); dfree(lm.d_sel); dfree(lm.d_tmp); dfree(lm.partial); dfree(lm.d_cand);
+    dfree(lm.idx2d); dfree(lm.idx3d); dfree(lm.d_sel); dfree(lm.d_tmp); dfree(lm.partial); dfree(lm.frames); dfree(lm.d_cand);
     if (lm.h_cand) cudaFreeHost(lm.h_cand);
     if (lm.h_counts) cudaFreeHost(lm.h_counts);
     if (lm.h_amap) cudaFreeHost(lm.h_amap);
@@ -1236,6 +1293,43 @@ cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, co
     }
     if (before_finish) TRY(cudaStreamWaitEvent(st, before_finish, 0));
     k_lin_finish<<<B, 1024, 0, st>>>(lm.partial, stride, d_out, out_stride > 0 ? out_stride : STL_LIN_NSUMS, p2p ? *p2p : P2pView());
+    TRY(cudaGetLastError());
+#undef TRY
+    return cudaSuccess;
+}
+
+// Per-keyframe rows of B candidates (stl_linearize_frames): the plane / point rows (k_linearize<false, 1, true>), the GPR rows
+// (k_linearize_gpr<false, true>), then k_lin_frames_finish adds them and scatters them into the zeroed [B][n_kf][STL_LIN_NSUMS]
+// output in lm.frames, returned in *d_out.  No exchange: the rows are this context's keyframes.
+cudaError_t lm_linearize_frames(const DevPack &pk, const DevParams &pr, LmState &lm, const double *x, const int *problem, int B, double **d_out,
+                                cudaStream_t st) {
+    cudaError_t e;
+#define TRY(x) do { e = (x); if (e != cudaSuccess) return e; } while (0)
+    TRY(lm_stage_candidates(lm, x, problem, B, st));
+    const LmCand *cands = reinterpret_cast<const LmCand *>(lm.d_cand);
+    const int *cprob = problem ? reinterpret_cast<const int *>(cands + B) : nullptr;
+    const long long nrow = (long long)B * pk.n_sel, nout = (long long)B * pk.n_kf * STL_LIN_NSUMS;
+    const long long need = nrow * kLinVals * (lm.use_gpr ? 2 : 1) + nout;  // 8 (41 + 41 use_gpr + 62) bytes per (candidate, keyframe)
+    if (need > lm.frames_cap) {
+        dfree(lm.frames);
+        lm.frames_cap = 0;
+        TRY(cudaMalloc(&lm.frames, 8 * need));
+        lm.frames_cap = need;
+    }
+    double *rows = lm.frames, *rows_gpr = lm.use_gpr ? rows + nrow * kLinVals : nullptr;
+    double *out = lm.frames + nrow * kLinVals * (lm.use_gpr ? 2 : 1);
+    *d_out = out;
+    if (pk.sel || pk.n_sel < pk.n_kf) TRY(cudaMemsetAsync(out, 0, 8 * (size_t)nout, st));  // rows of unselected keyframes
+    if (pk.n_sel == 0) return cudaSuccess;
+    const int fw = kLinThreads / 32;  // keyframes per CTA
+    k_linearize<false, 1, true><<<dim3((unsigned)((pk.n_sel + fw - 1) / fw), (unsigned)B), kLinThreads, 0, st>>>(pk, pr, lm, cands, cprob, rows, pk.n_sel, BlockOut());
+    TRY(cudaGetLastError());
+    if (rows_gpr) {
+        k_linearize_gpr<false, true><<<dim3((unsigned)pk.n_sel, (unsigned)B), 32, 0, st>>>(pk, pr, lm, cands, cprob, rows_gpr, pk.n_sel, 0, BlockOut());
+        TRY(cudaGetLastError());
+    }
+    const long long nv = nrow * STL_LIN_NSUMS;
+    k_lin_frames_finish<<<(unsigned)((nv + 255) / 256), 256, 0, st>>>(pk, rows, rows_gpr, B, out);
     TRY(cudaGetLastError());
 #undef TRY
     return cudaSuccess;

@@ -66,6 +66,8 @@ struct LmState {
     // ---- linearisation
     double *partial = nullptr;    // [B][grid][kLinVals]
     long long partial_cap = 0;
+    double *frames = nullptr;     // stl_linearize_frames: [B][n_sel][kLinVals] rows (GPR rows after them), then [B][n_kf][62] out
+    long long frames_cap = 0;
     void *d_cand = nullptr;       // [B] LmCand, then [B] int problem of each candidate
     void *h_cand = nullptr;       // pinned
     int cand_cap = 0;
@@ -112,6 +114,10 @@ struct BlockOut {
 cudaError_t lm_linearize(const DevPack &pk, const DevParams &pr, LmState &lm, const double *x, const int *problem, int B, double *d_out,
                          cudaStream_t st, const BlockOut *blocks = nullptr, int out_stride = 0, const P2pView *p2p = nullptr,
                          cudaEvent_t before_finish = nullptr, bool cand_staged = false);
+// Per-keyframe normal equations (stl_linearize_frames): x, problem as lm_linearize; *d_out = DEVICE [B][n_kf][STL_LIN_NSUMS] (in
+// lm.frames, valid until the next call), row f = the blocks of keyframe f alone, zero for unselected keyframes.  No exchange.
+cudaError_t lm_linearize_frames(const DevPack &pk, const DevParams &pr, LmState &lm, const double *x, const int *problem, int B, double **d_out,
+                                cudaStream_t st);
 cudaError_t lm_compact3d(const DevPack &pk, LmState &lm, cudaStream_t st);
 // cand_staged: the caller has already run lm_stage_candidates(lm, x, problem, B, st) for exactly these x on this stream
 // before_finish (optional): event the finishing kernel waits for (the rest of the record it completes / exchanges)
